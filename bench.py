@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference ...                    # the reference's algorithm on the host cores (the oracle port)
+    python bench.py ... --dump-outputs DIR                  # also DIR/frame.npy, the frame of the last timed step (same seed, same inputs)
 
 A step = one pass of the hot path over one frame: W*H*spp paths through camera ray generation,
 Scene::intersect (sphere / planes / uniform-grid DDA), the BRDF bounce loop and the tile accumulator.
@@ -67,7 +68,14 @@ def parse_args():
     p.add_argument("--c3-spp", type=int, default=1000, help="samples of the configs[2] run in other_configs (tests shrink it)")
     p.add_argument("--c5-spp", type=int, default=4096, help="samples of the configs[4] run in other_configs (tests shrink it)")
     p.add_argument("--no-c4", action="store_true", help="skip the configs[3] leg of other_configs")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the frame of the last timed step to DIR/frame.npy (f64 H x W x 3; above 64 MB a fixed sample of its pixels)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs records the CUDA path; the reference arm picks its sample count from its own speed")
+    return args
 
 
 def scene_objects(name):
@@ -343,6 +351,19 @@ def roofline_record(A, args, scene, settings, local, world, st0, st1, samples_ra
 
 
 PRECISIONS = {"f64": 0, "f32shade": 1}
+DUMP_BYTES = 60_000_000          # under 64 MB with the .npy header; a 1920x1080 f64 frame is 49.8 MB
+
+
+def dump_frame(out_dir: str, frame: np.ndarray) -> None:
+    """frame.npy: the whole frame when it fits in DUMP_BYTES, otherwise the pixels of a seeded sample (rows of a (k, 3) array,
+    in pixel order), the same pixels for every run at the same resolution so that two builds can be compared."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = np.ascontiguousarray(frame, dtype=np.float64)
+    if out.nbytes > DUMP_BYTES:
+        pixels = out.reshape(-1, out.shape[-1])
+        keep = np.random.default_rng(0).choice(pixels.shape[0], DUMP_BYTES // pixels[0].nbytes, replace=False)
+        out = pixels[np.sort(keep)]
+    np.save(os.path.join(out_dir, "frame.npy"), out)
 
 
 def bench_ours(args):
@@ -426,7 +447,9 @@ def bench_ours(args):
     value = samples_total / ms_total / 1e3
     launches = int(sum_over_ranks(float(s1["kernel_launches"] - s0["kernel_launches"])))
     rays = int(sum_over_ranks(float(s1["rays"] - s0["rays"])))
-    frame = dr.frame(spp)
+    frame = dr.frame(spp)               # the running sums of the last timed step over spp (a view of a buffer the legs below reuse)
+    if frame is not None and args.dump_outputs:
+        dump_frame(args.dump_outputs, frame)
     mean_radiance = [float(x) for x in frame.mean(axis=(0, 1))] if frame is not None else None
 
     roofline = stages = None

@@ -1,6 +1,6 @@
-"""Regenerate tests/golden/* from the reference checkout (run in the build container, where /root/reference exists).
+"""Regenerate tests/golden/* from a checkout of the reference project (Nyrox/raymond).
 
-    python scripts/make_golden.py
+    RAYMOND_REFERENCE_DIR=<reference checkout> python scripts/make_golden.py
 
 1. reference_png_blocks.json — 16x16-pixel block means (8-bit RGB) of the reference's OWN renders
    examples/ReflectiveSpheres.png and examples/GoldDragon.png (592x340, 500 spp, 5 bounces, README.md:24-28).
@@ -8,8 +8,8 @@
    tests/test_oracle.py renders the same scene with the oracle and compares block means.
 2. reference_mesh_kats.json — what the ORACLE computes on the reference's shipped PLY meshes (assets/meshes):
    bounds, grid resolution, cell/reference counts, CRC32 of the cell lists and of the hit results of a fixed
-   160x120 primary-ray frame.  Not reference truth — a regression pin that also travels to the GPU box,
-   where /root/reference does not exist.
+   160x120 primary-ray frame.  Not reference truth — a regression pin, checked by the tests when the reference's
+   meshes are at hand.
 """
 import json
 import os
@@ -20,7 +20,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("RAYMOND_REFERENCE_DIR") or sys.exit("make_golden.py: set RAYMOND_REFERENCE_DIR to a checkout of the reference project (Nyrox/raymond)")
 OUT = os.path.join(ROOT, "tests", "golden")
 
 

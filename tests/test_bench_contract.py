@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,6 +36,42 @@ def test_reference_arm_other_ranks_print_nothing():
     res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"] + SMALL, capture_output=True, text=True,
                          cwd=ROOT, env=env, timeout=120)
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+def test_bench_rejects_what_it_cannot_time_or_dump():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, cwd=ROOT, timeout=120)
+        assert res.returncode == 2 and "error" in res.stderr, extra
+
+
+def test_dump_frame_samples_a_large_frame_the_same_way_every_time(tmp_path, monkeypatch):
+    import bench
+    frame = np.random.default_rng(5).random((20, 30, 3))
+    bench.dump_frame(str(tmp_path / "whole"), frame)
+    assert np.array_equal(np.load(tmp_path / "whole" / "frame.npy"), frame)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * 24)
+    bench.dump_frame(str(tmp_path / "a"), frame)
+    bench.dump_frame(str(tmp_path / "b"), frame.copy())
+    a, b = np.load(tmp_path / "a" / "frame.npy"), np.load(tmp_path / "b" / "frame.npy")
+    assert a.shape == (100, 3) and a.dtype == np.float64 and np.array_equal(a, b)
+    rows = [int(np.nonzero((frame.reshape(-1, 3) == p).all(axis=1))[0][0]) for p in a]
+    assert rows == sorted(set(rows))                       # distinct pixels of the frame, in pixel order
+
+
+@pytest.mark.gpu
+def test_dumped_frame_is_the_same_for_any_number_of_steps(tmp_path):
+    """--dump-outputs writes the last timed step's frame; every step renders the same seeded frame, so --steps does not change
+    it, while the timed region holds exactly --steps frames' worth of kernel launches."""
+    quick = ["--no-extras", "--no-e2e", "--no-cpu-baseline"]
+    one = run_bench(quick + ["--dump-outputs", str(tmp_path / "one")])
+    three = run_bench(quick + ["--steps", "3", "--dump-outputs", str(tmp_path / "three")])
+    assert (one["steps"], three["steps"]) == (1, 3)
+    assert one["gpu_launches"] > 0 and three["gpu_launches"] == 3 * one["gpu_launches"]
+    assert three["rays_per_path"] == one["rays_per_path"]
+    a, b = np.load(tmp_path / "one" / "frame.npy"), np.load(tmp_path / "three" / "frame.npy")
+    assert a.shape == (90, 160, 3) and a.dtype == np.float64 and np.isfinite(a).all() and a.max() > 0
+    assert np.array_equal(a, b)
+    assert np.allclose(a.mean(axis=(0, 1)), one["mean_radiance"], rtol=1e-12, atol=0)
 
 
 @pytest.mark.gpu

@@ -7,11 +7,15 @@ from oracle import oracle as O
 from raymond_b200 import api as A
 from raymond_b200 import fixtures as F
 
-REFERENCE_MESHES = "/root/reference/assets/meshes"   # only exists in the build container
+# A checkout of the reference project (Nyrox/raymond): its PLY meshes and renders are not part of this repository, so the
+# tests that read them skip unless RAYMOND_REFERENCE_DIR names one.
+REFERENCE_DIR = os.environ.get("RAYMOND_REFERENCE_DIR", "")
+REFERENCE_MESHES = os.path.join(REFERENCE_DIR, "assets", "meshes")
+NEEDS_REFERENCE = "needs a checkout of the reference project in RAYMOND_REFERENCE_DIR"
 
 
 def have_reference_assets() -> bool:
-    return os.path.isdir(REFERENCE_MESHES)
+    return bool(REFERENCE_DIR) and os.path.isdir(REFERENCE_MESHES)
 
 
 def oracle_scene(objects) -> O.Scene:
