@@ -209,12 +209,17 @@ typedef enum rm_precision {
     RM_PRECISION_F32_SHADING = 1 /* lobe sampling, Fresnel, GGX and Smith terms in f32 with FMA; agrees with the f64 mode within Monte-Carlo noise */
 } rm_precision;
 
-#define RM_FLAG_KEEP_NONFINITE 1u  /* accumulate NaN/Inf samples like the reference instead of dropping+counting them */
+/* Non-finite samples.  By default a sample whose value is NaN / Inf is dropped and counted (rm_stats.nonfinite_samples), and a
+ * path whose throughput became exactly (0,0,0) is stopped early.  With RM_FLAG_KEEP_NONFINITE every path is traced the way the
+ * reference traces it — no early stop; a path that ends without emission delivers throughput (*) 0, and at the bounce limit
+ * throughput (*) last weight (*) 0 — and every sample is accumulated, so a NaN / Inf weight anywhere on a path poisons its
+ * pixel exactly where the reference's does, and nonfinite_samples equals the reference's count. */
+#define RM_FLAG_KEEP_NONFINITE 1u
 #define RM_FLAG_STAGE_TIMING 2u    /* bracket every kernel launch with CUDA events; totals per wavefront stage in rm_stage_stats */
 #define RM_FLAG_COUNT_WORK 4u      /* instrumented kernels: count grid cells visited and triangle tests per stage (slower) */
-#define RM_FLAG_NO_RAY_BINNING 8u  /* tuning: traverse the bounced rays in queue order instead of binned by (start cell, direction octant) */
-#define RM_FLAG_FUSE_SETUP 16u     /* tuning: force the fused shade + next-depth set-up kernel (default: only for scenes without a grid) */
-#define RM_FLAG_SPLIT_SETUP 32u    /* tuning: force separate shade and set-up kernels */
+#define RM_FLAG_NO_RAY_BINNING 8u  /* reserved: accepted, no effect (the bounced rays are always traversed in queue order) */
+#define RM_FLAG_FUSE_SETUP 16u     /* reserved: accepted, no effect (shading and the next depth's set-up are separate kernels) */
+#define RM_FLAG_SPLIT_SETUP 32u    /* reserved: accepted, no effect (shading and the next depth's set-up are separate kernels) */
 
 /* GPU-side knobs that have no counterpart in the reference. Zero-initialise
  * for defaults (device 0, one rank, library-owned stream and buffers). */
@@ -288,7 +293,10 @@ int rm_task_finished(rm_task* task);
 typedef struct rm_stats {
     uint64_t samples;            /* paths started */
     uint64_t rays;               /* Scene::intersect evaluations */
-    uint64_t nonfinite_samples;  /* dropped (or kept, with RM_FLAG_KEEP_NONFINITE) */
+    uint64_t nonfinite_samples;  /* samples with a NaN / Inf channel.  With RM_FLAG_KEEP_NONFINITE: kept, and the reference's count.
+                                  * Without it: dropped, and counted as this library's paths produce them — a lower bound of the
+                                  * reference's count, since a path stopped at a zero throughput, a miss or the bounce limit
+                                  * delivers an exact 0 where the reference's product with a NaN / Inf weight is NaN. */
     uint64_t kernel_launches;    /* launches of this library's kernels */
     double device_ms;            /* CUDA-event time of the render section */
     double upload_ms;            /* host flatten + H2D of the scene */
@@ -338,8 +346,8 @@ int rm_renderer_stats(rm_renderer* r, rm_stats* out);
 /* Per-stage breakdown of the wavefront.  Slot d (1 <= d < RM_STAGE_SLOTS) is the stage that traces
  * and shades the rays of depth d (deeper stages share the last slot).  A stage is three kernels —
  * kind 0 set-up (ray generation / analytic objects / grid entry), kind 1 grid traversal, kind 2
- * shading (fused with the next depth's set-up where the library fuses them) — kind 3, slot 0 is the accumulator kernel,
- * and kind 4 the ray-binning kernels that order depth d's traversal records.  `ms` / `launches` need
+ * shading — kind 3, slot 0 is the accumulator kernel; kind 4 is reserved (no kernel of this version is counted
+ * there, it stays zero).  `ms` / `launches` need
  * RM_FLAG_STAGE_TIMING; `cells` / `triangle_tests` need RM_FLAG_COUNT_WORK; the rest is always
  * counted.  cells = C and triangle_tests = T of the algorithmic bytes-per-ray model
  * (SURVEY.md §8d: 64 + 8 C + 76 T, + 72 per shaded triangle hit). */

@@ -50,7 +50,7 @@ PARTITION_TILES = 1
 FLAG_KEEP_NONFINITE = 1
 FLAG_STAGE_TIMING = 2
 FLAG_COUNT_WORK = 4
-FLAG_NO_RAY_BINNING = 8
+FLAG_NO_RAY_BINNING = 8     # 8, 16, 32: reserved values, accepted with no effect
 FLAG_FUSE_SETUP = 16
 FLAG_SPLIT_SETUP = 32
 PRECISION_F64 = 0
@@ -108,7 +108,7 @@ class StatsC(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
-KERNEL_KINDS = ("setup", "traverse", "shade", "accumulate", "bin")
+KERNEL_KINDS = ("setup", "traverse", "shade", "accumulate", "bin")      # kind 4 ("bin") is reserved and stays zero
 
 
 class StageStatsC(C.Structure):

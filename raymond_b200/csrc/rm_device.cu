@@ -939,6 +939,7 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
     const unsigned limit = rp.bounce_limit;
     if (n_paths == 0) return RM_OK;
     const bool count = (r->opt.flags & RM_FLAG_COUNT_WORK) != 0;
+    const bool keep = (r->opt.flags & RM_FLAG_KEEP_NONFINITE) != 0;
     const unsigned persistent_grid = (unsigned)r->sms * 8u;
     RM_CUDA(cudaMemsetAsync(r->counters, 0, r->counter_slots * 3 * sizeof(unsigned), r->stream));
     if (limit == 0) RM_CUDA(cudaMemsetAsync(rp.contrib, 0, (size_t)rp.cap * 3 * sizeof(double), r->stream));   // trace() returns 0 at depth 1 > 0
@@ -962,16 +963,18 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         hook.begin(2);
         if (depth == 1) {
             const unsigned grid = std::min<unsigned>((n_paths + kBlock - 1) / kBlock, persistent_grid * 4u);
-            k_shade<true, PREC><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            if (keep) k_shade<true, PREC, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            else k_shade<true, PREC, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
         } else {
-            k_shade<false, PREC><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            if (keep) k_shade<false, PREC, true><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            else k_shade<false, PREC, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
         }
         hook.end(2);
     }
     {
         StageHook hook(r, 0);
         hook.begin(3);
-        k_accumulate<<<(rp.n_pixels + kBlock - 1) / kBlock, kBlock, 0, r->stream>>>(rp, r->accum, n_samples, (r->opt.flags & RM_FLAG_KEEP_NONFINITE) ? 1u : 0u);
+        k_accumulate<<<(rp.n_pixels + kBlock - 1) / kBlock, kBlock, 0, r->stream>>>(rp, r->accum, n_samples, keep ? 1u : 0u);
         hook.end(3);
     }
     RM_CUDA(cudaGetLastError());

@@ -633,16 +633,19 @@ __device__ __forceinline__ void lobe_f32(const RenderParams& rp, D3 normal64, D3
 // What one bounce does to a path, before the path's throughput T is involved (T is read from the queue only afterwards, so
 // its six registers are free during the bounce): BOUNCE_NONE = the path ends with no radiance, BOUNCE_EMIT = it delivers
 // T (*) v, BOUNCE_CONTINUE = it goes on from (o, d) with T (*) v.
+// KEEP (RM_FLAG_KEEP_NONFINITE): at the bounce limit the last weight is still computed and returned in v with BOUNCE_NONE,
+// because the reference multiplies the child's zero by it (:235-237, :281-282, :315-319) and a NaN / Inf weight makes the
+// sample NaN.  The lobe's draws are counter-based, so the extra evaluation leaves every other draw unchanged.
 enum Bounce : int { BOUNCE_NONE = 0, BOUNCE_EMIT = 1, BOUNCE_CONTINUE = 2 };
 
-template <int PREC>
+template <int PREC, bool KEEP>
 __device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, double hit_t, int hit_obj, unsigned hit_sub, unsigned pixel,
                                         unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
     if (hit_obj < 0) return BOUNCE_NONE;                                    // :242
     const DevObject& ob = sc.obj[hit_obj];
     const D3 frag = o + d * hit_t;                                          // :246
     if (ob.mat == RM_MATERIAL_EMISSION) { v = ld3(ob.color); return BOUNCE_EMIT; }   // :250
-    if (depth >= rp.bounce_limit) return BOUNCE_NONE;                       // the child call returns 0 (:235-237)
+    if (!KEEP && depth >= rp.bounce_limit) return BOUNCE_NONE;              // the child call returns 0 (:235-237)
     D3 normal;                                                              // :244
     if (ob.geom == GEOM_PLANE) normal = ld3(ob.g + 3);
     else if (ob.geom == GEOM_SPHERE) normal = normalize(frag - ld3(ob.g));
@@ -653,6 +656,7 @@ __device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& 
     double eps;
     if (PREC == RM_PRECISION_F32_SHADING) lobe_f32(rp, normal, to_camera, ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
     else lobe_f64(rp, normal, to_camera, ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
+    if (KEEP && depth >= rp.bounce_limit) return BOUNCE_NONE;
     o = frag + normal * eps;
     d = dir;
     return BOUNCE_CONTINUE;
@@ -1197,7 +1201,11 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
 }
 
 // Stage part 3: shade, then deliver radiance or append the next ray (warp-aggregated compaction) to the next depth's queue.
-template <bool FIRST, int PREC>
+// KEEP = RM_FLAG_KEEP_NONFINITE: the path's value is formed as the reference forms it, so that a NaN / Inf weight anywhere on
+// the path poisons the sample: no path is stopped for a zero throughput (D5), and a path that ends without emission delivers
+// T (*) 0 on a miss and T (*) w (*) 0 at the bounce limit instead of an exact (0, 0, 0).  The default instantiation is the
+// one the benchmark runs.
+template <bool FIRST, int PREC, bool KEEP>
 __global__ void __launch_bounds__(kBlock, RM_SHADE_BLOCKS_PER_SM) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
                                                    const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first) {
     const unsigned n = FIRST ? n_first : rp.cnt.rays[depth - 1];
@@ -1216,13 +1224,14 @@ __global__ void __launch_bounds__(kBlock, RM_SHADE_BLOCKS_PER_SM) k_shade(const 
             d = d3(qin.f[3][i], qin.f[4][i], qin.f[5][i]);
             const unsigned q = slot % rp.n_pixels, s_local = slot / rp.n_pixels;
             D3 v = d3(0.0, 0.0, 0.0);
-            const Bounce b = shade<PREC>(sc, rp, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
+            const Bounce b = shade<PREC, KEEP>(sc, rp, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
             // the path's value is (prod of weights) (*) emission (src/trace.rs:281-282,315-319): the throughput so far comes in only now
             T = d3(0.0, 0.0, 0.0);
-            if (b != BOUNCE_NONE) T = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), v);
-            cont = b == BOUNCE_CONTINUE && !(T.x == 0.0 && T.y == 0.0 && T.z == 0.0);   // nothing downstream can change a zero path value
+            if (KEEP || b != BOUNCE_NONE) T = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), v);
+            if (KEEP) cont = b == BOUNCE_CONTINUE;
+            else cont = b == BOUNCE_CONTINUE && !(T.x == 0.0 && T.y == 0.0 && T.z == 0.0);   // nothing downstream can change a zero path value
             if (!cont) {
-                const D3 result = b == BOUNCE_EMIT ? T : d3(0.0, 0.0, 0.0);
+                const D3 result = b == BOUNCE_EMIT ? T : KEEP ? mul(T, d3(0.0, 0.0, 0.0)) : d3(0.0, 0.0, 0.0);
                 rp.contrib[slot] = result.x;
                 rp.contrib[(size_t)rp.cap + slot] = result.y;
                 rp.contrib[2 * (size_t)rp.cap + slot] = result.z;
