@@ -7,6 +7,8 @@
 // --serve PORT is the reference's intended server role (server/src/main.rs:174-192 binds 127.0.0.1:17025 and never renders;
 // server/src/protocol.rs:9-14 is the message): listen on 127.0.0.1:PORT, accept one client, and write every Message of the
 // render — TileProgressed every --spi samples, then TileFinished — as one JSON text per line ("\r\n", like editor/src/main.js:35).
+// --adaptive T [--min-spp N] stops every tile at the first --spi checkpoint where its error estimate is <= T
+// (rm_render_tiled_adaptive) and prints the samples actually rendered.
 // Compile:  g++ -O2 -std=c++17 -Iinclude examples/cli_old.cpp -Lraymond_b200 -lraymond_cuda -Wl,-rpath,$PWD/raymond_b200 -o cli_old
 #include <arpa/inet.h>
 #include <netinet/in.h>
@@ -36,6 +38,8 @@ int main(int argc, char** argv) {
     unsigned gpus = 1, repeat = 1;
     int serve_port = 0;
     size_t spi = 0;
+    double adaptive = 0.0;
+    size_t min_spp = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--mesh") && i + 1 < argc) mesh_path = argv[++i];
         else if (!strcmp(argv[i], "--out") && i + 1 < argc) out_path = argv[++i];
@@ -47,7 +51,13 @@ int main(int argc, char** argv) {
         else if (!strcmp(argv[i], "--repeat") && i + 1 < argc) repeat = (unsigned)strtoul(argv[++i], nullptr, 10);
         else if (!strcmp(argv[i], "--serve") && i + 1 < argc) serve_port = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--spi") && i + 1 < argc) spi = strtoull(argv[++i], nullptr, 10);
-        else { fprintf(stderr, "usage: cli_old [--mesh dragon.ply] [--out output.png] [--width W --height H --spp N --seed S --gpus G --repeat R --serve PORT --spi N]\n"); return 2; }
+        else if (!strcmp(argv[i], "--adaptive") && i + 1 < argc) adaptive = strtod(argv[++i], nullptr);
+        else if (!strcmp(argv[i], "--min-spp") && i + 1 < argc) min_spp = strtoull(argv[++i], nullptr, 10);
+        else {
+            fprintf(stderr, "usage: cli_old [--mesh dragon.ply] [--out output.png] [--width W --height H --spp N --seed S --gpus G --repeat R --serve PORT --spi N"
+                            " --adaptive T --min-spp N]\n");
+            return 2;
+        }
     }
     const auto now = std::chrono::steady_clock::now();
     auto lap = [&](const char* what) {       // phase times on stderr (the reference prints only the total)
@@ -129,7 +139,9 @@ int main(int argc, char** argv) {
     for (unsigned rep = 0; rep < (repeat ? repeat : 1); rep++) {
         const auto r0 = std::chrono::steady_clock::now();
         opt.seed = seed + rep;
-        rm_task* task = rm_render_tiled(scene, &settings, &opt);                              // :152
+        const rm_adaptive_settings adapt{adaptive, min_spp};
+        rm_task* task = adaptive != 0.0 ? rm_render_tiled_adaptive(scene, &settings, &opt, &adapt)
+                                        : rm_render_tiled(scene, &settings, &opt);                   // :152
         if (!task) { fprintf(stderr, "render_tiled: %s\n", rm_last_error()); return 1; }
         lap("render_tiled returned");
         if (client >= 0) {
@@ -182,6 +194,7 @@ int main(int argc, char** argv) {
     lap("tonemap");
     const double secs = std::chrono::duration<double>(std::chrono::steady_clock::now() - now).count();
     printf("Finished render.\nTotal render time: %.3fs\nTotal amount of trace calls: %llu\n", secs, (unsigned long long)stats.rays);   // :183-188
+    if (adaptive != 0.0) printf("Samples rendered: %llu of %llu\n", (unsigned long long)stats.samples, (unsigned long long)(width * height * spp));
     CHECK(rm_write_png(out_path, export_.data(), width, height));                             // :194-197
     lap("png written");
     fprintf(stderr, "[cli_old] device time %.1f ms, %llu kernel launches, upload %.1f ms\n", stats.device_ms, (unsigned long long)stats.kernel_launches, stats.upload_ms);

@@ -64,6 +64,21 @@ extern "C" {
     pub fn rm_measure_fp64_rate(device: c_int, gops_out: *mut f64) -> c_int;                                // diagnostic (roofline)
 }
 
+// ---- per-tile adaptive sampling (include/raymond.h).  E_t of a tile after n >= 2 samples, per pixel and channel from the
+// running sum S and the running sum of squares Q: m = S/n, v = max(Q - S*m, 0)/(n-1), se2 = v/n;
+// r_p = sqrt(se2_R + se2_G + se2_B) / (m_R + m_G + m_B + 1e-3); E_t = sqrt(mean over the tile of r_p^2); converged iff E_t <= threshold.
+#[repr(C)] #[derive(Clone, Copy)] pub struct rm_adaptive_settings { pub threshold: f64, pub min_samples: usize }
+pub enum rm_renderer {}
+extern "C" {
+    // render_tiled with TileFinished(n) for every tile that converged at checkpoint n; NULL settings = rm_render_tiled.
+    // rm_task_pump still stops at the first message that is not TileProgressed: read an adaptive task with poll / await.
+    pub fn rm_render_tiled_adaptive(s: *const rm_scene, st: *const rm_settings, o: *const rm_gpu_options,
+                                    a: *const rm_adaptive_settings) -> *mut rm_task;
+    pub fn rm_renderer_read_moments(r: *mut rm_renderer, out: *mut rm_vec3) -> c_int;
+    pub fn rm_renderer_tile_errors(r: *mut rm_renderer, sample_count: usize, out: *mut f64, capacity: usize) -> usize;
+    pub fn rm_renderer_set_active_tiles(r: *mut rm_renderer, active: *const u8, tile_count: usize) -> c_int;
+}
+
 // ---- values of the enum / flag fields (include/raymond.h, RM_ABI_VERSION 2)
 pub const RM_PARTITION_SAMPLES: u32 = 0;        // rank g renders global samples g, g+G, ...
 pub const RM_PARTITION_TILES: u32 = 1;          // tiles dealt round-robin in the reference's queue order (src/trace.rs:146-172)
@@ -72,5 +87,6 @@ pub const RM_PRECISION_F32_SHADING: u32 = 1;    // BRDF sampling / weights in f3
 pub const RM_FLAG_KEEP_NONFINITE: u32 = 1;
 pub const RM_FLAG_STAGE_TIMING: u32 = 2;
 pub const RM_FLAG_COUNT_WORK: u32 = 4;
+pub const RM_FLAG_MOMENTS: u32 = 64;            // keep the running sums of squared samples (rm_renderer_read_moments / tile_errors)
 pub const RM_TILE_FINISHED: u32 = 0;            // Message::TileFinished
 pub const RM_TILE_PROGRESSED: u32 = 1;          // Message::TileProgressed

@@ -220,6 +220,10 @@ typedef enum rm_precision {
 #define RM_FLAG_NO_RAY_BINNING 8u  /* reserved: accepted, no effect (the bounced rays are always traversed in queue order) */
 #define RM_FLAG_FUSE_SETUP 16u     /* reserved: accepted, no effect (shading and the next depth's set-up are separate kernels) */
 #define RM_FLAG_SPLIT_SETUP 32u    /* reserved: accepted, no effect (shading and the next depth's set-up are separate kernels) */
+/* Second moments: next to the running sum S the renderer keeps, per pixel and channel, the running sum of squared sample
+ * values Q, under the same rule as S — samples added in global sample order; non-finite samples left out of both by default,
+ * added to both with RM_FLAG_KEEP_NONFINITE.  Read with rm_renderer_read_moments; used by rm_renderer_tile_errors. */
+#define RM_FLAG_MOMENTS 64u
 
 /* GPU-side knobs that have no counterpart in the reference. Zero-initialise
  * for defaults (device 0, one rank, library-owned stream and buffers). */
@@ -305,6 +309,28 @@ typedef struct rm_stats {
 int rm_task_stats(rm_task* task, rm_stats* out);
 void rm_task_destroy(rm_task* task);
 
+/* Per-tile adaptive sampling.  The error estimate of a tile after n >= 2 samples, per pixel p and channel c, from the
+ * running sum S and the running sum of squares Q (RM_FLAG_MOMENTS):
+ *   m = S / n,   v = max(Q - S * m, 0) / (n - 1),   se2 = v / n,
+ *   r_p = sqrt(se2_R + se2_G + se2_B) / (m_R + m_G + m_B + 1e-3),   E_t = sqrt(mean over the tile's pixels of r_p^2).
+ * A tile has converged iff E_t <= threshold.  A NaN anywhere makes that comparison false, so a NaN-poisoned tile of
+ * RM_FLAG_KEEP_NONFINITE renders to the full count.  Without that flag n still counts the dropped samples, as the mean does. */
+typedef struct rm_adaptive_settings {
+    double threshold;       /* finite, > 0 */
+    size_t min_samples;     /* no tile stops before max(min_samples, 2) samples */
+} rm_adaptive_settings;
+/* render_tiled with per-tile early stopping.  `adaptive` NULL = exactly rm_render_tiled.  Otherwise, at every progressive
+ * checkpoint n (every samples_per_iteration samples) with n >= max(min_samples, 2) and n < sample_count, each tile still
+ * rendering with E_t <= threshold gets TileFinished(sample_count = n) and is never rendered again; the others get
+ * TileProgressed(n) as in rm_render_tiled.  The messages of one checkpoint are in queue order.  A tile that stops early holds
+ * exactly the first n samples of the full render.  rm_task_await divides every tile by its own count; rm_stats.samples
+ * counts the paths actually started.  rm_task_pump keeps its reference semantics — it stops at the first message that is
+ * not TileProgressed — so read an adaptive task with rm_task_poll or rm_task_await.
+ * Checked before any device work: a threshold that is not finite or <= 0 and samples_per_iteration == 0 fail with
+ * RM_ERR_INVALID_ARGUMENT; one rank of a multi-process job (world_size > 1 with device_count <= 1) with RM_ERR_UNSUPPORTED. */
+rm_task* rm_render_tiled_adaptive(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options,
+                                  const rm_adaptive_settings* adaptive);
+
 /* -------------------------------------------------- device-level interface
  * The pieces rm_render_tiled is made of, for hosts that own the device memory,
  * the stream and the cross-GPU exchange themselves (one process per GPU with
@@ -341,6 +367,16 @@ int rm_renderer_read_frame(rm_renderer* r, size_t sample_count, rm_vec3* out_hos
  * accumulator: p = sum / sample_count; 1 - exp(p * -1.0 * exposure); powf(1 / gamma); * 255; cast::<u8>() — a pixel
  * with a NaN / out-of-range channel stays (0, 0, 0).  Writes W*H*3 bytes, row-major RGB, to HOST memory. */
 int rm_renderer_read_rgb8(rm_renderer* r, size_t sample_count, double exposure, double gamma, uint8_t* out_host);
+/* D2H of the running sums of squared samples Q (RM_FLAG_MOMENTS), row-major W*H; RM_ERR_STATE without the flag. */
+int rm_renderer_read_moments(rm_renderer* r, rm_vec3* out_host);
+/* E_t (defined above rm_adaptive_settings) of every tile after `sample_count` samples, computed on the device from this renderer's S and
+ * Q, in rm_tile_layout order; tiles outside the renderer's share (RM_PARTITION_TILES) are NaN.  Writes min(count, capacity)
+ * values and returns the tile count (0 on failure, with rm_last_error set).  Needs RM_FLAG_MOMENTS. */
+size_t rm_renderer_tile_errors(rm_renderer* r, size_t sample_count, double* out, size_t capacity);
+/* Later rm_renderer_render calls render only the tiles of the renderer's share whose `active` entry (rm_tile_layout order,
+ * `tile_count` = the layout's count) is non-zero; the sums of the other tiles are left untouched.  NULL = every tile.
+ * Asynchronous on the renderer's stream. */
+int rm_renderer_set_active_tiles(rm_renderer* r, const uint8_t* active, size_t tile_count);
 int rm_renderer_stats(rm_renderer* r, rm_stats* out);
 
 /* Per-stage breakdown of the wavefront.  Slot d (1 <= d < RM_STAGE_SLOTS) is the stage that traces

@@ -53,6 +53,7 @@ FLAG_COUNT_WORK = 4
 FLAG_NO_RAY_BINNING = 8     # 8, 16, 32: reserved values, accepted with no effect
 FLAG_FUSE_SETUP = 16
 FLAG_SPLIT_SETUP = 32
+FLAG_MOMENTS = 64           # keep the running sums of squared samples next to the sums (Renderer.read_moments / tile_errors)
 PRECISION_F64 = 0
 PRECISION_F32_SHADING = 1
 STAGE_SLOTS = 16
@@ -89,6 +90,10 @@ class GpuOptionsC(C.Structure):
     _fields_ = [("device", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("partition", C.c_uint32), ("seed", C.c_uint64),
                 ("stream", C.c_void_p), ("accum_device", C.c_void_p), ("batch_spp", C.c_size_t), ("flags", C.c_uint32), ("device_count", C.c_uint32),
                 ("device_list", C.POINTER(C.c_int32)), ("precision", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class AdaptiveSettingsC(C.Structure):
+    _fields_ = [("threshold", C.c_double), ("min_samples", C.c_size_t)]
 
 
 class TileC(C.Structure):
@@ -137,6 +142,7 @@ ABI_SYMBOLS = [
     "rm_renderer_accum_device", "rm_renderer_clear", "rm_renderer_sync", "rm_renderer_read_sums", "rm_renderer_read_frame",
     "rm_renderer_stats", "rm_renderer_stage_stats", "rm_renderer_destroy", "rm_tile_layout", "rm_renderer_read_rgb8", "rm_tonemap_rgb8",
     "rm_write_png", "rm_project_load_scene", "rm_message_to_json", "rm_release_cached_memory", "rm_measure_fp64_rate",
+    "rm_render_tiled_adaptive", "rm_renderer_read_moments", "rm_renderer_tile_errors", "rm_renderer_set_active_tiles",
 ]
 
 _lib = None
@@ -178,6 +184,10 @@ def lib():
         "rm_scene_intersect": (i32, [vp, i32, vp, sz, vp, vp, vp]),
         "rm_tile_free": (None, [P(TileC)]),
         "rm_render_tiled": (vp, [vp, P(SettingsC), P(GpuOptionsC)]),
+        "rm_render_tiled_adaptive": (vp, [vp, P(SettingsC), P(GpuOptionsC), P(AdaptiveSettingsC)]),
+        "rm_renderer_read_moments": (i32, [vp, vp]),
+        "rm_renderer_tile_errors": (sz, [vp, sz, vp, sz]),
+        "rm_renderer_set_active_tiles": (i32, [vp, vp, sz]),
         "rm_task_poll": (i32, [vp, P(MessageC)]),
         "rm_task_await": (i32, [vp, vp]),
         "rm_task_set_callback": (i32, [vp, TILE_CALLBACK, vp]),
@@ -612,11 +622,28 @@ class TaskHandle:
             self._h = None
 
 
-def render_tiled(scene: Scene, settings: Settings, options: Optional[GpuOptions] = None) -> TaskHandle:
-    """render_tiled(scene, settings) -> TaskHandle (src/trace.rs:137-230). Returns immediately."""
+@dataclass
+class AdaptiveSettings:
+    """rm_adaptive_settings: a tile stops at the first checkpoint n >= max(min_samples, 2) where its error estimate E_t
+    (include/raymond.h) is <= threshold, and is delivered as TileFinished(sample_count = n)."""
+    threshold: float
+    min_samples: int = 0
+
+    def _c(self) -> AdaptiveSettingsC:
+        return AdaptiveSettingsC(float(self.threshold), int(self.min_samples))
+
+
+def render_tiled(scene: Scene, settings: Settings, options: Optional[GpuOptions] = None,
+                 adaptive: Optional[AdaptiveSettings] = None) -> TaskHandle:
+    """render_tiled(scene, settings) -> TaskHandle (src/trace.rs:137-230). Returns immediately.  `adaptive` adds per-tile early
+    stopping at the samples_per_iteration checkpoints (rm_render_tiled_adaptive); read such a task with poll() or await_()."""
     s = settings._c()
     o = (options or GpuOptions())._c()
-    h = _require(lib().rm_render_tiled(scene._h, C.byref(s), C.byref(o)), "render_tiled")
+    if adaptive is None:
+        h = _require(lib().rm_render_tiled(scene._h, C.byref(s), C.byref(o)), "render_tiled")
+    else:
+        a = adaptive._c()
+        h = _require(lib().rm_render_tiled_adaptive(scene._h, C.byref(s), C.byref(o), C.byref(a)), "render_tiled_adaptive")
     return TaskHandle(h, settings)
 
 
@@ -711,6 +738,28 @@ class Renderer:
         out = self._frame() if out is None else out
         _check(lib().rm_renderer_read_frame(self._h, sample_count, _ptr(out)))
         return out
+
+    def read_moments(self, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """Running sums of squared samples (FLAG_MOMENTS), (H, W, 3) f64."""
+        out = self._frame() if out is None else out
+        _check(lib().rm_renderer_read_moments(self._h, _ptr(out)))
+        return out
+
+    def tile_errors(self, sample_count: int) -> np.ndarray:
+        """E_t of every tile after `sample_count` samples, in tile_layout order; NaN for tiles of other shares (FLAG_MOMENTS)."""
+        n = len(tile_layout(self.settings))
+        out = np.zeros(max(n, 1))
+        if lib().rm_renderer_tile_errors(self._h, sample_count, _ptr(out), n) != n:
+            raise RaymondError(lib().rm_last_status(), last_error())
+        return out[:n]
+
+    def set_active_tiles(self, mask: Optional[Sequence[bool]]) -> None:
+        """Later render() calls render only the tiles whose entry (tile_layout order) is true; None = every tile."""
+        if mask is None:
+            _check(lib().rm_renderer_set_active_tiles(self._h, None, 0))
+            return
+        m = np.ascontiguousarray(np.asarray(mask, dtype=bool).astype(np.uint8))
+        _check(lib().rm_renderer_set_active_tiles(self._h, _ptr(m), m.size))
 
     def read_rgb8(self, sample_count: int, exposure: float = 1.0, gamma: float = 2.2) -> np.ndarray:
         """sum / sample_count -> cli_old's tonemap (src cli_old/src/main.rs:157-181) on the GPU -> (H, W, 3) uint8."""

@@ -725,6 +725,10 @@ struct rm_renderer {
     double* accum = nullptr;
     bool owns_accum = false;
     size_t accum_bytes = 0;
+    double* moments = nullptr;                      // RM_FLAG_MOMENTS: W*H rm_vec3 running sums of squares (peers read it in place)
+    unsigned* active_map = nullptr;                 // rm_renderer_set_active_tiles: the active tiles' runs of the pixel map
+    uint3* active_runs = nullptr;                   // ... and the {source, destination, length} list that gathered them
+    size_t full_batch_spp = 1;                      // batch_spp for the whole share
     DevTotals* totals = nullptr;
     size_t batch_spp = 1;
     uint64_t launches = 0;
@@ -748,6 +752,8 @@ struct rm_renderer {
         dev_free(queue_mem); dev_free(id_mem); dev_free(rp.contrib); dev_free(counters); dev_free(totals);
         isect.release();
         if (owns_accum) visible_release(device, accum_bytes, accum);
+        if (moments) visible_release(device, accum_bytes, moments);
+        dev_free(active_map); dev_free(active_runs);
         if (owns_stream && stream) cudaStreamDestroy(stream);
         if (owns_scene) delete ds;
     }
@@ -864,7 +870,7 @@ static int renderer_init(rm_renderer* r) {
         spp = std::min<size_t>(spp, own);
     }
     while (spp > 1 && spp * npix >= 0xffffffffull) spp--;
-    r->batch_spp = spp;
+    r->batch_spp = r->full_batch_spp = spp;
     const size_t cap = std::max<size_t>(npix * spp, 32);
 
     RM_CUDA(dev_malloc(&r->queue_mem, cap * 9 * 2 * sizeof(double)));
@@ -891,13 +897,17 @@ static int renderer_init(rm_renderer* r) {
     RM_CUDA(dev_malloc(&r->totals, sizeof(DevTotals)));
     rp.totals = r->totals;
     RM_CUDA(cudaMemsetAsync(r->totals, 0, sizeof(DevTotals), r->stream));
+    r->accum_bytes = std::max<size_t>(W * H, 1) * 3 * sizeof(double);
     if (r->opt.accum_device) r->accum = (double*)r->opt.accum_device;
     else {      // not from the pool: peers read it in place
-        r->accum_bytes = std::max<size_t>(W * H, 1) * 3 * sizeof(double);
         RM_CUDA(visible_acquire(r->device, r->accum_bytes, (void**)&r->accum));
         r->owns_accum = true;
     }
     RM_CUDA(cudaMemsetAsync(r->accum, 0, W * H * 3 * sizeof(double), r->stream));
+    if (r->opt.flags & RM_FLAG_MOMENTS) {
+        RM_CUDA(visible_acquire(r->device, r->accum_bytes, (void**)&r->moments));
+        RM_CUDA(cudaMemsetAsync(r->moments, 0, W * H * 3 * sizeof(double), r->stream));
+    }
     trace.mark("renderer_init: queues, counters, accumulator allocated");
     return RM_OK;
 }
@@ -974,7 +984,9 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
     {
         StageHook hook(r, 0);
         hook.begin(3);
-        k_accumulate<<<(rp.n_pixels + kBlock - 1) / kBlock, kBlock, 0, r->stream>>>(rp, r->accum, n_samples, keep ? 1u : 0u);
+        const unsigned blocks = (rp.n_pixels + kBlock - 1) / kBlock;
+        if (r->moments) k_accumulate<true><<<blocks, kBlock, 0, r->stream>>>(rp, r->accum, n_samples, keep ? 1u : 0u, r->moments);
+        else k_accumulate<false><<<blocks, kBlock, 0, r->stream>>>(rp, r->accum, n_samples, keep ? 1u : 0u, nullptr);
         hook.end(3);
     }
     RM_CUDA(cudaGetLastError());
@@ -1016,7 +1028,6 @@ __global__ void __launch_bounds__(256) k_add(double* __restrict__ total, const d
 // "total += part" chain, so the frame does not depend on which device sums which slice) and written straight into the
 // pinned host frame the tile messages are sliced from.  Every device runs this on its own slice: reduce-scatter over
 // peer memory + the D2H of the result over that device's own PCIe link, no staging copy, no gather onto one device.
-constexpr int kMaxShares = 64;
 struct SharePointers {
     const double* acc[kMaxShares];
     int count;
@@ -1120,6 +1131,77 @@ static int reduce_gather_to_host(rm_renderer* const* rs, int count, rm_vec3* out
     dev_free(part);
     if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("accumulator reduce: ") + cudaGetErrorString(e));
     return RM_OK;
+}
+
+// E_t (include/raymond.h) of tiles first, first + step, ... of the layout after `n` samples, from the sums listed in `sm`,
+// on r's stream, into out_dev[tile].
+static int launch_tile_error(rm_renderer* r, const ShareMoments& sm, double* out_dev, size_t n_tiles, size_t first, size_t step, double n) {
+    if (first >= n_tiles) return RM_OK;
+    const rm_settings& s = r->settings;
+    const size_t W = s.camera_settings.backbuffer_width, H = s.camera_settings.backbuffer_height;
+    const unsigned blocks = (unsigned)((n_tiles - first + step - 1) / step);
+    RM_CUDA(cudaSetDevice(r->device));
+    k_tile_error<<<blocks, kTileErrorBlock, 0, r->stream>>>(sm, out_dev, (unsigned)W, (unsigned)H, (unsigned)std::min(s.tile_size[0], W),
+                                                             (unsigned)std::min(s.tile_size[1], H), (unsigned)first, (unsigned)step, n);
+    r->launches++;
+    RM_CUDA(cudaGetLastError());
+    return RM_OK;
+}
+
+int tile_errors_to_host(rm_renderer* const* rs, int count, size_t n, double* out_pinned, size_t n_tiles) {
+    if (count <= 0 || !rs || !out_pinned) return fail(RM_ERR_INVALID_ARGUMENT, "tile_errors_to_host: bad argument");
+    for (int g = 0; g < count; g++) {
+        if (!rs[g]->moments) return fail(RM_ERR_STATE, "tile errors need RM_FLAG_MOMENTS");
+        RM_CUDA(cudaSetDevice(rs[g]->device));
+        RM_CUDA(cudaStreamSynchronize(rs[g]->stream));      // every share's sums are complete before any device reads them
+    }
+    double* out_dev = nullptr;
+    RM_CUDA(cudaHostGetDevicePointer((void**)&out_dev, (void*)out_pinned, 0));
+    rm_renderer* r0 = rs[0];
+    bool peers = count <= kMaxShares;
+    for (int g = 0; g < count && peers; g++)
+        for (int j = 0; j < count && peers; j++) peers = enable_peer(rs[g]->device, rs[j]->device);
+    if (count == 1 || peers) {
+        // every device sums the shares in place (peer reads, in device order) for tiles g, g + count, ...
+        ShareMoments sm{};
+        sm.count = count;
+        for (int g = 0; g < count; g++) { sm.acc[g] = rs[g]->accum; sm.mom[g] = rs[g]->moments; }
+        for (int g = 0; g < count; g++)
+            if (int st = launch_tile_error(rs[g], sm, out_dev, n_tiles, (size_t)g, (size_t)count, (double)n)) return st;
+        for (int g = 0; g < count; g++) {
+            RM_CUDA(cudaSetDevice(rs[g]->device));
+            RM_CUDA(cudaStreamSynchronize(rs[g]->stream));
+        }
+        return RM_OK;
+    }
+    // no peer mapping: the staged fallback of the accumulator exchange — S and Q summed onto the first device in renderer order
+    const size_t len = r0->settings.camera_settings.backbuffer_width * r0->settings.camera_settings.backbuffer_height * 3;
+    RM_CUDA(cudaSetDevice(r0->device));
+    double *S = nullptr, *Q = nullptr, *part = nullptr;
+    cudaError_t e = dev_malloc(&S, len * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&Q, len * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&part, len * sizeof(double));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(S, r0->accum, len * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(Q, r0->moments, len * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
+    const unsigned blocks = (unsigned)std::min<size_t>((len + 255) / 256, (size_t)r0->sms * 16);
+    for (int g = 1; g < count && e == cudaSuccess; g++) {
+        e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->accum, rs[g]->device, len * sizeof(double), r0->stream);
+        if (e == cudaSuccess) { k_add<<<blocks, 256, 0, r0->stream>>>(S, part, len); r0->launches++; e = cudaGetLastError(); }
+        if (e == cudaSuccess) e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->moments, rs[g]->device, len * sizeof(double), r0->stream);
+        if (e == cudaSuccess) { k_add<<<blocks, 256, 0, r0->stream>>>(Q, part, len); r0->launches++; e = cudaGetLastError(); }
+    }
+    int st = RM_OK;
+    if (e == cudaSuccess) {
+        ShareMoments sm{};
+        sm.count = 1;
+        sm.acc[0] = S;
+        sm.mom[0] = Q;
+        st = launch_tile_error(r0, sm, out_dev, n_tiles, 0, 1, (double)n);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(r0->stream);
+    dev_free(S); dev_free(Q); dev_free(part);
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("tile errors: ") + cudaGetErrorString(e));
+    return st;
 }
 
 }  // namespace rm
@@ -1298,6 +1380,7 @@ int rm_renderer_clear(rm_renderer* r) {
     RM_CUDA(cudaSetDevice(r->device));
     const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height * 3;
     RM_CUDA(cudaMemsetAsync(r->accum, 0, n * sizeof(double), r->stream));   // statistics stay cumulative
+    if (r->moments) RM_CUDA(cudaMemsetAsync(r->moments, 0, n * sizeof(double), r->stream));
     return RM_OK;
 }
 
@@ -1311,11 +1394,11 @@ int rm_renderer_sync(rm_renderer* r) {
 
 // The accumulator to (pageable) caller memory: D2H at link speed into a cached pinned block, then a few host threads move
 // it on, dividing by `divisor` on the way (tile.data[..] / tile.sample_count as f64, src/trace.rs:95) when it is not 0.
-static int read_accumulator(rm_renderer* r, rm_vec3* out, double divisor) {
+static int read_accumulator(rm_renderer* r, rm_vec3* out, double divisor, const double* source = nullptr) {
     RM_CUDA(cudaSetDevice(r->device));
     const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height;
     rm_vec3* pin = (rm_vec3*)pinned_acquire(std::max<size_t>(n, 1) * sizeof(rm_vec3));
-    cudaError_t e = cudaMemcpyAsync(pin ? pin : out, r->accum, n * sizeof(rm_vec3), cudaMemcpyDeviceToHost, r->stream);
+    cudaError_t e = cudaMemcpyAsync(pin ? pin : out, source ? source : r->accum, n * sizeof(rm_vec3), cudaMemcpyDeviceToHost, r->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(r->stream);
     if (e != cudaSuccess) {
         pinned_release(pin);
@@ -1370,6 +1453,82 @@ int rm_renderer_read_rgb8(rm_renderer* r, size_t sample_count, double exposure, 
     dev_free(d_out);
     harvest_events(r);
     return st;
+}
+
+int rm_renderer_read_moments(rm_renderer* r, rm_vec3* out) {
+    if (!r || !out) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_moments: null argument");
+    if (!r->moments) return fail(RM_ERR_STATE, "rm_renderer_read_moments: the renderer was created without RM_FLAG_MOMENTS");
+    return read_accumulator(r, out, 0.0, r->moments);
+}
+
+size_t rm_renderer_tile_errors(rm_renderer* r, size_t sample_count, double* out, size_t capacity) {
+    if (!r) { fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_tile_errors: null renderer"); return 0; }
+    if (!r->moments) { fail(RM_ERR_STATE, "rm_renderer_tile_errors: the renderer was created without RM_FLAG_MOMENTS"); return 0; }
+    if (sample_count < 2) { fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_tile_errors: the estimate needs sample_count >= 2"); return 0; }
+    const rm_settings& s = r->settings;
+    const size_t n_tiles = tile_layout(s.camera_settings.backbuffer_width, s.camera_settings.backbuffer_height, s.tile_size[0], s.tile_size[1]).size();
+    double* pin = (double*)pinned_acquire(std::max<size_t>(n_tiles, 1) * sizeof(double));
+    if (!pin) { fail(RM_ERR_OUT_OF_MEMORY, "rm_renderer_tile_errors: cannot pin the result block"); return 0; }
+    for (size_t t = 0; t < n_tiles; t++) pin[t] = NAN;           // tiles of other shares stay NaN
+    const bool tiles = r->opt.partition == RM_PARTITION_TILES && r->opt.world_size > 1;
+    int st = RM_OK;
+    if (tiles) {
+        ShareMoments sm{};
+        sm.count = 1; sm.acc[0] = r->accum; sm.mom[0] = r->moments;
+        double* out_dev = nullptr;
+        if (cudaSetDevice(r->device) != cudaSuccess || cudaHostGetDevicePointer((void**)&out_dev, (void*)pin, 0) != cudaSuccess)
+            st = fail(RM_ERR_CUDA, "rm_renderer_tile_errors: no device view of the result block");
+        if (st == RM_OK) st = launch_tile_error(r, sm, out_dev, n_tiles, (size_t)r->opt.rank, (size_t)r->opt.world_size, (double)sample_count);
+        if (st == RM_OK && cudaStreamSynchronize(r->stream) != cudaSuccess) st = fail(RM_ERR_CUDA, "rm_renderer_tile_errors: kernel failed");
+    } else {
+        st = tile_errors_to_host(&r, 1, sample_count, pin, n_tiles);
+    }
+    if (st == RM_OK && out) memcpy(out, pin, std::min(n_tiles, capacity) * sizeof(double));
+    pinned_release(pin);
+    return st == RM_OK ? n_tiles : 0;
+}
+
+int rm_renderer_set_active_tiles(rm_renderer* r, const uint8_t* active, size_t tile_count) {
+    if (!r) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_set_active_tiles: null renderer");
+    const rm_settings& s = r->settings;
+    const std::vector<TileRect> layout = tile_layout(s.camera_settings.backbuffer_width, s.camera_settings.backbuffer_height, s.tile_size[0], s.tile_size[1]);
+    if (active && tile_count != layout.size())
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_set_active_tiles: tile_count is not the tile count of the layout");
+    RM_CUDA(cudaSetDevice(r->device));
+    // the share's pixel map holds its tiles in queue order, each as one contiguous run (build_pixel_map)
+    const int world = r->opt.world_size > 1 ? r->opt.world_size : 1;
+    const bool tiles = r->opt.partition == RM_PARTITION_TILES && world > 1;
+    std::vector<uint3> runs;
+    size_t src = 0, n_active = 0, owned = 0;
+    for (size_t t = 0; t < layout.size(); t++) {
+        if (tiles && (int)(t % (size_t)world) != r->opt.rank) continue;
+        const size_t len = layout[t].width * layout[t].height;
+        if (active && active[t]) { runs.push_back(make_uint3((unsigned)src, (unsigned)n_active, (unsigned)len)); n_active += len; }
+        src += len;
+        owned++;
+    }
+    if (!active || runs.size() == owned) {          // the whole share: the shared map, as created
+        r->rp.pixel_map = r->pixel_map;
+        r->rp.n_pixels = (unsigned)r->pixel_map_ref->n;
+        r->batch_spp = r->full_batch_spp;
+        return RM_OK;
+    }
+    // never written to the cached shared map: the renderer gets its own compacted copy of the active runs
+    if (!r->active_map) RM_CUDA(dev_malloc(&r->active_map, std::max<size_t>(r->pixel_map_ref->n, 1) * sizeof(unsigned)));
+    if (!r->active_runs) RM_CUDA(dev_malloc(&r->active_runs, std::max<size_t>(owned, 1) * sizeof(uint3)));
+    if (!runs.empty()) {
+        RM_CUDA(cudaMemcpyAsync(r->active_runs, runs.data(), runs.size() * sizeof(uint3), cudaMemcpyHostToDevice, r->stream));
+        k_gather_pixels<<<(unsigned)runs.size(), kBlock, 0, r->stream>>>(r->pixel_map, r->active_runs, r->active_map);
+        r->launches++;
+        RM_CUDA(cudaGetLastError());
+    }
+    r->rp.pixel_map = r->active_map;
+    r->rp.n_pixels = (unsigned)n_active;
+    // as many samples per batch as the queues hold for the active pixels (rm_renderer_render cuts a batch at the range's end)
+    size_t spp = n_active ? std::max<size_t>(1, (size_t)r->rp.cap / n_active) : r->full_batch_spp;
+    while (spp > 1 && spp * n_active >= 0xffffffffull) spp--;
+    r->batch_spp = spp;
+    return RM_OK;
 }
 
 int rm_renderer_stats(rm_renderer* r, rm_stats* out) {

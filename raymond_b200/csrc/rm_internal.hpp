@@ -90,6 +90,10 @@ std::vector<TileRect> tile_layout(size_t W, size_t H, size_t tw, size_t th);
 // the exchange) and sets *mean_written; the other paths leave it alone.
 int reduce_accumulators_to_host(rm_renderer* const* renderers, int count, rm_vec3* out, bool out_is_pinned, rm_vec3* mean_pinned = nullptr,
                                 double divisor = 1.0, bool* mean_written = nullptr);
+// E_t (include/raymond.h) of every tile after `n` samples from the S and Q summed over the renderers (RM_FLAG_MOMENTS) in
+// renderer order, into `out_pinned` (a pinned_acquire block of n_tiles doubles).  Device g computes tiles g, g + count, ...
+// reading its peers' sums in place; without peer mappings the sums are staged onto the first device.  Synchronous.
+int tile_errors_to_host(rm_renderer* const* renderers, int count, size_t n, double* out_pinned, size_t n_tiles);
 // display transform kernel (rm_display.cu): sums / divisor -> tonemap -> 8-bit RGB, device pointers
 int tonemap_device(const double* sums_device, size_t n_pixels, double divisor, double exposure, double gamma, unsigned char* out_device, void* stream);
 int dev_alloc(void** p, size_t bytes);

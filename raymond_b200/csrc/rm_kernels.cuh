@@ -1257,23 +1257,31 @@ __global__ void __launch_bounds__(kBlock, RM_SHADE_BLOCKS_PER_SM) k_shade(const 
 // tile.data[..] += sample, one pass after the other          src/trace.rs:203
 // Adds the batch's per-path radiance to the running sums in global sample order, so the
 // association is the reference's ((0 + s0) + s1) + ...  Non-finite samples are dropped and counted
-// unless RM_FLAG_KEEP_NONFINITE.
+// unless RM_FLAG_KEEP_NONFINITE.  MOMENTS (RM_FLAG_MOMENTS): the same samples' squares go into `moments`, in the same order.
+// `moments` is the last parameter so that the default instantiation keeps the parameter layout (and the code) it always had.
+template <bool MOMENTS>
 __global__ void __launch_bounds__(kBlock) k_accumulate(const __grid_constant__ RenderParams rp, double* __restrict__ accum,
-                                                        const unsigned n_batch_samples, const unsigned keep_nonfinite) {
+                                                        const unsigned n_batch_samples, const unsigned keep_nonfinite, double* __restrict__ moments) {
     DevTotals* totals = rp.totals;
     const unsigned q = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned bad = 0;
     if (q < rp.n_pixels) {
         const size_t p = (size_t)rp.pixel_map[q] * 3;
         double sx = accum[p], sy = accum[p + 1], sz = accum[p + 2];
+        double qx = 0.0, qy = 0.0, qz = 0.0;
+        if (MOMENTS) { qx = moments[p]; qy = moments[p + 1]; qz = moments[p + 2]; }
         for (unsigned s = 0; s < n_batch_samples; s++) {
             const size_t k = (size_t)s * rp.n_pixels + q;
             const double cx = rp.contrib[k], cy = rp.contrib[(size_t)rp.cap + k], cz = rp.contrib[2 * (size_t)rp.cap + k];
             const bool finite = isfinite(cx) && isfinite(cy) && isfinite(cz);
             if (!finite) bad++;
-            if (finite || keep_nonfinite) { sx += cx; sy += cy; sz += cz; }
+            if (finite || keep_nonfinite) {
+                sx += cx; sy += cy; sz += cz;
+                if (MOMENTS) { qx += cx * cx; qy += cy * cy; qz += cz * cz; }
+            }
         }
         accum[p] = sx; accum[p + 1] = sy; accum[p + 2] = sz;
+        if (MOMENTS) { moments[p] = qx; moments[p + 1] = qy; moments[p + 2] = qz; }
     }
     bad = __reduce_add_sync(0xffffffffu, bad);
     if ((threadIdx.x & 31u) == 0 && bad) atomicAdd(&totals->nonfinite, (unsigned long long)bad);
@@ -1284,6 +1292,56 @@ __global__ void __launch_bounds__(kBlock) k_accumulate(const __grid_constant__ R
         totals->rays += rp.bounce_limit ? rays : 0ull;
         totals->samples += (unsigned long long)n_batch_samples * rp.n_pixels;
     }
+}
+
+// Sums of several renderers' accumulators (and second moments), read in place in device order like the accumulator exchange.
+constexpr int kMaxShares = 64;
+struct ShareMoments {
+    const double* acc[kMaxShares];
+    const double* mom[kMaxShares];
+    int count;
+};
+
+// E_t of one tile per block (include/raymond.h, rm_adaptive_settings): tile `first + blockIdx.x * step` of the layout, the
+// tiles in the reference's column-major order.  Every thread sums r_p^2 over a fixed stride of the tile's pixels, then a fixed
+// tree in shared memory: the result does not depend on scheduling.  max(x, 0) keeps a NaN (a NaN tile never converges).
+constexpr int kTileErrorBlock = 256;
+__global__ void __launch_bounds__(kTileErrorBlock) k_tile_error(const __grid_constant__ ShareMoments sm, double* __restrict__ out, unsigned W, unsigned H,
+                                                                 unsigned tw, unsigned th, unsigned first, unsigned step, double n) {
+    __shared__ double part[kTileErrorBlock];
+    const unsigned t = first + blockIdx.x * step;
+    const unsigned tiles_y = (H + th - 1) / th;
+    const unsigned left = (t / tiles_y) * tw, top = (t % tiles_y) * th;
+    const unsigned w = min(tw, W - left), h = min(th, H - top);
+    double acc = 0.0;
+    for (unsigned k = threadIdx.x; k < w * h; k += kTileErrorBlock) {
+        const size_t p = ((size_t)(top + k / w) * W + left + k % w) * 3;
+        double se2 = 0.0, msum = 0.0;
+        for (int c = 0; c < 3; c++) {
+            double S = sm.acc[0][p + c], Q = sm.mom[0][p + c];
+            for (int j = 1; j < sm.count; j++) { S += sm.acc[j][p + c]; Q += sm.mom[j][p + c]; }
+            const double m = S / n;
+            const double d = Q - S * m;
+            const double v = (d < 0.0 ? 0.0 : d) / (n - 1.0);
+            se2 += v / n;
+            msum += m;
+        }
+        const double r = sqrt(se2) / (msum + 1e-3);
+        acc += r * r;
+    }
+    part[threadIdx.x] = acc;
+    __syncthreads();
+    for (unsigned half = kTileErrorBlock / 2; half > 0; half >>= 1) {
+        if (threadIdx.x < half) part[threadIdx.x] += part[threadIdx.x + half];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) out[t] = sqrt(part[0] / (double)(w * h));
+}
+
+// Active-tile compaction: entry i = {source offset, destination offset, length} copies one tile's run of the full pixel map.
+__global__ void __launch_bounds__(kBlock) k_gather_pixels(const unsigned* __restrict__ src, const uint3* __restrict__ runs, unsigned* __restrict__ dst) {
+    const uint3 e = runs[blockIdx.x];
+    for (unsigned k = threadIdx.x; k < e.z; k += blockDim.x) dst[e.y + k] = src[e.x + k];
 }
 
 // Hit records -> the caller's Scene::intersect outputs (distance left untouched on a miss).

@@ -3,6 +3,8 @@
 // tiles from a queue and send Tile messages over an mpsc channel; here one driver thread per
 // task feeds the GPU and posts the same messages into a single-consumer queue.
 
+#include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 
@@ -47,6 +49,8 @@ struct rm_task {
     rm_stats stats{};
     rm_tile_callback callback = nullptr;
     void* callback_user = nullptr;
+    bool adaptive = false;          // rm_render_tiled_adaptive with settings
+    rm_adaptive_settings adaptive_settings{};
 };
 
 namespace {
@@ -88,14 +92,16 @@ bool make_tile(const PendingMessage& m, rm_tile* out) {
     return true;
 }
 
-void post_tiles(rm_task* t, uint32_t kind, size_t sample_count, const std::shared_ptr<FrameSnapshot>& frame) {
+// `kinds` (optional): one message kind per tile of the layout, 0xff = no message (a tile that finished at an earlier checkpoint)
+void post_tiles(rm_task* t, uint32_t kind, size_t sample_count, const std::shared_ptr<FrameSnapshot>& frame, const std::vector<uint8_t>* kinds = nullptr) {
     const size_t W = t->settings.camera_settings.backbuffer_width, H = t->settings.camera_settings.backbuffer_height;
     std::vector<TileRect> tiles = tile_layout(W, H, t->settings.tile_size[0], t->settings.tile_size[1]);
     const int world = t->options.world_size > 1 ? t->options.world_size : 1;
     std::deque<PendingMessage> batch;
     for (size_t i = 0; i < tiles.size(); i++) {
         if (t->options.partition == RM_PARTITION_TILES && (int)(i % (size_t)world) != t->options.rank) continue;
-        batch.push_back(PendingMessage{kind, sample_count, tiles[i], frame});
+        if (kinds && (*kinds)[i] == 0xff) continue;
+        batch.push_back(PendingMessage{kinds ? (uint32_t)(*kinds)[i] : kind, sample_count, tiles[i], frame});
     }
     std::lock_guard<std::mutex> lk(t->mu);
     for (PendingMessage& m : batch) t->messages.push_back(std::move(m));
@@ -122,13 +128,19 @@ void drive(rm_task* t) {
     const bool split_local = G > 1 && t->options.partition == RM_PARTITION_SAMPLES;
     int st = RM_OK;
     Trace trace;
+    // adaptive: which tiles still render, and at which checkpoint a tile may first stop
+    const size_t n_tiles = tile_layout(W, H, s.tile_size[0], s.tile_size[1]).size();
+    std::vector<uint8_t> active(n_tiles, 1);
+    bool stopped_early = false;
+    const size_t first_stop = std::max<size_t>(t->adaptive_settings.min_samples, 2);
+    double* errors = nullptr;
     // every checkpoint's frame of running sums lands in its own snapshot (a pinned block, cached across tasks: D2H at link
     // speed, and the messages slice their tiles straight out of it)
     try {
         // TileProgressed every `samples_per_iteration` passes (src/trace.rs:217-219)
         const size_t chunk = s.samples_per_iteration ? s.samples_per_iteration : (total ? total : 1);
         size_t done = 0;
-        while (done < total && st == RM_OK) {
+        while (done < total && st == RM_OK && std::find(active.begin(), active.end(), 1) != active.end()) {
             const size_t n = std::min(chunk, total - done);
             if (G == 1) {
                 st = rm_renderer_render(t->renderers[0], first + done * stride, n, stride);
@@ -145,25 +157,46 @@ void drive(rm_task* t) {
             if (st == RM_OK && done < total) {
                 std::shared_ptr<FrameSnapshot> frame = new_snapshot(W, H);
                 st = reduce_accumulators_to_host(t->renderers.data(), (int)G, frame->sums, frame->pinned);
-                if (st == RM_OK) post_tiles(t, RM_TILE_PROGRESSED, done, frame);
+                if (st == RM_OK && t->adaptive && done >= first_stop) {
+                    // TileFinished(done) for every still-active tile whose E_t <= threshold (NaN never is), TileProgressed for the rest
+                    if (!errors && !(errors = (double*)pinned_acquire(std::max<size_t>(n_tiles, 1) * sizeof(double)))) throw std::bad_alloc();
+                    st = tile_errors_to_host(t->renderers.data(), (int)G, done, errors, n_tiles);
+                    std::vector<uint8_t> kinds(n_tiles, 0xff);
+                    bool changed = false;
+                    for (size_t i = 0; i < n_tiles && st == RM_OK; i++) {
+                        if (!active[i]) continue;
+                        const bool converged = errors[i] <= t->adaptive_settings.threshold;
+                        kinds[i] = converged ? RM_TILE_FINISHED : RM_TILE_PROGRESSED;
+                        if (converged) { active[i] = 0; changed = true; }
+                    }
+                    if (st == RM_OK) post_tiles(t, RM_TILE_PROGRESSED, done, frame, &kinds);
+                    for (size_t g = 0; g < G && st == RM_OK && changed; g++) st = rm_renderer_set_active_tiles(t->renderers[g], active.data(), n_tiles);
+                    stopped_early = stopped_early || changed;
+                } else if (st == RM_OK) {
+                    post_tiles(t, RM_TILE_PROGRESSED, done, frame);      // no tile stops before first_stop
+                }
             }
         }
         trace.mark("driver: all launches enqueued");
         if (st == RM_OK) {
             std::shared_ptr<FrameSnapshot> frame = new_snapshot(W, H);
             // several devices: the exchange kernel also writes the averaged frame await() hands out (the finalize, fused in)
-            if (G > 1 && frame->pinned && t->options.partition == RM_PARTITION_SAMPLES && g_snapshot_pinned_bytes.load() + frame->bytes <= kSnapshotPinnedLimit) {
+            if (G > 1 && frame->pinned && t->options.partition == RM_PARTITION_SAMPLES && !stopped_early && g_snapshot_pinned_bytes.load() + frame->bytes <= kSnapshotPinnedLimit) {
                 frame->mean = (rm_vec3*)pinned_acquire(frame->bytes);
                 if (frame->mean) g_snapshot_pinned_bytes += frame->bytes;
             }
             st = reduce_accumulators_to_host(t->renderers.data(), (int)G, frame->sums, frame->pinned, frame->mean, (double)total, &frame->has_mean);
             trace.mark("driver: devices done, accumulators summed, frame on the host");
-            if (st == RM_OK) post_tiles(t, RM_TILE_FINISHED, total, frame);      // src/trace.rs:211-212
+            if (st == RM_OK) {                                                     // src/trace.rs:211-212
+                for (uint8_t& a : active) a = a ? (uint8_t)RM_TILE_FINISHED : 0xff;
+                post_tiles(t, RM_TILE_FINISHED, total, frame, t->adaptive ? &active : nullptr);
+            }
             trace.mark("driver: TileFinished messages posted");
         }
     } catch (const std::bad_alloc&) {
         st = fail(RM_ERR_OUT_OF_MEMORY, "out of host memory in the render driver");
     }
+    pinned_release(errors);
     rm_stats stats{};
     for (size_t g = 0; g < G; g++) {
         rm_stats one{};
@@ -182,15 +215,16 @@ void drive(rm_task* t) {
     t->cv.notify_all();
 }
 
-}  // namespace
-
-extern "C" {
-
-rm_task* rm_render_tiled(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options) {
-    if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled: null argument"); return nullptr; }
+// render_tiled; `adaptive` (optional, validated by the caller) adds per-tile early stopping, for which every share keeps Q
+rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive) {
     rm_task* t = new rm_task();
     t->settings = *settings;
     if (options) t->options = *options;
+    if (adaptive) {
+        t->adaptive = true;
+        t->adaptive_settings = *adaptive;
+        t->options.flags |= RM_FLAG_MOMENTS;
+    }
     const size_t G = t->options.device_count > 1 ? t->options.device_count : 1;
     if (G > 1 && (t->options.world_size > 1 || t->options.stream || t->options.accum_device)) {
         fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled: device_count > 1 excludes world_size, stream and accum_device (they describe one device)");
@@ -275,6 +309,34 @@ rm_task* rm_render_tiled(const rm_scene* scene, const rm_settings* settings, con
     return t;
 }
 
+}  // namespace
+
+extern "C" {
+
+rm_task* rm_render_tiled(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options) {
+    if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled: null argument"); return nullptr; }
+    return create_task(scene, settings, options, nullptr);
+}
+
+rm_task* rm_render_tiled_adaptive(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive) {
+    if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: null argument"); return nullptr; }
+    if (adaptive) {
+        if (!std::isfinite(adaptive->threshold) || adaptive->threshold <= 0.0) {
+            fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: threshold must be finite and > 0");
+            return nullptr;
+        }
+        if (settings->samples_per_iteration == 0) {
+            fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: samples_per_iteration must be > 0 (it is the checkpoint cadence)");
+            return nullptr;
+        }
+        if (options && options->world_size > 1 && options->device_count <= 1) {
+            fail(RM_ERR_UNSUPPORTED, "rm_render_tiled_adaptive: one rank of a multi-process job cannot see the other ranks' sums");
+            return nullptr;
+        }
+    }
+    return create_task(scene, settings, options, adaptive);
+}
+
 int rm_task_poll(rm_task* t, rm_message* out) {
     if (!t || !out) return fail(RM_ERR_INVALID_ARGUMENT, "rm_task_poll: null argument");
     PendingMessage m;
@@ -350,6 +412,7 @@ int rm_task_set_callback(rm_task* t, rm_tile_callback callback, void* user) {
 }
 
 // async_await: hand every queued TileProgressed to the callback; stop at anything else   src/trace.rs:119-134
+// (an adaptive task's early TileFinished messages stop it too, as the reference's would)
 int rm_task_pump(rm_task* t) {
     if (!t) return fail(RM_ERR_INVALID_ARGUMENT, "rm_task_pump: null task");
     int delivered = 0;
