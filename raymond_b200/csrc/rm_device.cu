@@ -255,6 +255,7 @@ struct rm_device_scene {
     int traverse_blocks_per_sm = 2;
     DevScene scene{};
     std::vector<int> grid_objects;          // object indices with Geometry::Grid, ascending
+    bool emissive_grid = false;             // a grid object has an Emission material: its traversal can decide a last-depth path
     std::vector<void*> allocations;         // one device block per distinct grid, in DevScene::grid order
     std::vector<size_t> allocation_bytes;
     std::vector<std::shared_ptr<Grid>> keep;
@@ -469,6 +470,7 @@ static int build_scene_table(rm_device_scene* ds, const rm_scene* scene, Place p
             }
             d.grid = it->second;
             ds->grid_objects.push_back((int)i);
+            if (d.mat == RM_MATERIAL_EMISSION) ds->emissive_grid = true;
         }
     }
     return RM_OK;
@@ -731,6 +733,7 @@ struct rm_renderer {
     size_t full_batch_spp = 1;                      // batch_spp for the whole share
     DevTotals* totals = nullptr;
     size_t batch_spp = 1;
+    bool last_depth_shortcut = true;                // RM_FULL_LAST_BOUNCE unset: see renderer_batch_t
     uint64_t launches = 0;
     double device_ms = 0.0;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
@@ -843,6 +846,7 @@ static int renderer_init(rm_renderer* r) {
     if (r->opt.world_size > 1 && (r->opt.rank < 0 || r->opt.rank >= r->opt.world_size)) return fail(RM_ERR_INVALID_ARGUMENT, "rank outside world_size");
     RM_CUDA(cudaSetDevice(r->device));
     r->sms = sm_count(r->device);
+    r->last_depth_shortcut = getenv("RM_FULL_LAST_BOUNCE") == nullptr;
     if (r->opt.stream) r->stream = (cudaStream_t)r->opt.stream;
     else { RM_CUDA(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking)); r->owns_stream = true; }
 
@@ -950,6 +954,12 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
     if (n_paths == 0) return RM_OK;
     const bool count = (r->opt.flags & RM_FLAG_COUNT_WORK) != 0;
     const bool keep = (r->opt.flags & RM_FLAG_KEEP_NONFINITE) != 0;
+    // Drop mode at depth == bounce_limit: only whether the closest object is an emitter decides the path (k_shade<..., LAST>).
+    // k_setup then skips the grids for rays whose closest analytic hit is not an emitter, unless a grid emits, or the work
+    // counters must stay comparable with the reference's at every depth.  RM_FULL_LAST_BOUNCE=1 in the environment renders
+    // the last depth like every other (tests compare the two; the frame is the same to the last bit).
+    const bool last_shade = !keep && r->last_depth_shortcut;
+    const bool last_skip = last_shade && !count && !r->ds->emissive_grid;
     const unsigned persistent_grid = (unsigned)r->sms * 8u;
     RM_CUDA(cudaMemsetAsync(r->counters, 0, r->counter_slots * 3 * sizeof(unsigned), r->stream));
     if (limit == 0) RM_CUDA(cudaMemsetAsync(rp.contrib, 0, (size_t)rp.cap * 3 * sizeof(double), r->stream));   // trace() returns 0 at depth 1 > 0
@@ -959,6 +969,7 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         const Queue& qout = r->q[depth & 1];
         SetupArgs sa{};
         for (int k = 0; k < 6; k++) sa.q[k] = qin.f[k];
+        sa.emitters_only = last_skip && depth == limit ? 1 : 0;
         int st;
         if (depth == 1) {
             sa.n_ptr = nullptr; sa.n_direct = n_paths;
@@ -971,13 +982,16 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         }
         if (st != RM_OK) return st;
         hook.begin(2);
+        const bool last = last_shade && depth == limit;
         if (depth == 1) {
             const unsigned grid = std::min<unsigned>((n_paths + kBlock - 1) / kBlock, persistent_grid * 4u);
-            if (keep) k_shade<true, PREC, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
-            else k_shade<true, PREC, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            if (keep) k_shade<true, PREC, true, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            else if (last) k_shade<true, PREC, false, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            else k_shade<true, PREC, false, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
         } else {
-            if (keep) k_shade<false, PREC, true><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
-            else k_shade<false, PREC, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            if (keep) k_shade<false, PREC, true, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            else if (last) k_shade<false, PREC, false, true><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            else k_shade<false, PREC, false, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
         }
         hook.end(2);
     }

@@ -12,7 +12,9 @@
 //               to reject, and Triangle::intersects runs on the survivors with full lanes; rays with a hit finish,
 //               idle lanes re-fill from the queue in groups
 //   k_shade     one thread per ray: surface normal, material, lobe choice, BRDF weight, next ray or
-//               delivered radiance; survivors are compacted into the next stage's ray queue
+//               delivered radiance; survivors are compacted into the next stage's ray queue.  At the bounce limit in
+//               drop mode only the emitter test is left (k_shade<..., LAST>), and k_setup queues no traversal for a ray
+//               whose closest hit so far is not an emitter (SetupArgs::emitters_only)
 // followed once per batch by k_accumulate (the tile accumulator).
 // (Round 2 measured two variations of this pipeline and kept neither — profiles/r2_ab_fusion_binning_f32.log: k_shade fused with
 // the next depth's k_setup starves on instruction fetch, 4 000-5 000 SASS instructions, stall_no_instruction 6.4 per issue;
@@ -676,6 +678,7 @@ struct SetupArgs {
     unsigned* trav_count;
     int grid_object;           // object index of the grid this pass sets up, -1 = none
     int analytic;              // 1: evaluate the Sphere/Plane objects and initialise the hit record
+    int emitters_only;         // 1: the grid can only matter when the closest hit so far is an emitter (see k_setup)
 };
 
 // Stage part 1.  See the header comment.
@@ -725,7 +728,11 @@ __global__ void __launch_bounds__(kBlock, RM_SETUP_BLOCKS_PER_SM) k_setup(const 
                 best_obj = a.hit.obj[i];
                 best_t = a.hit.t[i];
             }
-            if (a.grid_object >= 0) {
+            // emitters_only (drop mode at the bounce limit, no grid object emits): the path delivers its throughput times the
+            // emission of the closest object if that is an emitter, else an exact 0 (shade()).  A non-emissive grid can only
+            // hide an emitter, so when the closest hit so far is not one, every answer of the traversal delivers the same 0.
+            const bool decided = a.emitters_only && (best_obj < 0 || sc.obj[best_obj].mat != RM_MATERIAL_EMISSION);
+            if (a.grid_object >= 0 && !decided) {
                 const DevGrid& g = sc.grid[sc.obj[a.grid_object].grid];
                 double tmin, tmax;
                 push = grid_enter(g, o, d, s, tmin, tmax);
@@ -1205,13 +1212,30 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
 // the path poisons the sample: no path is stopped for a zero throughput (D5), and a path that ends without emission delivers
 // T (*) 0 on a miss and T (*) w (*) 0 at the bounce limit instead of an exact (0, 0, 0).  The default instantiation is the
 // one the benchmark runs.
-template <bool FIRST, int PREC, bool KEEP>
+// LAST (drop mode, depth == bounce_limit): shade() ends every path there, delivering T (*) emission for an emitter hit and an
+// exact (0, 0, 0) otherwise, so this instantiation reads only the hit object, the slot and the throughput of emitter hits,
+// and forms T (*) emission with the same multiplication as the general body.  No path continues and no triangle is shaded.
+template <bool FIRST, int PREC, bool KEEP, bool LAST>
 __global__ void __launch_bounds__(kBlock, RM_SHADE_BLOCKS_PER_SM) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
                                                    const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first) {
+    static_assert(!(LAST && KEEP), "keep mode computes the last weight: it has no last-depth shortcut");
     const unsigned n = FIRST ? n_first : rp.cnt.rays[depth - 1];
     const unsigned lane = threadIdx.x & 31u;
     const unsigned warps_total = (gridDim.x * blockDim.x) >> 5;
     const unsigned warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (LAST) {
+        for (unsigned i = warp * 32u + lane; i < n; i += warps_total * 32u) {
+            const unsigned slot = FIRST ? i : qin.id[i];
+            const int ob = hit.obj[i];
+            D3 result = d3(0.0, 0.0, 0.0);
+            if (ob >= 0 && sc.obj[ob].mat == RM_MATERIAL_EMISSION)
+                result = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), ld3(sc.obj[ob].color));
+            rp.contrib[slot] = result.x;
+            rp.contrib[(size_t)rp.cap + slot] = result.y;
+            rp.contrib[2 * (size_t)rp.cap + slot] = result.z;
+        }
+        return;
+    }
     unsigned shaded_tri = 0;
     for (unsigned base = warp * 32u; base < n; base += warps_total * 32u) {
         const unsigned i = base + lane;
