@@ -8,6 +8,8 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] #[derive(Clone, Copy)] pub struct rm_vertex { pub position: rm_vec3, pub normal: rm_vec3, pub uv: rm_vec2, pub tangent: rm_vec3 }
 #[repr(C)] #[derive(Clone, Copy)] pub struct rm_triangle { pub v0: rm_vertex, pub v1: rm_vertex, pub v2: rm_vertex }   // == core::geometry::Triangle (264 B)
 #[repr(C)] #[derive(Clone, Copy)] pub struct rm_material { pub kind: u32, pub reserved: u32, pub a: rm_vec3, pub b: rm_vec3, pub p0: f64, pub p1: f64 }
+/// With `aperture_radius > 0` (depth of field), creating a renderer or task returns RM_ERR_INVALID_ARGUMENT unless
+/// `aperture_radius <= 1e150`, `position` is finite and `focal_length >= 0` (not NaN).
 #[repr(C)] #[derive(Clone, Copy)] pub struct rm_camera_settings {
     pub backbuffer_width: usize, pub backbuffer_height: usize, pub fov_vert: f64, pub position: rm_vec3,
     pub focal_length: f64, pub aperture_radius: f64 }

@@ -177,7 +177,10 @@ int rm_scene_intersect(const rm_scene* scene, int device, const rm_ray* rays, si
 /* --------------------------------------------------------------- settings */
 
 /* CameraSettings                                src/trace.rs:32-40
- * `position` is `transform.position` (Transform is position-only, src/transform.rs:4-6). */
+ * `position` is `transform.position` (Transform is position-only, src/transform.rs:4-6).
+ * With aperture_radius > 0 (depth of field), rm_renderer_create*, rm_render_tiled and rm_render_tiled_adaptive return
+ * RM_ERR_INVALID_ARGUMENT, before any device work, unless aperture_radius <= 1e150, position is finite and
+ * focal_length >= 0 (not NaN): otherwise the reference's aperture sampling never ends, or its focal-plane unwrap panics. */
 typedef struct rm_camera_settings {
     size_t backbuffer_width;
     size_t backbuffer_height;

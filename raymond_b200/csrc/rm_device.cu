@@ -1320,6 +1320,7 @@ int rm_scene_intersect(const rm_scene* scene, int device, const rm_ray* rays, si
  * multi-device task set themselves up while the scene is still being uploaded and gathered. */
 rm_renderer* rm_renderer_create_unbound(const rm_settings* settings, const rm_gpu_options* options) {
     if (!settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_create_unbound: null argument"); return nullptr; }
+    if (validate_camera(settings->camera_settings, "rm_renderer_create_unbound") != RM_OK) return nullptr;
     rm_renderer* r = new rm_renderer();
     r->settings = *settings;
     if (options) r->opt = *options;
@@ -1357,6 +1358,7 @@ rm_renderer* rm_renderer_create_on(rm_device_scene* ds, const rm_settings* setti
 
 rm_renderer* rm_renderer_create(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options) {
     if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_create: null argument"); return nullptr; }
+    if (validate_camera(settings->camera_settings, "rm_renderer_create") != RM_OK) return nullptr;   // before the scene upload
     rm_device_scene* ds = rm_device_scene_create(scene, options ? options->device : 0);
     if (!ds) return nullptr;
     rm_renderer* r = rm_renderer_create_on(ds, settings, options);

@@ -22,6 +22,20 @@ static thread_local int g_last_status = RM_OK;
 void set_error(const std::string& msg) { g_last_error = msg; if (g_last_status == RM_OK) g_last_status = RM_ERR_INVALID_ARGUMENT; }
 int fail(int status, const std::string& msg) { g_last_error = msg; g_last_status = status; return status; }
 
+// generate_primary_ray_with_dof (src/trace.rs:335-360) rejection-samples the aperture disk until a point lies strictly inside
+// it, then unwraps the focal-plane hit.  An infinite radius, one whose square overflows (dx² + dy² = ∞) or a non-finite
+// position makes every distance ∞ or NaN, so the loop never ends; a negative or NaN focal length makes the unwrap panic.
+int validate_camera(const rm_camera_settings& c, const char* who) {
+    if (!(c.aperture_radius > 0.0)) return RM_OK;   // the pinhole camera (D2)
+    if (!(c.aperture_radius <= 1e150))
+        return fail(RM_ERR_INVALID_ARGUMENT, std::string(who) + ": aperture_radius must be <= 1e150 (a larger one never finishes the aperture sampling)");
+    if (!std::isfinite(c.position.x) || !std::isfinite(c.position.y) || !std::isfinite(c.position.z))
+        return fail(RM_ERR_INVALID_ARGUMENT, std::string(who) + ": a depth-of-field camera needs a finite position");
+    if (!(c.focal_length >= 0.0))
+        return fail(RM_ERR_INVALID_ARGUMENT, std::string(who) + ": a depth-of-field camera needs focal_length >= 0 (the focal plane must be in front of it)");
+    return RM_OK;
+}
+
 // ------------------------------------------------------------------ bounds
 
 // The reference seeds its min/max folds with these odd sentinels (mesh.rs:124-125,

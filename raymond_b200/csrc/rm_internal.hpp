@@ -22,6 +22,8 @@ namespace rm {
 
 void set_error(const std::string& msg);
 int fail(int status, const std::string& msg);
+// RM_ERR_INVALID_ARGUMENT for camera settings the reference's camera could not finish or would panic on (D2, D6); no device work
+int validate_camera(const rm_camera_settings& c, const char* who);
 
 // Mesh { triangles, bounding_box }                         reference core/src/geometry/mesh.rs:10-13
 struct Mesh {

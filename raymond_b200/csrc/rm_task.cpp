@@ -315,11 +315,13 @@ extern "C" {
 
 rm_task* rm_render_tiled(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options) {
     if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled: null argument"); return nullptr; }
+    if (validate_camera(settings->camera_settings, "rm_render_tiled") != RM_OK) return nullptr;
     return create_task(scene, settings, options, nullptr);
 }
 
 rm_task* rm_render_tiled_adaptive(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive) {
     if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: null argument"); return nullptr; }
+    if (validate_camera(settings->camera_settings, "rm_render_tiled_adaptive") != RM_OK) return nullptr;
     if (adaptive) {
         if (!std::isfinite(adaptive->threshold) || adaptive->threshold <= 0.0) {
             fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: threshold must be finite and > 0");

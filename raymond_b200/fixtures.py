@@ -254,10 +254,10 @@ def random_rays(n: int, seed: int = 0xD1CE, origin_box=((-2.0, 2.0), (-1.0, 2.0)
 
 # ---------------------------------------------------------------------------- display transform
 
-def tonemap(linear: np.ndarray) -> np.ndarray:
-    """cli_old/src/main.rs:157-181: 1 - exp(-p), gamma 1/2.2, x255, truncate; out-of-range/NaN pixel stays 0."""
+def tonemap(linear: np.ndarray, exposure: float = 1.0, gamma: float = 2.2) -> np.ndarray:
+    """cli_old/src/main.rs:157-181: 1 - exp(p * -1 * exposure), ^(1 / gamma), x255, truncate; out-of-range/NaN pixel stays 0."""
     p = np.asarray(linear, dtype=np.float64)
-    with np.errstate(invalid="ignore", over="ignore"):
-        c = np.power(1.0 - np.exp(-p), 1.0 / 2.2) * 255.0
+    with np.errstate(invalid="ignore", over="ignore", divide="ignore"):
+        c = np.power(1.0 - np.exp(p * -1.0 * exposure), 1.0 / gamma) * 255.0
     ok = np.all(np.isfinite(c) & (c > -1.0) & (c < 256.0), axis=-1, keepdims=True)
     return np.where(ok, np.nan_to_num(c), 0.0).astype(np.uint8)
