@@ -30,6 +30,15 @@ static int sm_count(int device) {
     return n > 0 ? n : 148;
 }
 
+// RM_OK, or RM_ERR_CUDA when `device` is not the ordinal of a CUDA device of this process
+static int check_device(int device) {
+    int count = 0;
+    const cudaError_t e = cudaGetDeviceCount(&count);
+    if (e == cudaSuccess && device >= 0 && device < count) return RM_OK;
+    return fail(RM_ERR_CUDA, std::string("no usable CUDA device ") + std::to_string(device) + " (" + (e != cudaSuccess ? cudaGetErrorString(e) : "ordinal out of range") +
+                                 "); this library has no CPU path");
+}
+
 // ---- device memory: stream-ordered allocations from a PRIVATE pool per device (the device's default pool, which torch and
 // other libraries in the process may use, is left alone).  The pool keeps up to kPoolKeepBytes of freed memory mapped, so the
 // multi-GB wavefront queues of one render are handed to the next one instead of being unmapped and re-mapped (cudaFree /
@@ -420,99 +429,22 @@ static cudaError_t spread_spheres(const GridImage& im, void* dev, int sms, cudaS
     return cudaGetLastError();
 }
 
-// One device allocation + one H2D copy per grid.
-static int upload_grid(rm_device_scene* ds, const Grid& g, DevGrid* out) {
-    GridImage im;
-    if (int st = prepare_grid_image(g, &im)) return st;
-    void* dev = nullptr;
-    cudaError_t e = visible_acquire(ds->device, im.total, &dev);
-    if (e == cudaSuccess) {
-        ds->allocations.push_back(dev);
-        ds->allocation_bytes.push_back(im.total);
-        ds->bytes += im.host_total;                               // bytes that crossed the bus
-        e = cudaMemcpyAsync(dev, im.host, im.host_total, cudaMemcpyHostToDevice, 0);
-        if (e == cudaSuccess) e = spread_spheres(im, dev, ds->sms, 0);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(0);      // a staging block goes back to the pool on return
-    }
-    release_grid_image(im);
-    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("scene upload: ") + cudaGetErrorString(e));
-    point_grid(im, dev, out);
-    return RM_OK;
-}
-
-// Object table of the device scene (analytic objects by value, grids by index); `place(grid, out)` puts one distinct grid on the device.
-template <class Place>
-static int build_scene_table(rm_device_scene* ds, const rm_scene* scene, Place place) {
-    if (scene->objects.size() > (size_t)kMaxObjects)
-        return fail(RM_ERR_UNSUPPORTED, "scene has more than " + std::to_string(kMaxObjects) + " objects");
-    std::map<const Grid*, int> grid_index;
-    DevScene& s = ds->scene;
-    s.n_objects = (int)scene->objects.size();
-    s.n_grids = 0;
-    for (size_t i = 0; i < scene->objects.size(); i++) {
-        const Object& o = scene->objects[i];
-        DevObject& d = s.obj[i];
-        d.geom = o.geometry;
-        d.mat = (int)o.material.kind;
-        d.grid = 0;
-        d.g[0] = o.origin.x; d.g[1] = o.origin.y; d.g[2] = o.origin.z;
-        if (o.geometry == GEOM_SPHERE) { d.g[3] = o.radius; d.g[4] = d.g[5] = 0.0; }
-        else { d.g[3] = o.normal.x; d.g[4] = o.normal.y; d.g[5] = o.normal.z; }
-        d.color[0] = o.material.a.x; d.color[1] = o.material.a.y; d.color[2] = o.material.a.z;
-        d.rough = o.material.p0;
-        if (o.geometry == GEOM_GRID) {
-            auto it = grid_index.find(o.grid.get());
-            if (it == grid_index.end()) {
-                if (s.n_grids >= kMaxGrids) return fail(RM_ERR_UNSUPPORTED, "scene has more than " + std::to_string(kMaxGrids) + " distinct grids");
-                if (int st = place(o.grid, &s.grid[s.n_grids])) return st;
-                ds->keep.push_back(o.grid);
-                it = grid_index.emplace(o.grid.get(), s.n_grids++).first;
-            }
-            d.grid = it->second;
-            ds->grid_objects.push_back((int)i);
-            if (d.mat == RM_MATERIAL_EMISSION) ds->emissive_grid = true;
-        }
-    }
-    return RM_OK;
-}
-
-static void device_scene_defaults(rm_device_scene* ds) {
-    ds->sms = sm_count(ds->device);
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_traverse<false>, kTravBlock, 0) == cudaSuccess && occ > 0) ds->traverse_blocks_per_sm = occ;
-}
-
-static int build_device_scene(rm_device_scene* ds, const rm_scene* scene) {
-    RM_CUDA(cudaSetDevice(ds->device));
-    device_scene_defaults(ds);
-    cudaEvent_t e0, e1;
-    RM_CUDA(cudaEventCreate(&e0));
-    RM_CUDA(cudaEventCreate(&e1));
-    RM_CUDA(cudaEventRecord(e0, 0));
-    if (int st = build_scene_table(ds, scene, [&](const std::shared_ptr<Grid>& g, DevGrid* out) { return upload_grid(ds, *g, out); })) return st;
-    RM_CUDA(cudaEventRecord(e1, 0));
-    RM_CUDA(cudaEventSynchronize(e1));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e0, e1);
-    ds->upload_ms = ms;
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    return RM_OK;
-}
-
 }  // namespace rm
 
-// --------------------------------------------------------------------- a scene on several devices at once
+// --------------------------------------------------------------------- placing a scene on its devices
 //
-// rm_render_tiled with several shares: instead of one full upload followed by device-to-device clones, the host image of every
-// grid crosses the bus ONCE, in slices — share g copies slice g to its own device over its own PCIe link — and every share then
-// pulls the other slices from its peers over NVLink (an all-gather of the image); the per-reference spheres are spread on
-// every device locally.  One host thread per share calls rm_scene_group_join; all of them must.
+// A scene goes onto one device or onto the devices of several shares at once: the host image of every grid crosses the bus
+// ONCE, in slices — share g copies slice g to its own device over its own PCIe link — and every share then pulls the other
+// slices from its peers over NVLink (an all-gather of the image); the per-reference spheres are spread on every device
+// locally.  One host thread per share calls rm_scene_group_join; all of them must.
 struct rm_scene_group {
-    const rm_scene* scene = nullptr;
     std::vector<int> devices;
+    DevScene table{};                               // every share's object table; the grid arrays are pointed per share
+    std::vector<int> grid_objects;                  // object indices with Geometry::Grid, ascending
+    bool emissive_grid = false;
     std::vector<std::shared_ptr<Grid>> grids;       // distinct grids, in DevScene::grid order
-    std::vector<GridImage> images;
+    std::vector<GridImage> images;                  // ... and their host images
+    double flatten_ms = 0.0;                        // host time of the table and the images
     std::mutex mu;
     std::condition_variable cv;
     std::vector<std::vector<void*>> blocks;         // [share][grid]: the share's device block
@@ -535,34 +467,56 @@ struct rm_scene_group {
     }
 };
 
+// Object table of the scene (analytic objects by value, grids by index) and the host image of every distinct grid.
+static int build_scene_table(rm_scene_group* grp, const rm_scene* scene) {
+    if (scene->objects.size() > (size_t)kMaxObjects)
+        return fail(RM_ERR_UNSUPPORTED, "scene has more than " + std::to_string(kMaxObjects) + " objects");
+    std::map<const Grid*, int> grid_index;
+    DevScene& s = grp->table;
+    s.n_objects = (int)scene->objects.size();
+    s.n_grids = 0;
+    for (size_t i = 0; i < scene->objects.size(); i++) {
+        const Object& o = scene->objects[i];
+        DevObject& d = s.obj[i];
+        d.geom = o.geometry;
+        d.mat = (int)o.material.kind;
+        d.grid = 0;
+        d.g[0] = o.origin.x; d.g[1] = o.origin.y; d.g[2] = o.origin.z;
+        if (o.geometry == GEOM_SPHERE) { d.g[3] = o.radius; d.g[4] = d.g[5] = 0.0; }
+        else { d.g[3] = o.normal.x; d.g[4] = o.normal.y; d.g[5] = o.normal.z; }
+        d.color[0] = o.material.a.x; d.color[1] = o.material.a.y; d.color[2] = o.material.a.z;
+        d.rough = o.material.p0;
+        if (o.geometry == GEOM_GRID) {
+            auto it = grid_index.find(o.grid.get());
+            if (it == grid_index.end()) {
+                if (s.n_grids >= kMaxGrids) return fail(RM_ERR_UNSUPPORTED, "scene has more than " + std::to_string(kMaxGrids) + " distinct grids");
+                GridImage im;
+                if (int st = prepare_grid_image(*o.grid, &im)) return st;
+                grp->grids.push_back(o.grid);
+                grp->images.push_back(im);
+                it = grid_index.emplace(o.grid.get(), s.n_grids++).first;
+            }
+            d.grid = it->second;
+            grp->grid_objects.push_back((int)i);
+            if (d.mat == RM_MATERIAL_EMISSION) grp->emissive_grid = true;
+        }
+    }
+    return RM_OK;
+}
+
 extern "C" {
 
 rm_scene_group* rm_scene_group_create(const rm_scene* scene, const int32_t* devices, int count) {
     if (!scene || !devices || count <= 0) { fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_group_create: bad argument"); return nullptr; }
-    int visible = 0;
-    cudaError_t e = cudaGetDeviceCount(&visible);
     for (int g = 0; g < count; g++)
-        if (e != cudaSuccess || devices[g] < 0 || devices[g] >= visible) {
-            fail(RM_ERR_CUDA, std::string("no usable CUDA device ") + std::to_string(devices[g]) + " (" + (e != cudaSuccess ? cudaGetErrorString(e) : "ordinal out of range") +
-                                  "); this library has no CPU path");
-            return nullptr;
-        }
+        if (check_device(devices[g]) != RM_OK) return nullptr;
     rm_scene_group* grp = new rm_scene_group();
-    grp->scene = scene;
     grp->devices.assign(devices, devices + count);
     grp->blocks.assign((size_t)count, {});
     grp->uploaded.assign((size_t)count, nullptr);
-    // the host images of the distinct grids, in the order build_scene_table meets them (flattened once per immutable grid, cached with it)
-    for (const Object& o : scene->objects) {
-        if (o.geometry != GEOM_GRID) continue;
-        bool seen = false;
-        for (const std::shared_ptr<Grid>& g : grp->grids) seen = seen || g.get() == o.grid.get();
-        if (seen) continue;
-        GridImage im;
-        if (prepare_grid_image(*o.grid, &im) != RM_OK) { delete grp; return nullptr; }
-        grp->grids.push_back(o.grid);
-        grp->images.push_back(im);
-    }
+    const auto t0 = std::chrono::steady_clock::now();
+    if (build_scene_table(grp, scene) != RM_OK) { delete grp; return nullptr; }
+    grp->flatten_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     return grp;
 }
 
@@ -580,7 +534,12 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* grp, int share) {
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     for (int j = 0; j < G; j++) enable_peer(device, grp->devices[(size_t)j]);      // direct NVLink copies where the hardware has them
     cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) { device_scene_defaults(ds); e = cudaEventCreate(&e0); }
+    if (e == cudaSuccess) {
+        ds->sms = sm_count(device);
+        int occ = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_traverse<false>, kTravBlock, 0) == cudaSuccess && occ > 0) ds->traverse_blocks_per_sm = occ;
+        e = cudaEventCreate(&e0);
+    }
     if (e == cudaSuccess) e = cudaEventCreate(&e1);
     if (e == cudaSuccess) e = cudaEventRecord(e0, 0);
     // phase 1: my slice of every image, host -> my device
@@ -620,23 +579,21 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* grp, int share) {
     }
     // nobody frees a block a peer may still be reading
     ok = grp->barrier(1, ok && e == cudaSuccess);
-    int st = RM_OK;
     if (ok) {
-        size_t next = 0;
-        st = build_scene_table(ds, grp->scene, [&](const std::shared_ptr<Grid>&, DevGrid* out) {
-            point_grid(grp->images[next], mine[next], out);
-            next++;
-            return (int)RM_OK;
-        });
+        ds->scene = grp->table;
+        for (size_t i = 0; i < grp->images.size(); i++) point_grid(grp->images[i], mine[i], &ds->scene.grid[i]);
+        ds->grid_objects = grp->grid_objects;
+        ds->emissive_grid = grp->emissive_grid;
+        ds->keep = grp->grids;
         float ms = 0.f;
         cudaEventElapsedTime(&ms, e0, e1);
-        ds->upload_ms = ms;
+        ds->upload_ms = grp->flatten_ms + ms;
     }
     if (e0) cudaEventDestroy(e0);
     if (e1) cudaEventDestroy(e1);
-    if (!ok || st != RM_OK) {
+    if (!ok) {
         if (e != cudaSuccess) fail(RM_ERR_CUDA, std::string("scene upload (share ") + std::to_string(share) + "): " + cudaGetErrorString(e));
-        else if (st == RM_OK) fail(RM_ERR_CUDA, "scene upload failed on another device of the group");
+        else fail(RM_ERR_CUDA, "scene upload failed on another device of the group");
         delete ds;
         return nullptr;
     }
@@ -767,14 +724,13 @@ namespace rm {
 // Owned pixels in launch order: tiles in the reference's queue order (src/trace.rs:146-172),
 // restricted to this rank's share; inside a tile, 8x4 pixel blocks so that a warp covers a compact
 // screen patch (coherent primary rays walk the same grid cells).
-static std::vector<unsigned> build_pixel_map(const rm_settings& s, const rm_gpu_options& o) {
+static std::vector<unsigned> build_pixel_map(const rm_settings& s, const Share& share) {
     const size_t W = s.camera_settings.backbuffer_width, H = s.camera_settings.backbuffer_height;
     std::vector<TileRect> tiles = tile_layout(W, H, s.tile_size[0], s.tile_size[1]);
-    const int world = o.world_size > 1 ? o.world_size : 1;
     std::vector<unsigned> map;
-    map.reserve(W * H / (o.partition == RM_PARTITION_TILES ? world : 1) + 1024);
+    map.reserve(W * H / share.tile_step() + 1024);
     for (size_t t = 0; t < tiles.size(); t++) {
-        if (o.partition == RM_PARTITION_TILES && (int)(t % (size_t)world) != o.rank) continue;
+        if (!share.owns_tile(t)) continue;
         const TileRect& r = tiles[t];
         for (size_t by = 0; by < r.height; by += 4)
             for (size_t bx = 0; bx < r.width; bx += 8)
@@ -786,13 +742,13 @@ static std::vector<unsigned> build_pixel_map(const rm_settings& s, const rm_gpu_
 }
 
 // The launch order of a share's pixels depends only on the frame, the tile size and the share: it is built on the host and
-// uploaded once per (device, frame, tiles, partition, rank, world) and shared by every renderer that needs it afterwards —
+// uploaded once per (device, frame, tiles, owned tiles) and shared by every renderer that needs it afterwards —
 // render_tiled makes a renderer per frame, and 8 MB of indices per 1080p share were 5-8 ms of every frame's start.
 namespace {
 struct PixelMapKey {
-    int device; size_t W, H, tw, th; unsigned partition; int rank, world;
+    int device; size_t W, H, tw, th, first, step;
     bool operator<(const PixelMapKey& o) const {
-        return std::tie(device, W, H, tw, th, partition, rank, world) < std::tie(o.device, o.W, o.H, o.tw, o.th, o.partition, o.rank, o.world);
+        return std::tie(device, W, H, tw, th, first, step) < std::tie(o.device, o.W, o.H, o.tw, o.th, o.first, o.step);
     }
 };
 std::mutex g_pixel_map_mu;
@@ -816,14 +772,13 @@ static void pixel_map_cache_trim(size_t keep_bytes) {      // g_pixel_map_mu hel
 
 static int pixel_map_for(rm_renderer* r) {
     const rm_settings& s = r->settings;
-    const int world = r->opt.world_size > 1 ? r->opt.world_size : 1;
-    const bool tiles = r->opt.partition == RM_PARTITION_TILES && world > 1;
+    const Share share(r->opt);
     const PixelMapKey key{r->device, s.camera_settings.backbuffer_width, s.camera_settings.backbuffer_height, s.tile_size[0], s.tile_size[1],
-                          tiles ? 1u : 0u, tiles ? r->opt.rank : 0, tiles ? world : 1};
+                          share.first_tile(), share.tile_step()};
     std::lock_guard<std::mutex> lk(g_pixel_map_mu);       // also serialises the build of a missing map between the shares of a task
     auto it = g_pixel_maps.find(key);
     if (it != g_pixel_maps.end()) { r->pixel_map_ref = it->second; return RM_OK; }
-    std::vector<unsigned> map = build_pixel_map(s, r->opt);
+    std::vector<unsigned> map = build_pixel_map(s, share);
     auto pm = std::make_shared<PixelMap>();
     pm->device = r->device;
     pm->n = map.size();
@@ -869,9 +824,8 @@ static int renderer_init(rm_renderer* r) {
         spp = npix ? std::max<size_t>(1, target / npix) : 1;
         spp = std::min<size_t>(spp, 64);
         // ... and never more than this share of the job renders (a rank / device of a sample-split job gets 1 / world_size of them)
-        size_t own = std::max<size_t>(s.sample_count, 1);
-        if (r->opt.world_size > 1 && r->opt.partition == RM_PARTITION_SAMPLES) own = (own + (size_t)r->opt.world_size - 1) / (size_t)r->opt.world_size;
-        spp = std::min<size_t>(spp, own);
+        const size_t stride = Share(r->opt).sample_stride();
+        spp = std::min<size_t>(spp, (std::max<size_t>(s.sample_count, 1) + stride - 1) / stride);
     }
     while (spp > 1 && spp * npix >= 0xffffffffull) spp--;
     r->batch_spp = r->full_batch_spp = spp;
@@ -1057,7 +1011,50 @@ __global__ void __launch_bounds__(256) k_reduce_slice(const __grid_constant__ Sh
     }
 }
 
-static int reduce_gather_to_host(rm_renderer* const* rs, int count, rm_vec3* out);
+// every device of the shares reads every other's memory in place, and one kernel parameter block takes all their pointers
+static bool peers_mapped(rm_renderer* const* rs, int count) {
+    if (count > kMaxShares) return false;
+    for (int g = 0; g < count; g++)
+        for (int j = 0; j < count; j++)
+            if (!enable_peer(rs[g]->device, rs[j]->device)) return false;
+    return true;
+}
+
+// The staged exchange, for shares whose devices cannot all read each other's memory: `total` = the n doubles at `buf` of every
+// renderer summed in renderer order, with a peer copy into `part` + k_add per renderer on the first renderer's stream (both
+// buffers on its device).  Everything the other renderers enqueued is complete on entry.
+static cudaError_t stage_sum(rm_renderer* const* rs, int count, double* rm_renderer::*buf, double* total, double* part, size_t n) {
+    rm_renderer* r0 = rs[0];
+    cudaError_t e = cudaMemcpyAsync(total, r0->*buf, n * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
+    const unsigned blocks = (unsigned)std::min<size_t>((n + 255) / 256, (size_t)r0->sms * 16);
+    for (int g = 1; g < count && e == cudaSuccess; g++) {
+        e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->*buf, rs[g]->device, n * sizeof(double), r0->stream);
+        if (e == cudaSuccess) { k_add<<<blocks, 256, 0, r0->stream>>>(total, part, n); r0->launches++; e = cudaGetLastError(); }
+    }
+    return e;
+}
+
+// Fallback when the destination is pageable memory (pinning failed) or k_reduce_slice cannot read every accumulator in place:
+// the staged sum, then one D2H copy.
+static int reduce_gather_to_host(rm_renderer* const* rs, int count, rm_vec3* out) {
+    rm_renderer* r0 = rs[0];
+    const size_t n = r0->settings.camera_settings.backbuffer_width * r0->settings.camera_settings.backbuffer_height * 3;
+    for (int g = 1; g < count; g++) {            // everything the peers rendered must be complete before it is copied
+        RM_CUDA(cudaSetDevice(rs[g]->device));
+        RM_CUDA(cudaStreamSynchronize(rs[g]->stream));
+    }
+    RM_CUDA(cudaSetDevice(r0->device));
+    double *total = nullptr, *part = nullptr;
+    cudaError_t e = dev_malloc(&total, n * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&part, n * sizeof(double));
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::accum, total, part, n);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, total, n * sizeof(double), cudaMemcpyDeviceToHost, r0->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(r0->stream);
+    dev_free(total);
+    dev_free(part);
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("accumulator reduce: ") + cudaGetErrorString(e));
+    return RM_OK;
+}
 
 int reduce_accumulators_to_host(rm_renderer* const* rs, int count, rm_vec3* out, bool out_is_pinned, rm_vec3* mean_pinned, double divisor, bool* mean_written) {
     if (mean_written) *mean_written = false;
@@ -1070,11 +1067,7 @@ int reduce_accumulators_to_host(rm_renderer* const* rs, int count, rm_vec3* out,
         RM_CUDA(cudaStreamSynchronize(r0->stream));
         return RM_OK;
     }
-    if (!out_is_pinned || count > kMaxShares) return reduce_gather_to_host(rs, count, out);
-    for (int g = 0; g < count; g++)
-        for (int j = 0; j < count; j++) {
-            if (!enable_peer(rs[g]->device, rs[j]->device)) return reduce_gather_to_host(rs, count, out);   // no peer mapping: staged copies
-        }
+    if (!out_is_pinned || !peers_mapped(rs, count)) return reduce_gather_to_host(rs, count, out);
     // the frame as the devices see it (the same address under unified addressing)
     double *out_dev = nullptr, *mean_dev = nullptr;
     RM_CUDA(cudaSetDevice(r0->device));
@@ -1117,36 +1110,6 @@ int reduce_accumulators_to_host(rm_renderer* const* rs, int count, rm_vec3* out,
     return RM_OK;
 }
 
-// Fallback when the destination is pageable memory (pinning failed) or there are more shares than one kernel takes: sum onto
-// the first device with peer copies + an add kernel per peer, in renderer order, then one D2H copy.
-static int reduce_gather_to_host(rm_renderer* const* rs, int count, rm_vec3* out) {
-    rm_renderer* r0 = rs[0];
-    const size_t n = r0->settings.camera_settings.backbuffer_width * r0->settings.camera_settings.backbuffer_height * 3;
-    for (int g = 1; g < count; g++) {            // everything the peers rendered must be complete before it is copied
-        RM_CUDA(cudaSetDevice(rs[g]->device));
-        RM_CUDA(cudaStreamSynchronize(rs[g]->stream));
-    }
-    RM_CUDA(cudaSetDevice(r0->device));
-    double *total = nullptr, *part = nullptr;
-    RM_CUDA(dev_malloc(&total, n * sizeof(double)));
-    RM_CUDA(dev_malloc(&part, n * sizeof(double)));
-    cudaError_t e = cudaMemcpyAsync(total, r0->accum, n * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
-    for (int g = 1; g < count && e == cudaSuccess; g++) {
-        e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->accum, rs[g]->device, n * sizeof(double), r0->stream);
-        if (e == cudaSuccess) {
-            k_add<<<(unsigned)std::min<size_t>((n + 255) / 256, (size_t)r0->sms * 16), 256, 0, r0->stream>>>(total, part, n);
-            r0->launches++;
-            e = cudaGetLastError();
-        }
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, total, n * sizeof(double), cudaMemcpyDeviceToHost, r0->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(r0->stream);
-    dev_free(total);
-    dev_free(part);
-    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("accumulator reduce: ") + cudaGetErrorString(e));
-    return RM_OK;
-}
-
 // E_t (include/raymond.h) of tiles first, first + step, ... of the layout after `n` samples, from the sums listed in `sm`,
 // on r's stream, into out_dev[tile].
 static int launch_tile_error(rm_renderer* r, const ShareMoments& sm, double* out_dev, size_t n_tiles, size_t first, size_t step, double n) {
@@ -1162,7 +1125,7 @@ static int launch_tile_error(rm_renderer* r, const ShareMoments& sm, double* out
     return RM_OK;
 }
 
-int tile_errors_to_host(rm_renderer* const* rs, int count, size_t n, double* out_pinned, size_t n_tiles) {
+int tile_errors_to_host(rm_renderer* const* rs, int count, size_t n, double* out_pinned, size_t n_tiles, size_t first, size_t step) {
     if (count <= 0 || !rs || !out_pinned) return fail(RM_ERR_INVALID_ARGUMENT, "tile_errors_to_host: bad argument");
     for (int g = 0; g < count; g++) {
         if (!rs[g]->moments) return fail(RM_ERR_STATE, "tile errors need RM_FLAG_MOMENTS");
@@ -1172,45 +1135,35 @@ int tile_errors_to_host(rm_renderer* const* rs, int count, size_t n, double* out
     double* out_dev = nullptr;
     RM_CUDA(cudaHostGetDevicePointer((void**)&out_dev, (void*)out_pinned, 0));
     rm_renderer* r0 = rs[0];
-    bool peers = count <= kMaxShares;
-    for (int g = 0; g < count && peers; g++)
-        for (int j = 0; j < count && peers; j++) peers = enable_peer(rs[g]->device, rs[j]->device);
-    if (count == 1 || peers) {
-        // every device sums the shares in place (peer reads, in device order) for tiles g, g + count, ...
+    if (peers_mapped(rs, count)) {
+        // every device sums the shares in place (peer reads, in device order) for its tiles
         ShareMoments sm{};
         sm.count = count;
         for (int g = 0; g < count; g++) { sm.acc[g] = rs[g]->accum; sm.mom[g] = rs[g]->moments; }
         for (int g = 0; g < count; g++)
-            if (int st = launch_tile_error(rs[g], sm, out_dev, n_tiles, (size_t)g, (size_t)count, (double)n)) return st;
+            if (int st = launch_tile_error(rs[g], sm, out_dev, n_tiles, first + (size_t)g * step, (size_t)count * step, (double)n)) return st;
         for (int g = 0; g < count; g++) {
             RM_CUDA(cudaSetDevice(rs[g]->device));
             RM_CUDA(cudaStreamSynchronize(rs[g]->stream));
         }
         return RM_OK;
     }
-    // no peer mapping: the staged fallback of the accumulator exchange — S and Q summed onto the first device in renderer order
+    // no peer mapping: S and Q staged onto the first device
     const size_t len = r0->settings.camera_settings.backbuffer_width * r0->settings.camera_settings.backbuffer_height * 3;
     RM_CUDA(cudaSetDevice(r0->device));
     double *S = nullptr, *Q = nullptr, *part = nullptr;
     cudaError_t e = dev_malloc(&S, len * sizeof(double));
     if (e == cudaSuccess) e = dev_malloc(&Q, len * sizeof(double));
     if (e == cudaSuccess) e = dev_malloc(&part, len * sizeof(double));
-    if (e == cudaSuccess) e = cudaMemcpyAsync(S, r0->accum, len * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(Q, r0->moments, len * sizeof(double), cudaMemcpyDeviceToDevice, r0->stream);
-    const unsigned blocks = (unsigned)std::min<size_t>((len + 255) / 256, (size_t)r0->sms * 16);
-    for (int g = 1; g < count && e == cudaSuccess; g++) {
-        e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->accum, rs[g]->device, len * sizeof(double), r0->stream);
-        if (e == cudaSuccess) { k_add<<<blocks, 256, 0, r0->stream>>>(S, part, len); r0->launches++; e = cudaGetLastError(); }
-        if (e == cudaSuccess) e = cudaMemcpyPeerAsync(part, r0->device, rs[g]->moments, rs[g]->device, len * sizeof(double), r0->stream);
-        if (e == cudaSuccess) { k_add<<<blocks, 256, 0, r0->stream>>>(Q, part, len); r0->launches++; e = cudaGetLastError(); }
-    }
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::accum, S, part, len);
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::moments, Q, part, len);
     int st = RM_OK;
     if (e == cudaSuccess) {
         ShareMoments sm{};
         sm.count = 1;
         sm.acc[0] = S;
         sm.mom[0] = Q;
-        st = launch_tile_error(r0, sm, out_dev, n_tiles, 0, 1, (double)n);
+        st = launch_tile_error(r0, sm, out_dev, n_tiles, first, step, (double)n);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(r0->stream);
     dev_free(S); dev_free(Q); dev_free(part);
@@ -1226,16 +1179,10 @@ extern "C" {
 
 rm_device_scene* rm_device_scene_create(const rm_scene* scene, int device) {
     if (!scene) { fail(RM_ERR_INVALID_ARGUMENT, "rm_device_scene_create: null scene"); return nullptr; }
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || device < 0 || device >= count) {
-        fail(RM_ERR_CUDA, std::string("no usable CUDA device ") + std::to_string(device) + " (" + (e != cudaSuccess ? cudaGetErrorString(e) : "ordinal out of range") +
-                              "); this library has no CPU path");
-        return nullptr;
-    }
-    rm_device_scene* ds = new rm_device_scene();
-    ds->device = device;
-    if (build_device_scene(ds, scene) != RM_OK) { delete ds; return nullptr; }
+    rm_scene_group* grp = rm_scene_group_create(scene, &device, 1);
+    if (!grp) return nullptr;
+    rm_device_scene* ds = rm_scene_group_join(grp, 0);
+    rm_scene_group_destroy(grp);
     return ds;
 }
 
@@ -1326,15 +1273,7 @@ rm_renderer* rm_renderer_create_unbound(const rm_settings* settings, const rm_gp
     if (options) r->opt = *options;
     r->opt.device_list = nullptr;
     r->device = r->opt.device;
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || r->device < 0 || r->device >= count) {
-        fail(RM_ERR_CUDA, std::string("no usable CUDA device ") + std::to_string(r->device) + " (" + (e != cudaSuccess ? cudaGetErrorString(e) : "ordinal out of range") +
-                              "); this library has no CPU path");
-        delete r;
-        return nullptr;
-    }
-    if (renderer_init(r) != RM_OK) { delete r; return nullptr; }
+    if (check_device(r->device) != RM_OK || renderer_init(r) != RM_OK) { delete r; return nullptr; }
     return r;
 }
 
@@ -1486,19 +1425,8 @@ size_t rm_renderer_tile_errors(rm_renderer* r, size_t sample_count, double* out,
     double* pin = (double*)pinned_acquire(std::max<size_t>(n_tiles, 1) * sizeof(double));
     if (!pin) { fail(RM_ERR_OUT_OF_MEMORY, "rm_renderer_tile_errors: cannot pin the result block"); return 0; }
     for (size_t t = 0; t < n_tiles; t++) pin[t] = NAN;           // tiles of other shares stay NaN
-    const bool tiles = r->opt.partition == RM_PARTITION_TILES && r->opt.world_size > 1;
-    int st = RM_OK;
-    if (tiles) {
-        ShareMoments sm{};
-        sm.count = 1; sm.acc[0] = r->accum; sm.mom[0] = r->moments;
-        double* out_dev = nullptr;
-        if (cudaSetDevice(r->device) != cudaSuccess || cudaHostGetDevicePointer((void**)&out_dev, (void*)pin, 0) != cudaSuccess)
-            st = fail(RM_ERR_CUDA, "rm_renderer_tile_errors: no device view of the result block");
-        if (st == RM_OK) st = launch_tile_error(r, sm, out_dev, n_tiles, (size_t)r->opt.rank, (size_t)r->opt.world_size, (double)sample_count);
-        if (st == RM_OK && cudaStreamSynchronize(r->stream) != cudaSuccess) st = fail(RM_ERR_CUDA, "rm_renderer_tile_errors: kernel failed");
-    } else {
-        st = tile_errors_to_host(&r, 1, sample_count, pin, n_tiles);
-    }
+    const Share share(r->opt);
+    const int st = tile_errors_to_host(&r, 1, sample_count, pin, n_tiles, share.first_tile(), share.tile_step());
     if (st == RM_OK && out) memcpy(out, pin, std::min(n_tiles, capacity) * sizeof(double));
     pinned_release(pin);
     return st == RM_OK ? n_tiles : 0;
@@ -1512,12 +1440,11 @@ int rm_renderer_set_active_tiles(rm_renderer* r, const uint8_t* active, size_t t
         return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_set_active_tiles: tile_count is not the tile count of the layout");
     RM_CUDA(cudaSetDevice(r->device));
     // the share's pixel map holds its tiles in queue order, each as one contiguous run (build_pixel_map)
-    const int world = r->opt.world_size > 1 ? r->opt.world_size : 1;
-    const bool tiles = r->opt.partition == RM_PARTITION_TILES && world > 1;
+    const Share share(r->opt);
     std::vector<uint3> runs;
     size_t src = 0, n_active = 0, owned = 0;
     for (size_t t = 0; t < layout.size(); t++) {
-        if (tiles && (int)(t % (size_t)world) != r->opt.rank) continue;
+        if (!share.owns_tile(t)) continue;
         const size_t len = layout[t].width * layout[t].height;
         if (active && active[t]) { runs.push_back(make_uint3((unsigned)src, (unsigned)n_active, (unsigned)len)); n_active += len; }
         src += len;

@@ -49,7 +49,7 @@ struct Grid {
     std::vector<uint32_t> cell_start;   // n_cells + 1
     std::vector<uint32_t> references;   // triangle indices
     uint64_t n_cells() const { return resolution[0] * resolution[1] * resolution[2]; }
-    // The grid as the device wants it (upload_grid's host block), kept in pinned memory after the first upload so that
+    // The grid as the device wants it (prepare_grid_image's host image), kept in pinned memory after the first upload so that
     // every later upload of this immutable grid is one H2D copy with no flattening.  Only for images <= kImageCacheLimit.
     mutable std::mutex image_mu;
     mutable void* image = nullptr;
@@ -83,7 +83,32 @@ struct TileRect { size_t left, top, width, height; };
 // tile split of render_tiled                               src/trace.rs:142-173
 std::vector<TileRect> tile_layout(size_t W, size_t H, size_t tw, size_t th);
 
-// Device memory from the cached stream-ordered pool (rm_device.cu); dev_alloc returns a cudaError_t value (0 = ok).
+// The part of a frame one share renders (rm_gpu_options rank / world_size / partition): share `rank` of `world` owns the tiles
+// t with t % world == rank under RM_PARTITION_TILES, and the global samples rank, rank + world, ... of every pixel under
+// RM_PARTITION_SAMPLES.  world_size <= 1, or any other partition value, is the whole frame.
+struct Share {
+    size_t rank = 0, world = 1;
+    bool tiles = false;
+    explicit Share(const rm_gpu_options& o) {
+        if (o.world_size > 1 && (o.partition == RM_PARTITION_SAMPLES || o.partition == RM_PARTITION_TILES)) {
+            rank = (size_t)o.rank;
+            world = (size_t)o.world_size;
+            tiles = o.partition == RM_PARTITION_TILES;
+        }
+    }
+    // owned tiles: first_tile(), first_tile() + tile_step(), ... of the layout
+    size_t first_tile() const { return tiles ? rank : 0; }
+    size_t tile_step() const { return tiles ? world : 1; }
+    bool owns_tile(size_t t) const { return t % tile_step() == first_tile(); }
+    // the global samples of [begin, end) this share renders: *count of them from *first, sample_stride() apart
+    size_t sample_stride() const { return tiles ? 1 : world; }
+    void samples(size_t begin, size_t end, size_t* first, size_t* count) const {
+        const size_t G = sample_stride();
+        *first = begin + (rank + G - begin % G) % G;
+        *count = *first < end ? (end - *first + G - 1) / G : 0;
+    }
+};
+
 // Sum of the accumulators of several renderers (one per share of a task) into a host frame (rm_device.cu).  With a pinned
 // destination every device sums its slice of the frame from all peers' accumulators in place (peer reads over NVLink) and
 // writes it straight to the host; otherwise the sums are gathered onto the first device and copied.  Either way the sum
@@ -92,12 +117,14 @@ std::vector<TileRect> tile_layout(size_t W, size_t H, size_t tw, size_t th);
 // the exchange) and sets *mean_written; the other paths leave it alone.
 int reduce_accumulators_to_host(rm_renderer* const* renderers, int count, rm_vec3* out, bool out_is_pinned, rm_vec3* mean_pinned = nullptr,
                                 double divisor = 1.0, bool* mean_written = nullptr);
-// E_t (include/raymond.h) of every tile after `n` samples from the S and Q summed over the renderers (RM_FLAG_MOMENTS) in
-// renderer order, into `out_pinned` (a pinned_acquire block of n_tiles doubles).  Device g computes tiles g, g + count, ...
-// reading its peers' sums in place; without peer mappings the sums are staged onto the first device.  Synchronous.
-int tile_errors_to_host(rm_renderer* const* renderers, int count, size_t n, double* out_pinned, size_t n_tiles);
+// E_t (include/raymond.h) of tiles first, first + step, ... after `n` samples from the S and Q summed over the renderers
+// (RM_FLAG_MOMENTS) in renderer order, into `out_pinned` (a pinned_acquire block of n_tiles doubles; other tiles are left
+// alone).  Device g computes every count-th of those tiles from the g-th on, reading its peers' sums in place; without peer
+// mappings the sums are staged onto the first device.  Synchronous.
+int tile_errors_to_host(rm_renderer* const* renderers, int count, size_t n, double* out_pinned, size_t n_tiles, size_t first, size_t step);
 // display transform kernel (rm_display.cu): sums / divisor -> tonemap -> 8-bit RGB, device pointers
 int tonemap_device(const double* sums_device, size_t n_pixels, double divisor, double exposure, double gamma, unsigned char* out_device, void* stream);
+// Device memory from the cached stream-ordered pool (rm_device.cu); dev_alloc returns a cudaError_t value (0 = ok).
 int dev_alloc(void** p, size_t bytes);
 void dev_release(void* p);
 
@@ -113,10 +140,10 @@ struct Trace {
 
 }  // namespace rm
 
-// internal entry points of rm_device.cu used by the multi-GPU task driver (C linkage, not part of include/raymond.h)
+// internal entry points of rm_device.cu used by the task driver (C linkage, not part of include/raymond.h)
 extern "C" {
 rm_renderer* rm_renderer_create_unbound(const rm_settings* settings, const rm_gpu_options* options);
-// a scene placed on several devices at once (slices over every device's PCIe link + an all-gather over NVLink): one host thread
+// a scene placed on one device or several at once (slices over every device's PCIe link + an all-gather over NVLink): one host thread
 // per share calls _join, ALL shares must; _join returns the share's device scene or NULL
 struct rm_scene_group;
 rm_scene_group* rm_scene_group_create(const rm_scene* scene, const int32_t* devices, int count);

@@ -39,6 +39,7 @@ struct rm_task {
     rm_settings settings{};
     rm_gpu_options options{};
     std::vector<rm_renderer*> renderers;     // one per GPU (options.device_count), in rank order
+    std::vector<Share> shares;               // ... and the part of the frame each renders
     std::thread driver;
     std::mutex mu;
     std::condition_variable cv;
@@ -96,10 +97,10 @@ bool make_tile(const PendingMessage& m, rm_tile* out) {
 void post_tiles(rm_task* t, uint32_t kind, size_t sample_count, const std::shared_ptr<FrameSnapshot>& frame, const std::vector<uint8_t>* kinds = nullptr) {
     const size_t W = t->settings.camera_settings.backbuffer_width, H = t->settings.camera_settings.backbuffer_height;
     std::vector<TileRect> tiles = tile_layout(W, H, t->settings.tile_size[0], t->settings.tile_size[1]);
-    const int world = t->options.world_size > 1 ? t->options.world_size : 1;
+    const Share share(t->options);
     std::deque<PendingMessage> batch;
     for (size_t i = 0; i < tiles.size(); i++) {
-        if (t->options.partition == RM_PARTITION_TILES && (int)(i % (size_t)world) != t->options.rank) continue;
+        if (!share.owns_tile(i)) continue;
         if (kinds && (*kinds)[i] == 0xff) continue;
         batch.push_back(PendingMessage{kinds ? (uint32_t)(*kinds)[i] : kind, sample_count, tiles[i], frame});
     }
@@ -108,24 +109,15 @@ void post_tiles(rm_task* t, uint32_t kind, size_t sample_count, const std::share
     t->cv.notify_all();
 }
 
-// global sample indices in [begin, end) that rank g of G renders under the sample partition: first, count (stride G)
-void sample_share(size_t begin, size_t end, size_t g, size_t G, size_t* first, size_t* count) {
-    const size_t f = begin + ((g + G - begin % G) % G);
-    *first = f;
-    *count = f < end ? (end - f + G - 1) / G : 0;
-}
-
 void drive(rm_task* t) {
     const rm_settings& s = t->settings;
     const size_t W = s.camera_settings.backbuffer_width, H = s.camera_settings.backbuffer_height;
     const size_t G = t->renderers.size();                 // GPUs driven by this task
     // a task that is itself one rank of a multi-process job (options.world_size) renders only its share
-    const size_t world = G > 1 ? 1 : (t->options.world_size > 1 ? (size_t)t->options.world_size : 1);
-    const bool split_samples = world > 1 && t->options.partition == RM_PARTITION_SAMPLES;
-    const size_t first = split_samples ? (size_t)t->options.rank : 0;
-    const size_t stride = split_samples ? world : 1;
-    const size_t total = split_samples ? (s.sample_count > first ? (s.sample_count - first + world - 1) / world : 0) : s.sample_count;
-    const bool split_local = G > 1 && t->options.partition == RM_PARTITION_SAMPLES;
+    const Share job(t->options);
+    size_t first, total;
+    job.samples(0, s.sample_count, &first, &total);
+    const size_t stride = job.sample_stride();
     int st = RM_OK;
     Trace trace;
     // adaptive: which tiles still render, and at which checkpoint a tile may first stop
@@ -148,9 +140,9 @@ void drive(rm_task* t) {
                 // every GPU gets its share of the samples [done, done + n) (or all of them for its own tiles); launches are
                 // asynchronous, so one host thread keeps all devices busy
                 for (size_t g = 0; g < G && st == RM_OK; g++) {
-                    size_t f = done, c = n;
-                    if (split_local) sample_share(done, done + n, g, G, &f, &c);
-                    if (c) st = rm_renderer_render(t->renderers[g], f, c, split_local ? G : 1);
+                    size_t f, c;
+                    t->shares[g].samples(done, done + n, &f, &c);
+                    if (c) st = rm_renderer_render(t->renderers[g], f, c, t->shares[g].sample_stride());
                 }
             }
             done += n;
@@ -160,7 +152,7 @@ void drive(rm_task* t) {
                 if (st == RM_OK && t->adaptive && done >= first_stop) {
                     // TileFinished(done) for every still-active tile whose E_t <= threshold (NaN never is), TileProgressed for the rest
                     if (!errors && !(errors = (double*)pinned_acquire(std::max<size_t>(n_tiles, 1) * sizeof(double)))) throw std::bad_alloc();
-                    st = tile_errors_to_host(t->renderers.data(), (int)G, done, errors, n_tiles);
+                    st = tile_errors_to_host(t->renderers.data(), (int)G, done, errors, n_tiles, 0, 1);
                     std::vector<uint8_t> kinds(n_tiles, 0xff);
                     bool changed = false;
                     for (size_t i = 0; i < n_tiles && st == RM_OK; i++) {
@@ -255,21 +247,14 @@ rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const r
         o.device_count = 0;
         return o;
     };
-    // several shares: the scene image crosses the bus once, in slices, and is gathered over NVLink (rm_scene_group)
-    rm_scene_group* group = nullptr;
-    if (G > 1) {
-        group = rm_scene_group_create(scene, devices.data(), (int)G);
-        if (!group) { delete t; return nullptr; }
-        trace.mark("rm_render_tiled: host images of the grids ready");
-    }
+    for (size_t g = 0; g < G; g++) t->shares.emplace_back(options_for(g));
+    // the scene image crosses the bus once, in slices, and is gathered over NVLink (rm_scene_group)
+    rm_scene_group* group = rm_scene_group_create(scene, devices.data(), (int)G);
+    if (!group) { delete t; return nullptr; }
+    trace.mark("rm_render_tiled: host images of the grids ready");
     auto record = [&](size_t g) { status[g] = rm_last_status(); errors[g] = rm_last_error(); };
     auto create = [&](size_t g) {
         rm_gpu_options o = options_for(g);
-        if (!group) {
-            t->renderers[0] = rm_renderer_create(scene, settings, &o);
-            if (!t->renderers[0]) record(0);
-            return;
-        }
         Trace share_trace;
         rm_renderer* r = rm_renderer_create_unbound(settings, &o);
         if (!r) record(g);
@@ -292,7 +277,7 @@ rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const r
         create(0);
         for (std::thread& th : pool) th.join();
     }
-    if (group) rm_scene_group_destroy(group);
+    rm_scene_group_destroy(group);
     trace.mark("rm_render_tiled: scene resident and renderers ready on every device");
     for (size_t g = 0; g < G; g++)
         if (!t->renderers[g]) {

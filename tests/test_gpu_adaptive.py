@@ -260,7 +260,8 @@ def adaptive_options(device_list, partition, flags=0):
     return A.GpuOptions(seed=SEED, device_list=device_list, partition=partition, flags=flags)
 
 
-SHARES = {"one": (None, A.PARTITION_SAMPLES), "samples2": ([0, 0], A.PARTITION_SAMPLES), "tiles3": ([0, 0, 0], A.PARTITION_TILES)}
+SHARES = {"one": (None, A.PARTITION_SAMPLES), "samples2": ([0, 0], A.PARTITION_SAMPLES), "tiles3": ([0, 0, 0], A.PARTITION_TILES),
+          "staged65": ([0] * 65, A.PARTITION_SAMPLES)}
 
 
 @pytest.mark.parametrize("name", list(SCENES))

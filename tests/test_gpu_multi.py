@@ -15,8 +15,9 @@ pytestmark = pytest.mark.gpu
 
 
 def device_lists():
-    """[0, 0] (two shares on one GPU), three shares, and — when the box has them — distinct GPUs."""
-    lists = [[0, 0], [0, 0, 0]]
+    """[0, 0] (two shares on one GPU), three shares, 65 (more than one exchange kernel takes: the staged exchange), and — when
+    the box has them — distinct GPUs."""
+    lists = [[0, 0], [0, 0, 0], [0] * 65]
     n = cuda_device_count()
     if n >= 2:
         lists += [[0, 1], [1, 0, 1]]
