@@ -81,6 +81,19 @@ extern "C" {
     pub fn rm_renderer_set_active_tiles(r: *mut rm_renderer, active: *const u8, tile_count: usize) -> c_int;
 }
 
+// ---- first-hit feature buffers (RM_FLAG_AOV) and the feature-guided a-trous denoiser (include/raymond.h states the filter).
+#[repr(C)] #[derive(Clone, Copy)] pub struct rm_denoise_settings {
+    pub iterations: u32,   // 1..10
+    pub reserved: u32,
+    pub sigma_color: f64, pub sigma_normal: f64, pub sigma_albedo: f64, pub sigma_depth: f64,   // finite, > 0
+}
+extern "C" {
+    // feature sums / sample_count, W*H each; any output may be null; RM_ERR_STATE without RM_FLAG_AOV
+    pub fn rm_renderer_read_aovs(r: *mut rm_renderer, sample_count: usize, albedo: *mut rm_vec3, normal: *mut rm_vec3, depth: *mut f64) -> c_int;
+    // null settings = the defaults; needs RM_FLAG_AOV | RM_FLAG_MOMENTS, sample_count >= 2 and a renderer with world_size <= 1
+    pub fn rm_renderer_read_denoised(r: *mut rm_renderer, sample_count: usize, settings: *const rm_denoise_settings, out: *mut rm_vec3) -> c_int;
+}
+
 // ---- values of the enum / flag fields (include/raymond.h, RM_ABI_VERSION 2)
 pub const RM_PARTITION_SAMPLES: u32 = 0;        // rank g renders global samples g, g+G, ...
 pub const RM_PARTITION_TILES: u32 = 1;          // tiles dealt round-robin in the reference's queue order (src/trace.rs:146-172)
@@ -90,5 +103,6 @@ pub const RM_FLAG_KEEP_NONFINITE: u32 = 1;
 pub const RM_FLAG_STAGE_TIMING: u32 = 2;
 pub const RM_FLAG_COUNT_WORK: u32 = 4;
 pub const RM_FLAG_MOMENTS: u32 = 64;            // keep the running sums of squared samples (rm_renderer_read_moments / tile_errors)
+pub const RM_FLAG_AOV: u32 = 128;               // keep the first-hit albedo / normal / depth sums (rm_renderer_read_aovs / read_denoised)
 pub const RM_TILE_FINISHED: u32 = 0;            // Message::TileFinished
 pub const RM_TILE_PROGRESSED: u32 = 1;          // Message::TileProgressed

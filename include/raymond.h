@@ -227,6 +227,16 @@ typedef enum rm_precision {
  * values Q, under the same rule as S — samples added in global sample order; non-finite samples left out of both by default,
  * added to both with RM_FLAG_KEEP_NONFINITE.  Read with rm_renderer_read_moments; used by rm_renderer_tile_errors. */
 #define RM_FLAG_MOMENTS 64u
+/* First-hit feature buffers.  For every sample, the closest hit Scene::intersect reports for its camera ray (the depth-1 ray,
+ * depth of field included) contributes
+ *   albedo: the hit object's rm_material.a (the colour of Diffuse / Metal, the emitted radiance of Emission),
+ *   normal: the shading normal the reference computes there (src/trace.rs:244: a plane's normal, the normalised frag - centre of
+ *           a sphere, the Heron-area triangle normal of a grid; emitters included),
+ *   depth:  Hit.distance;
+ * a miss contributes zeros.  The renderer keeps their running sums per pixel, added in global sample order like S, with no
+ * non-finite filtering.  Read with rm_renderer_read_aovs; used by rm_renderer_read_denoised.  For rm_renderer_* only: a task
+ * cannot read the sums, so rm_render_tiled and rm_render_tiled_adaptive refuse the flag with RM_ERR_UNSUPPORTED. */
+#define RM_FLAG_AOV 128u
 
 /* GPU-side knobs that have no counterpart in the reference. Zero-initialise
  * for defaults (device 0, one rank, library-owned stream and buffers). */
@@ -380,6 +390,36 @@ size_t rm_renderer_tile_errors(rm_renderer* r, size_t sample_count, double* out,
  * `tile_count` = the layout's count) is non-zero; the sums of the other tiles are left untouched.  NULL = every tile.
  * Asynchronous on the renderer's stream. */
 int rm_renderer_set_active_tiles(rm_renderer* r, const uint8_t* active, size_t tile_count);
+/* D2H of the first-hit feature sums (RM_FLAG_AOV) divided by sample_count, row-major W*H; any output may be NULL.
+ * RM_ERR_STATE without RM_FLAG_AOV; RM_ERR_INVALID_ARGUMENT for sample_count 0. */
+int rm_renderer_read_aovs(rm_renderer* r, size_t sample_count, rm_vec3* albedo_host, rm_vec3* normal_host, double* depth_host);
+
+/* Feature-guided denoiser (no counterpart in the reference).  From the renderer's S, Q and feature sums after n samples, per pixel
+ * p: the mean colour c = S / n, its variance v = se2_R + se2_G + se2_B (se2 as defined above rm_adaptive_settings), and the means
+ * of albedo a, normal m and depth z, rounded to f32.  Then `iterations` passes of an edge-avoiding a-trous filter; pass i
+ * (step = 2^i) takes the taps q = p + step * (dx, dy), dx, dy in -2..2 (dy outer, dx inner, both ascending; taps outside the
+ * frame skipped), h = k[dx] * k[dy] with k = (1/16, 1/4, 3/8, 1/4, 1/16), and
+ *   w  = h * expf(-( |c_p - c_q| / (sigma_color * sqrt(v_p) + 1e-6) + |m_p - m_q|^2 / sigma_normal^2
+ *                    + |a_p - a_q|^2 / sigma_albedo^2 + |z_p - z_q| / (sigma_depth * step * z_p + 1e-6) ))
+ *   c'_p = sum w c_q / sum w,   v'_p = sum w^2 v_q / (sum w)^2   (f32).
+ * A tap with any non-finite value has weight 0; a pixel with any non-finite value is copied unchanged.
+ * Defaults (settings NULL): iterations 1, sigma_color 1e4, sigma_normal 0.1, sigma_albedo 0.3, sigma_depth 1 — chosen from a sweep on
+ * GoldDragon (stand-in) and ReflectiveSpheres at 320x240 x 16 spp (scripts/denoise_bench.py; profiles/r5_denoise.jsonl).  The colour
+ * term weighs by the centre's variance only: a pixel whose samples were all equal (v = 0) takes no neighbour while its noisy
+ * neighbours take it, which darkens the frame with more passes or a smaller sigma_color (5 passes at sigma_color 4: -3.8 % and
+ * -6.2 % mean luminance at 16 spp; no swept setting with sigma_color <= 16 stays within 1 %).  With the defaults the colour term
+ * acts at v = 0 only: RMSE 0.36x / 0.55x of the raw 16-spp frame, mean luminance -0.7 % at 16 spp, within 0.03 % at 64 spp,
+ * 9-11 % darker at 4 spp. */
+typedef struct rm_denoise_settings {
+    uint32_t iterations;   /* 1..10 */
+    uint32_t reserved;
+    double sigma_color, sigma_normal, sigma_albedo, sigma_depth;   /* > 0; as f32 each a finite normal value, and so are the f32
+                                                                    * squares of sigma_normal and sigma_albedo (~1.1e-19 .. 1.8e19) */
+} rm_denoise_settings;
+/* The final c, row-major W*H, to HOST memory.  Needs RM_FLAG_AOV and RM_FLAG_MOMENTS (else RM_ERR_STATE); sample_count >= 2 and
+ * valid settings (else RM_ERR_INVALID_ARGUMENT, before any device work); a renderer with world_size > 1 gets RM_ERR_UNSUPPORTED.
+ * Tonemap the result with rm_tonemap_rgb8. */
+int rm_renderer_read_denoised(rm_renderer* r, size_t sample_count, const rm_denoise_settings* settings, rm_vec3* out_host);
 int rm_renderer_stats(rm_renderer* r, rm_stats* out);
 
 /* Per-stage breakdown of the wavefront.  Slot d (1 <= d < RM_STAGE_SLOTS) is the stage that traces

@@ -43,6 +43,7 @@ RM_ERR_DEGENERATE_BOUNDS = -5
 RM_ERR_GRID_CAST = -6
 RM_ERR_CUDA = -7
 RM_ERR_UNSUPPORTED = -8
+RM_ERR_STATE = -10
 RM_ERR_PROJECT = -11
 
 PARTITION_SAMPLES = 0
@@ -54,6 +55,7 @@ FLAG_NO_RAY_BINNING = 8     # 8, 16, 32: reserved values, accepted with no effec
 FLAG_FUSE_SETUP = 16
 FLAG_SPLIT_SETUP = 32
 FLAG_MOMENTS = 64           # keep the running sums of squared samples next to the sums (Renderer.read_moments / tile_errors)
+FLAG_AOV = 128              # keep the first-hit albedo / normal / depth sums (Renderer.read_aovs / read_denoised)
 PRECISION_F64 = 0
 PRECISION_F32_SHADING = 1
 STAGE_SLOTS = 16
@@ -94,6 +96,11 @@ class GpuOptionsC(C.Structure):
 
 class AdaptiveSettingsC(C.Structure):
     _fields_ = [("threshold", C.c_double), ("min_samples", C.c_size_t)]
+
+
+class DenoiseSettingsC(C.Structure):
+    _fields_ = [("iterations", C.c_uint32), ("reserved", C.c_uint32), ("sigma_color", C.c_double), ("sigma_normal", C.c_double),
+                ("sigma_albedo", C.c_double), ("sigma_depth", C.c_double)]
 
 
 class TileC(C.Structure):
@@ -143,6 +150,7 @@ ABI_SYMBOLS = [
     "rm_renderer_stats", "rm_renderer_stage_stats", "rm_renderer_destroy", "rm_tile_layout", "rm_renderer_read_rgb8", "rm_tonemap_rgb8",
     "rm_write_png", "rm_project_load_scene", "rm_message_to_json", "rm_release_cached_memory", "rm_measure_fp64_rate",
     "rm_render_tiled_adaptive", "rm_renderer_read_moments", "rm_renderer_tile_errors", "rm_renderer_set_active_tiles",
+    "rm_renderer_read_aovs", "rm_renderer_read_denoised",
 ]
 
 _lib = None
@@ -188,6 +196,8 @@ def lib():
         "rm_renderer_read_moments": (i32, [vp, vp]),
         "rm_renderer_tile_errors": (sz, [vp, sz, vp, sz]),
         "rm_renderer_set_active_tiles": (i32, [vp, vp, sz]),
+        "rm_renderer_read_aovs": (i32, [vp, sz, vp, vp, vp]),
+        "rm_renderer_read_denoised": (i32, [vp, sz, P(DenoiseSettingsC), vp]),
         "rm_task_poll": (i32, [vp, P(MessageC)]),
         "rm_task_await": (i32, [vp, vp]),
         "rm_task_set_callback": (i32, [vp, TILE_CALLBACK, vp]),
@@ -633,6 +643,20 @@ class AdaptiveSettings:
         return AdaptiveSettingsC(float(self.threshold), int(self.min_samples))
 
 
+@dataclass
+class DenoiseSettings:
+    """rm_denoise_settings: the a-trous filter of Renderer.read_denoised (include/raymond.h states it and the defaults)."""
+    iterations: int = 1
+    sigma_color: float = 1e4
+    sigma_normal: float = 0.1
+    sigma_albedo: float = 0.3
+    sigma_depth: float = 1.0
+
+    def _c(self) -> DenoiseSettingsC:
+        return DenoiseSettingsC(int(self.iterations), 0, float(self.sigma_color), float(self.sigma_normal), float(self.sigma_albedo),
+                                float(self.sigma_depth))
+
+
 def render_tiled(scene: Scene, settings: Settings, options: Optional[GpuOptions] = None,
                  adaptive: Optional[AdaptiveSettings] = None) -> TaskHandle:
     """render_tiled(scene, settings) -> TaskHandle (src/trace.rs:137-230). Returns immediately.  `adaptive` adds per-tile early
@@ -760,6 +784,21 @@ class Renderer:
             return
         m = np.ascontiguousarray(np.asarray(mask, dtype=bool).astype(np.uint8))
         _check(lib().rm_renderer_set_active_tiles(self._h, _ptr(m), m.size))
+
+    def read_aovs(self, sample_count: int):
+        """First-hit feature means after `sample_count` samples (FLAG_AOV): albedo (H, W, 3), normal (H, W, 3), depth (H, W), f64."""
+        albedo, normal = self._frame(), self._frame()
+        depth = np.zeros(albedo.shape[:2])
+        _check(lib().rm_renderer_read_aovs(self._h, sample_count, _ptr(albedo), _ptr(normal), _ptr(depth)))
+        return albedo, normal, depth
+
+    def read_denoised(self, sample_count: int, settings: Optional[DenoiseSettings] = None) -> np.ndarray:
+        """The mean frame after `sample_count` samples through the feature-guided a-trous filter (FLAG_AOV | FLAG_MOMENTS), (H, W, 3).
+        settings None = the library's defaults."""
+        out = self._frame()
+        s = None if settings is None else C.byref(settings._c())
+        _check(lib().rm_renderer_read_denoised(self._h, sample_count, s, _ptr(out)))
+        return out
 
     def read_rgb8(self, sample_count: int, exposure: float = 1.0, gamma: float = 2.2) -> np.ndarray:
         """sum / sample_count -> cli_old's tonemap (src cli_old/src/main.rs:157-181) on the GPU -> (H, W, 3) uint8."""

@@ -685,6 +685,8 @@ struct rm_renderer {
     bool owns_accum = false;
     size_t accum_bytes = 0;
     double* moments = nullptr;                      // RM_FLAG_MOMENTS: W*H rm_vec3 running sums of squares (peers read it in place)
+    double* aov = nullptr;                          // RM_FLAG_AOV: first-hit feature sums, W*H albedo rm_vec3, W*H normal rm_vec3, W*H depth
+    size_t aov_bytes = 0;
     unsigned* active_map = nullptr;                 // rm_renderer_set_active_tiles: the active tiles' runs of the pixel map
     uint3* active_runs = nullptr;                   // ... and the {source, destination, length} list that gathered them
     size_t full_batch_spp = 1;                      // batch_spp for the whole share
@@ -713,6 +715,7 @@ struct rm_renderer {
         isect.release();
         if (owns_accum) visible_release(device, accum_bytes, accum);
         if (moments) visible_release(device, accum_bytes, moments);
+        if (aov) visible_release(device, aov_bytes, aov);
         dev_free(active_map); dev_free(active_runs);
         if (owns_stream && stream) cudaStreamDestroy(stream);
         if (owns_scene) delete ds;
@@ -866,6 +869,11 @@ static int renderer_init(rm_renderer* r) {
         RM_CUDA(visible_acquire(r->device, r->accum_bytes, (void**)&r->moments));
         RM_CUDA(cudaMemsetAsync(r->moments, 0, W * H * 3 * sizeof(double), r->stream));
     }
+    if (r->opt.flags & RM_FLAG_AOV) {
+        r->aov_bytes = std::max<size_t>(W * H, 1) * 7 * sizeof(double);
+        RM_CUDA(visible_acquire(r->device, r->aov_bytes, (void**)&r->aov));
+        RM_CUDA(cudaMemsetAsync(r->aov, 0, W * H * 7 * sizeof(double), r->stream));
+    }
     trace.mark("renderer_init: queues, counters, accumulator allocated");
     return RM_OK;
 }
@@ -923,7 +931,8 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         const Queue& qout = r->q[depth & 1];
         SetupArgs sa{};
         for (int k = 0; k < 6; k++) sa.q[k] = qin.f[k];
-        sa.emitters_only = last_skip && depth == limit ? 1 : 0;
+        // the feature buffers need the closest hit of every camera ray, so depth 1 never skips a grid for them
+        sa.emitters_only = last_skip && depth == limit && !(depth == 1 && r->aov) ? 1 : 0;
         int st;
         if (depth == 1) {
             sa.n_ptr = nullptr; sa.n_direct = n_paths;
@@ -935,6 +944,11 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
                                              depth, count, r->totals, r->stream, hook);
         }
         if (st != RM_OK) return st;
+        if (depth == 1 && r->aov) {     // before k_shade: the next depth's k_setup overwrites the hit records
+            const size_t W = r->settings.camera_settings.backbuffer_width, H = r->settings.camera_settings.backbuffer_height;
+            k_aov<<<(rp.n_pixels + kBlock - 1) / kBlock, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, r->isect.hit, n_samples, W * H, r->aov);
+            r->launches++;
+        }
         hook.begin(2);
         const bool last = last_shade && depth == limit;
         if (depth == 1) {
@@ -1336,6 +1350,7 @@ int rm_renderer_clear(rm_renderer* r) {
     const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height * 3;
     RM_CUDA(cudaMemsetAsync(r->accum, 0, n * sizeof(double), r->stream));   // statistics stay cumulative
     if (r->moments) RM_CUDA(cudaMemsetAsync(r->moments, 0, n * sizeof(double), r->stream));
+    if (r->aov) RM_CUDA(cudaMemsetAsync(r->aov, 0, n / 3 * 7 * sizeof(double), r->stream));
     return RM_OK;
 }
 
@@ -1349,24 +1364,26 @@ int rm_renderer_sync(rm_renderer* r) {
 
 // The accumulator to (pageable) caller memory: D2H at link speed into a cached pinned block, then a few host threads move
 // it on, dividing by `divisor` on the way (tile.data[..] / tile.sample_count as f64, src/trace.rs:95) when it is not 0.
-static int read_accumulator(rm_renderer* r, rm_vec3* out, double divisor, const double* source = nullptr) {
+// `source` / `count`: another W*H-sized buffer of `count` doubles (default: the accumulator, W*H rm_vec3).
+static int read_accumulator(rm_renderer* r, void* out_host, double divisor, const double* source = nullptr, size_t count = 0) {
     RM_CUDA(cudaSetDevice(r->device));
-    const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height;
-    rm_vec3* pin = (rm_vec3*)pinned_acquire(std::max<size_t>(n, 1) * sizeof(rm_vec3));
-    cudaError_t e = cudaMemcpyAsync(pin ? pin : out, source ? source : r->accum, n * sizeof(rm_vec3), cudaMemcpyDeviceToHost, r->stream);
+    const size_t n = count ? count : r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height * 3;
+    double* const out = (double*)out_host;
+    double* pin = (double*)pinned_acquire(std::max<size_t>(n, 1) * sizeof(double));
+    cudaError_t e = cudaMemcpyAsync(pin ? pin : out, source ? source : r->accum, n * sizeof(double), cudaMemcpyDeviceToHost, r->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(r->stream);
     if (e != cudaSuccess) {
         pinned_release(pin);
         return fail(RM_ERR_CUDA, std::string("D2H of the accumulator: ") + cudaGetErrorString(e));
     }
     harvest_events(r);
-    const rm_vec3* src = pin ? pin : out;
+    const double* src = pin ? pin : out;
     auto rows = [&](size_t lo, size_t hi) {
-        if (divisor != 0.0) for (size_t i = lo; i < hi; i++) out[i] = rm_vec3{src[i].x / divisor, src[i].y / divisor, src[i].z / divisor};
-        else if (src != out) memcpy((void*)(out + lo), (const void*)(src + lo), (hi - lo) * sizeof(rm_vec3));
+        if (divisor != 0.0) for (size_t i = lo; i < hi; i++) out[i] = src[i] / divisor;
+        else if (src != out) memcpy((void*)(out + lo), (const void*)(src + lo), (hi - lo) * sizeof(double));
     };
     const unsigned hw = std::thread::hardware_concurrency();
-    const size_t workers = n < ((size_t)1 << 18) ? 1 : std::min<size_t>(hw ? hw : 4, 8);
+    const size_t workers = n < ((size_t)3 << 18) ? 1 : std::min<size_t>(hw ? hw : 4, 8);
     std::vector<std::thread> pool;
     for (size_t w = 1; w < workers; w++) pool.emplace_back(rows, n * w / workers, n * (w + 1) / workers);
     rows(0, n / workers);
@@ -1414,6 +1431,42 @@ int rm_renderer_read_moments(rm_renderer* r, rm_vec3* out) {
     if (!r || !out) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_moments: null argument");
     if (!r->moments) return fail(RM_ERR_STATE, "rm_renderer_read_moments: the renderer was created without RM_FLAG_MOMENTS");
     return read_accumulator(r, out, 0.0, r->moments);
+}
+
+int rm_renderer_read_aovs(rm_renderer* r, size_t sample_count, rm_vec3* albedo, rm_vec3* normal, double* depth) {
+    if (!r) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_aovs: null renderer");
+    if (!r->aov) return fail(RM_ERR_STATE, "rm_renderer_read_aovs: the renderer was created without RM_FLAG_AOV");
+    if (sample_count == 0) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_aovs: sample_count is 0");
+    const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height;
+    const double div = (double)sample_count;
+    if (albedo) if (int st = read_accumulator(r, albedo, div, r->aov, n * 3)) return st;
+    if (normal) if (int st = read_accumulator(r, normal, div, r->aov + n * 3, n * 3)) return st;
+    if (depth) if (int st = read_accumulator(r, depth, div, r->aov + n * 6, n)) return st;
+    return RM_OK;
+}
+
+int rm_renderer_read_denoised(rm_renderer* r, size_t sample_count, const rm_denoise_settings* settings, rm_vec3* out) {
+    if (!r || !out) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_denoised: null argument");
+    if (!r->aov || !r->moments) return fail(RM_ERR_STATE, "rm_renderer_read_denoised: needs a renderer created with RM_FLAG_AOV and RM_FLAG_MOMENTS");
+    if (r->opt.world_size > 1) return fail(RM_ERR_UNSUPPORTED, "rm_renderer_read_denoised: the filter needs the whole frame's sums (world_size > 1)");
+    if (sample_count < 2) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_denoised: the variance needs sample_count >= 2");
+    rm_denoise_settings s{1, 0, 1e4, 0.1, 0.3, 1.0};       // the defaults stated in include/raymond.h
+    if (settings) s = *settings;
+    // the filter uses each sigma as an f32, and the squares of sigma_normal and sigma_albedo: all of them must be normal f32 values
+    // (a square that underflows to 0 or a sigma that overflows to inf would make the centre tap's weight NaN)
+    const auto usable = [](double x, bool squared) {
+        const float f = (float)x, g = squared ? f * f : f;
+        return std::isfinite(x) && x > 0.0 && std::isfinite(g) && g >= FLT_MIN;
+    };
+    if (s.iterations < 1 || s.iterations > 10 || !usable(s.sigma_color, false) || !usable(s.sigma_normal, true) || !usable(s.sigma_albedo, true) ||
+        !usable(s.sigma_depth, false))
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_denoised: iterations outside 1..10 or a sigma outside the f32 range the filter needs");
+    RM_CUDA(cudaSetDevice(r->device));
+    const size_t W = r->settings.camera_settings.backbuffer_width, H = r->settings.camera_settings.backbuffer_height;
+    const int st = denoise_to_host(r->accum, r->moments, r->aov, W, H, (double)sample_count, s, out, r->stream);
+    harvest_events(r);
+    if (st == RM_OK) r->launches += 1 + s.iterations;
+    return st;
 }
 
 size_t rm_renderer_tile_errors(rm_renderer* r, size_t sample_count, double* out, size_t capacity) {

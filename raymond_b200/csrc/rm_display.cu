@@ -1,5 +1,6 @@
 // rm_display.cu — the display transform that follows the path in the reference's one working front-end
-// (cli_old/src/main.rs:157-181), as a GPU epilogue of the accumulator, and the host PNG writer (:194-197).
+// (cli_old/src/main.rs:157-181), as a GPU epilogue of the accumulator, the host PNG writer (:194-197), and the
+// feature-guided denoiser of rm_renderer_read_denoised (no counterpart in the reference).
 //
 //   tone_mapped = 1 - exp(p * -1.0 * exposure);  tone_mapped = tone_mapped.powf(1.0 / gamma);
 //   (tone_mapped * 255.0).cast::<u8>()  -> Some(v): the pixel;  None (any channel NaN or outside (-1, 256)): the
@@ -46,6 +47,101 @@ int tonemap_device(const double* sums_device, size_t n_pixels, double divisor, d
     k_tonemap<<<blocks, 256, 0, (cudaStream_t)stream>>>(sums_device, n_pixels, divisor, exposure, 1.0 / gamma, out_device);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("k_tonemap: ") + cudaGetErrorString(e));
+    return RM_OK;
+}
+
+// ---- the edge-avoiding a-trous denoiser of rm_renderer_read_denoised (include/raymond.h gives the filter).  Each pixel is one
+// float4 of (mean colour, variance) that the iterations update, and two of guides that stay: (albedo, depth) and (normal, 0).
+
+__device__ __forceinline__ bool finite4(float4 a) { return isfinite(a.x) && isfinite(a.y) && isfinite(a.z) && isfinite(a.w); }
+__device__ __forceinline__ bool finite3(float4 a) { return isfinite(a.x) && isfinite(a.y) && isfinite(a.z); }
+
+// The means after n samples, formed in f64 exactly as include/raymond.h defines m and se2, then rounded to f32 once.
+__global__ void __launch_bounds__(256) k_denoise_pack(const double* __restrict__ sums, const double* __restrict__ moments, const double* __restrict__ aov,
+                                                      size_t n_pixels, double n, float4* __restrict__ cv, float4* __restrict__ az, float4* __restrict__ nm) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_pixels) {
+        float m[3];
+        double se2 = 0.0;
+#pragma unroll
+        for (int c = 0; c < 3; c++) {
+            const double S = sums[i * 3 + c], Q = moments[i * 3 + c];
+            const double mean = S / n;
+            const double d = Q - S * mean;
+            se2 += (d < 0.0 ? 0.0 : d) / (n - 1.0) / n;
+            m[c] = (float)mean;
+        }
+        const double* alb = aov + i * 3;
+        const double* nrm = aov + (n_pixels + i) * 3;
+        cv[i] = make_float4(m[0], m[1], m[2], (float)se2);
+        az[i] = make_float4((float)(alb[0] / n), (float)(alb[1] / n), (float)(alb[2] / n), (float)(aov[6 * n_pixels + i] / n));
+        nm[i] = make_float4((float)(nrm[0] / n), (float)(nrm[1] / n), (float)(nrm[2] / n), 0.0f);
+    }
+}
+
+// One iteration at tap distance `step`: 5x5 taps, dy outer and dx inner, both ascending, so the sums have one order.
+__global__ void __launch_bounds__(256) k_atrous(const float4* __restrict__ cv_in, const float4* __restrict__ az, const float4* __restrict__ nm,
+                                                float4* __restrict__ cv_out, int W, int H, int step, float sigma_c, float sigma_n2, float sigma_a2,
+                                                float sigma_z) {
+    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (x >= W || y >= H) return;
+    const size_t p = (size_t)y * W + x;
+    const float4 cp = cv_in[p], ap = az[p], np = nm[p];
+    if (!(finite4(cp) && finite4(ap) && finite3(np))) { cv_out[p] = cp; return; }
+    const float kern[5] = {1.0f / 16.0f, 1.0f / 4.0f, 3.0f / 8.0f, 1.0f / 4.0f, 1.0f / 16.0f};
+    // the denominators depend on p only: each division becomes a product with the f32 reciprocal, formed once per pixel
+    const float rc = 1.0f / (sigma_c * sqrtf(cp.w) + 1e-6f), rn = 1.0f / sigma_n2, ra = 1.0f / sigma_a2;
+    const float rz = 1.0f / (sigma_z * (float)step * ap.w + 1e-6f);
+    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, sv = 0.0f;
+#pragma unroll
+    for (int dy = -2; dy <= 2; dy++) {
+        const int qy = y + dy * step;
+#pragma unroll
+        for (int dx = -2; dx <= 2; dx++) {
+            const int qx = x + dx * step;
+            if (qx < 0 || qx >= W || qy < 0 || qy >= H) continue;
+            const size_t q = (size_t)qy * W + qx;
+            const float4 cq = cv_in[q], aq = az[q], nq = nm[q];
+            if (!(finite4(cq) && finite4(aq) && finite3(nq))) continue;
+            const float cr = cp.x - cq.x, cg = cp.y - cq.y, cb = cp.z - cq.z;
+            const float nx = np.x - nq.x, ny = np.y - nq.y, nz = np.z - nq.z;
+            const float ax = ap.x - aq.x, ay = ap.y - aq.y, azz = ap.z - aq.z;
+            const float e = sqrtf(cr * cr + cg * cg + cb * cb) * rc + (nx * nx + ny * ny + nz * nz) * rn + (ax * ax + ay * ay + azz * azz) * ra +
+                            fabsf(ap.w - aq.w) * rz;
+            const float w = kern[dx + 2] * kern[dy + 2] * expf(-e);
+            sw += w;
+            sr += w * cq.x; sg += w * cq.y; sb += w * cq.z;
+            sv += w * w * cq.w;
+        }
+    }
+    cv_out[p] = make_float4(sr / sw, sg / sw, sb / sw, sv / (sw * sw));
+}
+
+int denoise_to_host(const double* sums, const double* moments, const double* aov, size_t W, size_t H, double n, const rm_denoise_settings& s,
+                    rm_vec3* out, void* stream_) {
+    cudaStream_t stream = (cudaStream_t)stream_;
+    const size_t np = W * H;
+    float4* buf = nullptr;      // cv ping, cv pong, albedo + depth, normal
+    cudaError_t e = (cudaError_t)dev_alloc((void**)&buf, std::max<size_t>(np, 1) * 4 * sizeof(float4));
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("denoiser buffers: ") + cudaGetErrorString(e));
+    float4* const cv[2] = {buf, buf + np};
+    k_denoise_pack<<<(unsigned)((np + 255) / 256), 256, 0, stream>>>(sums, moments, aov, np, n, cv[0], buf + 2 * np, buf + 3 * np);
+    const dim3 tb(16, 16), grid((unsigned)((W + 15) / 16), (unsigned)((H + 15) / 16));
+    const float sn = (float)s.sigma_normal, sa = (float)s.sigma_albedo;
+    for (uint32_t i = 0; i < s.iterations; i++)
+        k_atrous<<<grid, tb, 0, stream>>>(cv[i & 1], buf + 2 * np, buf + 3 * np, cv[(i + 1) & 1], (int)W, (int)H, 1 << i, (float)s.sigma_color,
+                                          sn * sn, sa * sa, (float)s.sigma_depth);
+    e = cudaGetLastError();
+    float4* pin = (float4*)pinned_acquire(std::max<size_t>(np, 1) * sizeof(float4));
+    if (e == cudaSuccess && !pin) e = cudaErrorMemoryAllocation;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(pin, cv[s.iterations & 1], np * sizeof(float4), cudaMemcpyDeviceToHost, stream);
+    const cudaError_t done = cudaStreamSynchronize(stream);      // before the buffers go back to the pool
+    if (e == cudaSuccess) e = done;
+    dev_release(buf);
+    if (e == cudaSuccess)
+        for (size_t i = 0; i < np; i++) out[i] = rm_vec3{pin[i].x, pin[i].y, pin[i].z};
+    if (pin) pinned_release(pin);
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("denoiser: ") + cudaGetErrorString(e));
     return RM_OK;
 }
 

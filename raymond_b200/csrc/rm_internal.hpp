@@ -124,6 +124,10 @@ int reduce_accumulators_to_host(rm_renderer* const* renderers, int count, rm_vec
 int tile_errors_to_host(rm_renderer* const* renderers, int count, size_t n, double* out_pinned, size_t n_tiles, size_t first, size_t step);
 // display transform kernel (rm_display.cu): sums / divisor -> tonemap -> 8-bit RGB, device pointers
 int tonemap_device(const double* sums_device, size_t n_pixels, double divisor, double exposure, double gamma, unsigned char* out_device, void* stream);
+// the a-trous denoiser (rm_display.cu, rm_renderer_read_denoised): from the device sums S, Q and the RM_FLAG_AOV planes of a W x H
+// frame after n samples to W*H denoised means in HOST memory, on `stream`.  Synchronous; launches 1 + s.iterations kernels.
+int denoise_to_host(const double* sums, const double* moments, const double* aov, size_t W, size_t H, double n, const rm_denoise_settings& s,
+                    rm_vec3* out_host, void* stream);
 // Device memory from the cached stream-ordered pool (rm_device.cu); dev_alloc returns a cudaError_t value (0 = ok).
 int dev_alloc(void** p, size_t bytes);
 void dev_release(void* p);

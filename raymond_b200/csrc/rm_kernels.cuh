@@ -640,6 +640,15 @@ __device__ __forceinline__ void lobe_f32(const RenderParams& rp, D3 normal64, D3
 // sample NaN.  The lobe's draws are counter-based, so the extra evaluation leaves every other draw unchanged.
 enum Bounce : int { BOUNCE_NONE = 0, BOUNCE_EMIT = 1, BOUNCE_CONTINUE = 2 };
 
+// The shading normal of object `ob` at the hit point `frag` (src/trace.rs:244), for shade() and k_aov; counts a grid hit in `shaded_tri`.
+__device__ __forceinline__ D3 surface_normal(const DevScene& sc, const DevObject& ob, unsigned hit_sub, D3 frag, unsigned& shaded_tri) {
+    D3 normal;
+    if (ob.geom == GEOM_PLANE) normal = ld3(ob.g + 3);
+    else if (ob.geom == GEOM_SPHERE) normal = normalize(frag - ld3(ob.g));
+    else { normal = triangle_normal(sc.grid[ob.grid], hit_sub, frag); shaded_tri++; }
+    return normal;
+}
+
 template <int PREC, bool KEEP>
 __device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, double hit_t, int hit_obj, unsigned hit_sub, unsigned pixel,
                                         unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
@@ -648,10 +657,7 @@ __device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& 
     const D3 frag = o + d * hit_t;                                          // :246
     if (ob.mat == RM_MATERIAL_EMISSION) { v = ld3(ob.color); return BOUNCE_EMIT; }   // :250
     if (!KEEP && depth >= rp.bounce_limit) return BOUNCE_NONE;              // the child call returns 0 (:235-237)
-    D3 normal;                                                              // :244
-    if (ob.geom == GEOM_PLANE) normal = ld3(ob.g + 3);
-    else if (ob.geom == GEOM_SPHERE) normal = normalize(frag - ld3(ob.g));
-    else { normal = triangle_normal(sc.grid[ob.grid], hit_sub, frag); shaded_tri++; }
+    const D3 normal = surface_normal(sc, ob, hit_sub, frag, shaded_tri);    // :244
     const D3 to_camera = ld3(rp.cam.pos) - frag;
     const double metal = ob.mat == RM_MATERIAL_METAL ? 1.0 : 0.0;
     D3 dir;
@@ -1316,6 +1322,41 @@ __global__ void __launch_bounds__(kBlock) k_accumulate(const __grid_constant__ R
         totals->rays += rp.bounce_limit ? rays : 0ull;
         totals->samples += (unsigned long long)n_batch_samples * rp.n_pixels;
     }
+}
+
+// RM_FLAG_AOV: the first-hit feature sums (include/raymond.h), launched between the depth-1 intersection and k_shade<FIRST>, while
+// the depth-1 queue holds the camera rays and `hit` their closest hits.  One thread per owned pixel adds the batch's samples
+// i = s * n_pixels + q in global sample order, as k_accumulate does; a miss adds zeros.  `aov` holds three planes of the frame:
+// albedo (3 doubles per pixel), normal (3), depth (1).
+__global__ void __launch_bounds__(kBlock) k_aov(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue q1,
+                                                 const HitArrays hit, const unsigned n_batch_samples, const size_t frame_pixels,
+                                                 double* __restrict__ aov) {
+    const unsigned q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= rp.n_pixels) return;
+    const size_t p = rp.pixel_map[q];
+    double* const alb = aov + p * 3;
+    double* const nrm = aov + (frame_pixels + p) * 3;
+    double* const dep = aov + frame_pixels * 6 + p;
+    D3 sa = ld3(alb), sn = ld3(nrm);
+    double sz = *dep;
+    unsigned unused = 0;
+    for (unsigned s = 0; s < n_batch_samples; s++) {
+        const size_t i = (size_t)s * rp.n_pixels + q;
+        const int ob = hit.obj[i];
+        D3 a = d3(0.0, 0.0, 0.0), n = d3(0.0, 0.0, 0.0);
+        double t = 0.0;
+        if (ob >= 0) {
+            const DevObject& o = sc.obj[ob];
+            t = hit.t[i];
+            const D3 frag = d3(q1.f[0][i], q1.f[1][i], q1.f[2][i]) + d3(q1.f[3][i], q1.f[4][i], q1.f[5][i]) * t;
+            a = ld3(o.color);
+            n = surface_normal(sc, o, hit.sub[i], frag, unused);
+        }
+        sa = sa + a; sn = sn + n; sz += t;
+    }
+    alb[0] = sa.x; alb[1] = sa.y; alb[2] = sa.z;
+    nrm[0] = sn.x; nrm[1] = sn.y; nrm[2] = sn.z;
+    *dep = sz;
 }
 
 // Sums of several renderers' accumulators (and second moments), read in place in device order like the accumulator exchange.

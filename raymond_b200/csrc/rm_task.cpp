@@ -294,6 +294,13 @@ rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const r
     return t;
 }
 
+// A task has no reader of the first-hit feature sums: RM_FLAG_AOV would cost a kernel per batch and 56 B per pixel for nothing.
+bool refuse_aov(const rm_gpu_options* options, const char* who) {
+    if (!options || !(options->flags & RM_FLAG_AOV)) return false;
+    fail(RM_ERR_UNSUPPORTED, std::string(who) + ": RM_FLAG_AOV is for rm_renderer_* (a task cannot read the feature sums)");
+    return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -301,12 +308,14 @@ extern "C" {
 rm_task* rm_render_tiled(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options) {
     if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled: null argument"); return nullptr; }
     if (validate_camera(settings->camera_settings, "rm_render_tiled") != RM_OK) return nullptr;
+    if (refuse_aov(options, "rm_render_tiled")) return nullptr;
     return create_task(scene, settings, options, nullptr);
 }
 
 rm_task* rm_render_tiled_adaptive(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive) {
     if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: null argument"); return nullptr; }
     if (validate_camera(settings->camera_settings, "rm_render_tiled_adaptive") != RM_OK) return nullptr;
+    if (refuse_aov(options, "rm_render_tiled_adaptive")) return nullptr;
     if (adaptive) {
         if (!std::isfinite(adaptive->threshold) || adaptive->threshold <= 0.0) {
             fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_adaptive: threshold must be finite and > 0");
