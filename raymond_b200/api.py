@@ -21,7 +21,7 @@ from typing import Callable, Optional, Sequence
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# RAYMOND_CUDA_LIB selects another build of the same library (kernel tuning experiments); there is still no CPU path
+# RAYMOND_CUDA_LIB selects another build of the same library (the RM_TRAV_PROFILE build); there is still no CPU path
 LIB_PATH = os.environ.get("RAYMOND_CUDA_LIB") or os.path.join(_HERE, "libraymond_cuda.so")
 
 TRI_DOUBLES = 33

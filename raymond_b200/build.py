@@ -40,7 +40,8 @@ def needs_build() -> bool:
 
 
 def build(force: bool = False, verbose: bool = False, defines=(), out: str = LIB) -> str:
-    """`defines` / `out` build a tuning variant (e.g. defines=["RM_TRAV_MAX_STEPS=12"], out=".../variant.so")."""
+    """`defines` / `out` build an instrumented library next to the default one: defines=["RM_TRAV_PROFILE"],
+    out=".../trav_profile.so" adds k_traverse's per-phase cycle counters (read by scripts/trav_profile.py)."""
     if not force and out == LIB and not needs_build():
         return LIB
     cmd = [nvcc()] + NVCC_FLAGS + [f"-D{d}" for d in defines] + (["-Xptxas", "-v"] if verbose else []) + \

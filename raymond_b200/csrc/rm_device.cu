@@ -1642,7 +1642,7 @@ int rm_release_cached_memory(void) {
 }
 
 #if defined(RM_TRAV_PROFILE)
-// tuning builds only: cycles per k_traverse phase {refill, walk, tests, finish, loop head, -, -, warps}; reading resets
+// profiling builds only: cycles per k_traverse phase {refill, walk, tests, finish, loop head, -, -, warps}; reading resets
 int rm_debug_trav_profile(unsigned long long* out8) {
     cudaDeviceSynchronize();
     unsigned long long z[8] = {0, 0, 0, 0, 0, 0, 0, 0};

@@ -37,13 +37,9 @@ namespace rm {
 constexpr int kMaxObjects = 64;   // objects carried in the kernel parameter block (constant bank)
 constexpr int kMaxGrids = 8;
 constexpr int kBlock = 256;
-// resident blocks per SM the register allocation of each kernel is bounded for (tuning: -DRM_..._BLOCKS_PER_SM=n)
-#ifndef RM_SHADE_BLOCKS_PER_SM
-#define RM_SHADE_BLOCKS_PER_SM 4
-#endif
-#ifndef RM_SETUP_BLOCKS_PER_SM
-#define RM_SETUP_BLOCKS_PER_SM 4
-#endif
+// resident blocks per SM the register allocation of each kernel is bounded for
+constexpr int kShadeBlocksPerSm = 4;
+constexpr int kSetupBlocksPerSm = 4;
 
 // One AccGrid resident in HBM.
 //   cells : {first reference, count} per cell            (8 B, one 64-bit load per visited cell)
@@ -272,24 +268,9 @@ __device__ __forceinline__ bool grid_cell_index(const DevGrid& g, int cx, int cy
 }
 
 // One step of the 3D-DDA (acc_grid.rs:155-183); ties go to the later axis (A4).  False = left the grid.
-// Written with selects instead of the reference's four branches: the lanes of a warp step along different
-// axes, and the arithmetic of the chosen axis (one compare pair, one integer add, one f64 add) is the same.
-__device__ __forceinline__ bool dda_step(const DevGrid& g, Dda& s) {
-    const bool xy = s.tmx < s.tmy, xz = s.tmx < s.tmz, yz = s.tmy < s.tmz;
-    const bool ax = xy && xz;              // x
-    const bool ay = !xy && yz;             // y; otherwise z
-    const unsigned bit = ax ? 1u : (ay ? 2u : 4u);
-    const int dir = (s.step & bit) ? -1 : 1;
-    const int c = (ax ? s.cx : (ay ? s.cy : s.cz)) + dir;
-    const int r = ax ? g.res[0] : (ay ? g.res[1] : g.res[2]);
-    if (c >= r || c < 0) return false;
-    const double tm = (ax ? s.tmx : (ay ? s.tmy : s.tmz)) + (ax ? s.tdx : (ay ? s.tdy : s.tdz));
-    if (ax) { s.cx = c; s.tmx = tm; } else if (ay) { s.cy = c; s.tmy = tm; } else { s.cz = c; s.tmz = tm; }
-    return true;
-}
-
-// The same step as predicated instructions (what the hot loop of k_traverse runs): three f64 compares choose the
-// axis, then one integer add, one f64 add and one unsigned range check execute under that axis' predicate.
+// Predicated instructions instead of the reference's four branches: the lanes of a warp step along different axes, and
+// the arithmetic of the chosen axis is the same.  Three f64 compares choose the axis, then one integer add, one f64 add
+// and one unsigned range check execute under that axis' predicate.
 // sx/sy/sz = the reference's `step` (+1 / -1).  t_max of a ray that leaves the grid is advanced too; it is dead.
 __device__ __forceinline__ bool dda_step_pred(double& tmx, double& tmy, double& tmz, double tdx, double tdy, double tdz, int& cx, int& cy, int& cz,
                                               int sx, int sy, int sz, unsigned rx, unsigned ry, unsigned rz) {
@@ -689,7 +670,7 @@ struct SetupArgs {
 
 // Stage part 1.  See the header comment.
 template <int SRC>
-__global__ void __launch_bounds__(kBlock, RM_SETUP_BLOCKS_PER_SM) k_setup(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp,
+__global__ void __launch_bounds__(kBlock, kSetupBlocksPerSm) k_setup(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp,
                                                    const __grid_constant__ SetupArgs a) {
     const unsigned n = a.n_ptr ? *a.n_ptr : a.n_direct;
     const unsigned lane = threadIdx.x & 31u;
@@ -792,37 +773,17 @@ struct TraverseArgs {
 //      the earliest list position (the reference's strict `<` while walking the list in order)
 //   C  rays with a hit are finished (hit record merged), the others go back to A
 // Idle lanes re-fill from the traversal queue in groups.
-#ifndef RM_TRAV_BLOCK
-#define RM_TRAV_BLOCK 256
-#endif
-constexpr int kTravBlock = RM_TRAV_BLOCK;          // threads per block of k_traverse
+constexpr int kTravBlock = 256;                 // threads per block of k_traverse
 constexpr int kTravWarps = kTravBlock / 32;
-#ifndef RM_TRAV_MAX_STEPS
-#define RM_TRAV_MAX_STEPS 2
-#endif
-#ifndef RM_TRAV_REFILL_MIN
-#define RM_TRAV_REFILL_MIN 8
-#endif
 // 4 blocks of 256 threads = 32 warps per SM at 64 registers.  Possible since the DDA state, the ray index and the per-cell best hit
-// live in shared memory outside the phases that use them (RM_TRAV_PARK): 12 B of spills, one reload inside the pooled round.
+// live in shared memory outside the phases that use them (TravWarpShared::dda_t and what follows it): 8 B of spills, one reload
+// inside the pooled round.
 // 3 blocks (76 registers, no spills) is 3 % slower on the L2-resident GoldDragon and 1.5 % faster on multi-million-triangle soups.
-#ifndef RM_TRAV_BLOCKS_PER_SM
-#define RM_TRAV_BLOCKS_PER_SM 4
-#endif
-#ifndef RM_TRAV_LOOK
-#define RM_TRAV_LOOK 4
-#endif
-constexpr unsigned kLook = RM_TRAV_LOOK;                  // cells looked ahead per walk iteration
-constexpr unsigned kTravMaxSteps = RM_TRAV_MAX_STEPS;     // walk iterations per phase A
-constexpr unsigned kRefillMin = RM_TRAV_REFILL_MIN;       // idle lanes that trigger a re-fill while others still have work
+constexpr int kTravBlocksPerSm = 4;
+constexpr unsigned kLook = 4;             // cells looked ahead per walk iteration
+constexpr unsigned kTravMaxSteps = 2;     // walk iterations per phase A
+constexpr unsigned kRefillMin = 8;        // idle lanes that trigger a re-fill while others still have work
 
-// RM_TRAV_PARK (default on): the lane's DDA state lives in shared memory between walks, see TravWarpShared::dda_t
-#ifndef RM_TRAV_PARK
-#define RM_TRAV_PARK 1
-#endif
-#ifndef RM_TRAV_EXCL_SHARED
-#define RM_TRAV_EXCL_SHARED 1
-#endif
 struct TravWarpShared {
     double2 ray[32][3];                // {o.x o.y} {o.z d.x} {d.y d.z} of the lane's ray (three 128-bit accesses)
     unsigned long long cand_t[32];     // this round's smallest distance bits per ray
@@ -834,7 +795,6 @@ struct TravWarpShared {
     unsigned char s_owner[64];         // ... and the lane that owns the ray
     double best_t[32];                 // the lane's ray: closest hit among the objects evaluated before this grid (from the
     int best_obj[32];                  // traversal record), merged with the grid's answer when the ray finishes
-#if RM_TRAV_PARK
     double dda_t[6][32];               // t_max xyz, t_delta xyz of the lane's ray while it is not walking (phase B / C): the DDA state
     int dda_c[3][32];                  // lives in registers only inside phase A, which lets the pooled loops run with 18 fewer
     unsigned dda_s[32];                // live registers (current cell; bit a set: step along axis a is -1)
@@ -842,16 +802,13 @@ struct TravWarpShared {
     unsigned long long cell_t[32];     // closest hit of the lane's ray in its current cell (distance bits, triangle): touched only
     unsigned cell_tri[32];             // when a round found a hit and when the ray finishes
     unsigned char state[32];           // the lane's TravState during the pooled phase
-#endif
-#if RM_TRAV_EXCL_SHARED
     unsigned excl[32];                 // first pool item of the lane's list (~0: none): read by locate() every round
-#endif
 };
 
 enum TravState : unsigned { TS_IDLE = 0, TS_LOOK = 1, TS_STEP = 2, TS_READY = 3 };
 
 #if defined(RM_TRAV_PROFILE)
-// -DRM_TRAV_PROFILE: SM-clock cycles per phase, summed over warps (tuning builds only; read with rm_debug_trav_profile)
+// -DRM_TRAV_PROFILE: SM-clock cycles per phase, summed over warps (profiling builds only; read with rm_debug_trav_profile)
 __device__ unsigned long long g_trav_prof[8];
 #define RM_PROF_MARK(slot) do { const long long now__ = clock64(); prof[slot] += (unsigned long long)(now__ - prof_t); prof_t = now__; } while (0)
 #else
@@ -859,7 +816,7 @@ __device__ unsigned long long g_trav_prof[8];
 #endif
 
 template <bool COUNT>
-__global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(const __grid_constant__ DevGrid g, const __grid_constant__ TraverseArgs a) {
+__global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const __grid_constant__ DevGrid g, const __grid_constant__ TraverseArgs a) {
     __shared__ TravWarpShared shared[kTravWarps];
     TravWarpShared& sh = shared[threadIdx.x >> 5];
     const unsigned n = *a.n_ptr;
@@ -871,17 +828,9 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
 
     unsigned state = TS_IDLE;
     bool exhausted = false;                 // the queue has no more records for this warp
-    // DDA state of MY ray (acc_grid.rs:100-125)
-#if !RM_TRAV_PARK
-    double tmx = 0, tmy = 0, tmz = 0, tdx = 0, tdy = 0, tdz = 0;
-    int cx = 0, cy = 0, cz = 0, sx = 1, sy = 1, sz = 1;
-#endif
+    // DDA state of MY ray (acc_grid.rs:100-125): parked in sh.dda_t / dda_c / dda_s, in registers only during phase A
     const unsigned rx = (unsigned)g.res[0], ry = (unsigned)g.res[1], rz = (unsigned)g.res[2];
-#if RM_TRAV_PARK
     unsigned k = 0, cnt = 0;
-#else
-    unsigned ray = 0, k = 0, cnt = 0;
-#endif
     unsigned n_cells = 0, n_tests = 0, n_surv = 0, n_occ = 0, n_flops = 0;
 #if defined(RM_TRAV_PROFILE)
     unsigned long long prof[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -903,7 +852,6 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
                     const double* rec = a.trav + (size_t)idx * kTravDoubles;
                     double ox, oy, oz, dx, dy, dz, q0, q1, q2, q3;
                     ld256(rec, ox, oy, oz, dx);
-#if RM_TRAV_PARK
                     {
                         double t0, t1, t2, t3, t4, t5;
                         ld256(rec + 4, dy, dz, t0, t1);
@@ -914,19 +862,7 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
                         sh.dda_c[0][lane] = __double2loint(q0); sh.dda_c[1][lane] = __double2hiint(q0); sh.dda_c[2][lane] = __double2loint(q1);
                         sh.dda_s[lane] = (unsigned)__double2hiint(q1);
                     }
-#else
-                    ld256(rec + 4, dy, dz, tmx, tmy);
-                    ld256(rec + 8, tmz, tdx, tdy, tdz);
-                    ld256(rec + 12, q0, q1, q2, q3);
-                    cx = __double2loint(q0); cy = __double2hiint(q0); cz = __double2loint(q1);
-                    const unsigned neg = (unsigned)__double2hiint(q1);
-                    sx = (neg & 1u) ? -1 : 1; sy = (neg & 2u) ? -1 : 1; sz = (neg & 4u) ? -1 : 1;
-#endif
-#if RM_TRAV_PARK
                     sh.ray_index[lane] = (unsigned)__double2loint(q2);
-#else
-                    ray = (unsigned)__double2loint(q2);
-#endif
                     sh.best_obj[lane] = __double2hiint(q2);
                     sh.best_t[lane] = q3;
                     sh.ray[lane][0] = make_double2(ox, oy);
@@ -946,7 +882,6 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
         // so each iteration looks kLook cells ahead: the DDA is advanced kLook times in registers (the arithmetic is
         // cheap and exactly the reference's sequence), the kLook occupancy words are fetched together, and the ray
         // commits up to the first occupied cell (re-walking from the saved state) or all kLook empty ones.
-#if RM_TRAV_PARK
         double tmx = 0, tmy = 0, tmz = 0, tdx = 0, tdy = 0, tdz = 0;
         int cx = 0, cy = 0, cz = 0, sx = 1, sy = 1, sz = 1;
         const bool walking = state == TS_LOOK || state == TS_STEP;
@@ -957,7 +892,6 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
             const unsigned neg = sh.dda_s[lane];
             sx = (neg & 1u) ? -1 : 1; sy = (neg & 2u) ? -1 : 1; sz = (neg & 4u) ? -1 : 1;
         }
-#endif
 #pragma unroll 1
         for (unsigned it = 0; it < kTravMaxSteps; it++) {
             if (state == TS_LOOK) {                              // a fresh ray: its start cell, no step (acc_grid.rs:127-131)
@@ -1008,12 +942,10 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
             }
             if (!__any_sync(FULL, state == TS_STEP)) break;
         }
-#if RM_TRAV_PARK
         if (walking) {
             sh.dda_t[0][lane] = tmx; sh.dda_t[1][lane] = tmy; sh.dda_t[2][lane] = tmz;
             sh.dda_c[0][lane] = cx; sh.dda_c[1][lane] = cy; sh.dda_c[2][lane] = cz;
         }
-#endif
         // the cell records of every ray that found an occupied cell, in one round trip (not one per walk iteration)
         if (state == TS_READY) {
             const uint2 cell = __ldg(&g.cells[k]);
@@ -1031,9 +963,7 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
         }
         const unsigned total = __reduce_add_sync(FULL, mine);        // warp-uniform by construction (a uniform register, not one per lane)
         if (total == 0) continue;
-#if RM_TRAV_PARK
         sh.state[lane] = (unsigned char)state;                       // not needed until phase C
-#endif
         // The pool: items [excl, excl + mine) belong to this lane's cell.  Contributing lanes are compacted into
         // olane / odelta; a round of 32 consecutive items finds its owners with one ballot and one redux:
         //   first = contributors whose list starts at or before the round, bits = list starts inside the round
@@ -1041,9 +971,7 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
         // tests of locate() need no separate flag)
         {
             const unsigned excl = mine ? incl - mine : ~0u;
-#if RM_TRAV_EXCL_SHARED
             sh.excl[lane] = excl;
-#endif
             const unsigned contrib = __ballot_sync(FULL, mine != 0u);
             if (mine) {
                 const unsigned q = __popc(contrib & lt);
@@ -1051,24 +979,14 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
                 sh.odelta[q] = k - excl;
             }
         }
-#if !RM_TRAV_EXCL_SHARED
-        const unsigned excl = mine ? incl - mine : ~0u;
-#endif
         sh.cand_t[lane] = ~0ull;
         sh.cand_tri[lane] = ~0u;
-#if RM_TRAV_PARK
         sh.cell_t[lane] = kClosest0;                 // per-cell closest of MY ray
         sh.cell_tri[lane] = ~0u;
-#else
-        unsigned long long best_t = kClosest0;       // per-cell closest of MY ray
-        unsigned best_tri = ~0u;
-#endif
         __syncwarp();
         // (owner lane, list position) of item rbase + lane; rbase is warp-uniform and every lane takes part
         auto locate = [&](unsigned rbase, unsigned& owner, unsigned& pos) {
-#if RM_TRAV_EXCL_SHARED
             const unsigned excl = sh.excl[lane];
-#endif
             const unsigned first = __popc(__ballot_sync(FULL, excl <= rbase)) - 1u;
             const unsigned off = excl - rbase;                                   // 1..31 when my list starts inside the round
             const unsigned bits = __reduce_or_sync(FULL, (off - 1u < 31u) ? (1u << off) : 0u);
@@ -1155,11 +1073,7 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
                 __syncwarp();
                 // strict < against the earlier rounds (they hold earlier list positions) and against 5712515.0
                 const unsigned long long ct = sh.cand_t[lane];
-#if RM_TRAV_PARK
                 if (ct < sh.cell_t[lane]) { sh.cell_t[lane] = ct; sh.cell_tri[lane] = sh.cand_tri[lane]; }
-#else
-                if (ct < best_t) { best_t = ct; best_tri = sh.cand_tri[lane]; }
-#endif
                 sh.cand_t[lane] = ~0ull;
                 sh.cand_tri[lane] = ~0u;
             }
@@ -1168,22 +1082,16 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
         }
         RM_PROF_MARK(2);
         // ---- C
-#if RM_TRAV_PARK
         state = sh.state[lane];
-#endif
         if (state == TS_READY) {
-#if RM_TRAV_PARK
             const unsigned best_tri = sh.cell_tri[lane];
             const unsigned long long best_t = sh.cell_t[lane];
-#endif
             if (best_tri != ~0u) {
                 const double closest = __longlong_as_double((long long)best_t);
                 // the cell's closest hit is the grid's answer; merge with what the other objects found (the hit record of
                 // this ray as k_setup left it came in with the traversal record: no global read here)
                 if (closer(closest, a.grid_object, sh.best_t[lane], sh.best_obj[lane])) {
-#if RM_TRAV_PARK
                     const unsigned ray = sh.ray_index[lane];
-#endif
                     a.hit.t[ray] = closest; a.hit.obj[ray] = a.grid_object; a.hit.sub[ray] = best_tri;
                 }
                 state = TS_IDLE;
@@ -1222,7 +1130,7 @@ __global__ void __launch_bounds__(kTravBlock, RM_TRAV_BLOCKS_PER_SM) k_traverse(
 // exact (0, 0, 0) otherwise, so this instantiation reads only the hit object, the slot and the throughput of emitter hits,
 // and forms T (*) emission with the same multiplication as the general body.  No path continues and no triangle is shaded.
 template <bool FIRST, int PREC, bool KEEP, bool LAST>
-__global__ void __launch_bounds__(kBlock, RM_SHADE_BLOCKS_PER_SM) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
+__global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
                                                    const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first) {
     static_assert(!(LAST && KEEP), "keep mode computes the last weight: it has no last-depth shortcut");
     const unsigned n = FIRST ? n_first : rp.cnt.rays[depth - 1];

@@ -1,4 +1,6 @@
-"""Cycles per k_traverse phase (needs a library built with -DRM_TRAV_PROFILE; RAYMOND_CUDA_LIB selects it)."""
+"""Cycles per k_traverse phase, for the library named by RAYMOND_CUDA_LIB.  It needs the profiling build:
+    python -c 'from raymond_b200 import build; build.build(defines=["RM_TRAV_PROFILE"], out="/tmp/trav_profile.so")'
+    RAYMOND_CUDA_LIB=/tmp/trav_profile.so python scripts/trav_profile.py [spp]"""
 import ctypes as C, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from raymond_b200 import api as A, fixtures as F
