@@ -9,6 +9,8 @@
 // render — TileProgressed every --spi samples, then TileFinished — as one JSON text per line ("\r\n", like editor/src/main.js:35).
 // --adaptive T [--min-spp N] stops every tile at the first --spi checkpoint where its error estimate is <= T
 // (rm_render_tiled_adaptive) and prints the samples actually rendered.
+// --denoise [ITERATIONS] renders through rm_render_tiled_denoised and writes the filtered frame (the library's default sigmas;
+// ITERATIONS a-trous passes, 1 when omitted).
 // Compile:  g++ -O2 -std=c++17 -Iinclude examples/cli_old.cpp -Lraymond_b200 -lraymond_cuda -Wl,-rpath,$PWD/raymond_b200 -o cli_old
 #include <arpa/inet.h>
 #include <netinet/in.h>
@@ -40,6 +42,8 @@ int main(int argc, char** argv) {
     size_t spi = 0;
     double adaptive = 0.0;
     size_t min_spp = 0;
+    bool denoise = false;
+    rm_denoise_settings denoise_settings{1, 0, 1e4, 0.1, 0.3, 1.0};      // the defaults of include/raymond.h
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--mesh") && i + 1 < argc) mesh_path = argv[++i];
         else if (!strcmp(argv[i], "--out") && i + 1 < argc) out_path = argv[++i];
@@ -53,9 +57,12 @@ int main(int argc, char** argv) {
         else if (!strcmp(argv[i], "--spi") && i + 1 < argc) spi = strtoull(argv[++i], nullptr, 10);
         else if (!strcmp(argv[i], "--adaptive") && i + 1 < argc) adaptive = strtod(argv[++i], nullptr);
         else if (!strcmp(argv[i], "--min-spp") && i + 1 < argc) min_spp = strtoull(argv[++i], nullptr, 10);
-        else {
+        else if (!strcmp(argv[i], "--denoise")) {
+            denoise = true;
+            if (i + 1 < argc && argv[i + 1][0] >= '0' && argv[i + 1][0] <= '9') denoise_settings.iterations = (uint32_t)strtoul(argv[++i], nullptr, 10);
+        } else {
             fprintf(stderr, "usage: cli_old [--mesh dragon.ply] [--out output.png] [--width W --height H --spp N --seed S --gpus G --repeat R --serve PORT --spi N"
-                            " --adaptive T --min-spp N]\n");
+                            " --adaptive T --min-spp N --denoise [ITERATIONS]]\n");
             return 2;
         }
     }
@@ -141,6 +148,7 @@ int main(int argc, char** argv) {
         opt.seed = seed + rep;
         const rm_adaptive_settings adapt{adaptive, min_spp};
         rm_task* task = adaptive != 0.0 ? rm_render_tiled_adaptive(scene, &settings, &opt, &adapt)
+                        : denoise       ? rm_render_tiled_denoised(scene, &settings, &opt, &denoise_settings)
                                         : rm_render_tiled(scene, &settings, &opt);                   // :152
         if (!task) { fprintf(stderr, "render_tiled: %s\n", rm_last_error()); return 1; }
         lap("render_tiled returned");
@@ -181,6 +189,10 @@ int main(int argc, char** argv) {
             CHECK(rm_task_await(task, render.data()));                                        // :153
         }
         lap("await returned");
+        if (denoise) {
+            CHECK(rm_task_await_denoised(task, render.data()));                                // the filtered frame replaces the mean
+            lap("await_denoised returned");
+        }
         rm_task_stats(task, &stats);
         rm_task_destroy(task);
         fprintf(stderr, "[cli_old] frame %u: render_tiled + await %.3f s (device %.1f ms)\n", rep,

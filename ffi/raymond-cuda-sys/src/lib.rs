@@ -92,6 +92,12 @@ extern "C" {
     pub fn rm_renderer_read_aovs(r: *mut rm_renderer, sample_count: usize, albedo: *mut rm_vec3, normal: *mut rm_vec3, depth: *mut f64) -> c_int;
     // null settings = the defaults; needs RM_FLAG_AOV | RM_FLAG_MOMENTS, sample_count >= 2 and a renderer with world_size <= 1
     pub fn rm_renderer_read_denoised(r: *mut rm_renderer, sample_count: usize, settings: *const rm_denoise_settings, out: *mut rm_vec3) -> c_int;
+    // render_tiled that also filters the finished frame across the task's devices; messages and rm_task_await are rm_render_tiled's.
+    // null settings = the defaults; sample_count >= 2; not for one rank of a multi-process job
+    pub fn rm_render_tiled_denoised(s: *const rm_scene, st: *const rm_settings, o: *const rm_gpu_options,
+                                    d: *const rm_denoise_settings) -> *mut rm_task;
+    // blocks until the task is finished, then the W*H filtered frame; RM_ERR_STATE for a task not made by rm_render_tiled_denoised
+    pub fn rm_task_await_denoised(t: *mut rm_task, out: *mut rm_vec3) -> c_int;
 }
 
 // ---- values of the enum / flag fields (include/raymond.h, RM_ABI_VERSION 2)

@@ -234,8 +234,9 @@ typedef enum rm_precision {
  *           a sphere, the Heron-area triangle normal of a grid; emitters included),
  *   depth:  Hit.distance;
  * a miss contributes zeros.  The renderer keeps their running sums per pixel, added in global sample order like S, with no
- * non-finite filtering.  Read with rm_renderer_read_aovs; used by rm_renderer_read_denoised.  For rm_renderer_* only: a task
- * cannot read the sums, so rm_render_tiled and rm_render_tiled_adaptive refuse the flag with RM_ERR_UNSUPPORTED. */
+ * non-finite filtering.  Read with rm_renderer_read_aovs; used by rm_renderer_read_denoised.  A task reads the sums only to filter
+ * the frame (rm_render_tiled_denoised sets the flag on every share itself), so rm_render_tiled and rm_render_tiled_adaptive refuse
+ * the flag with RM_ERR_UNSUPPORTED. */
 #define RM_FLAG_AOV 128u
 
 /* GPU-side knobs that have no counterpart in the reference. Zero-initialise
@@ -420,6 +421,22 @@ typedef struct rm_denoise_settings {
  * valid settings (else RM_ERR_INVALID_ARGUMENT, before any device work); a renderer with world_size > 1 gets RM_ERR_UNSUPPORTED.
  * Tonemap the result with rm_tonemap_rgb8. */
 int rm_renderer_read_denoised(rm_renderer* r, size_t sample_count, const rm_denoise_settings* settings, rm_vec3* out_host);
+/* render_tiled whose shares also keep Q (RM_FLAG_MOMENTS) and the first-hit feature sums (RM_FLAG_AOV), and which, after the
+ * final accumulator exchange, runs the filter of rm_renderer_read_denoised on the whole frame across the task's devices.
+ * Messages, rm_task_await and rm_task_stats.samples are exactly rm_render_tiled's. `denoise` NULL = the defaults.
+ * The filter sees the sums of all shares added in device order (those of one device: the result equals rm_renderer_read_denoised
+ * of a renderer that rendered the same samples).  Share g of G filters rows [H*g/G, H*(g+1)/G), reading the rows its taps reach
+ * beyond them in place from the shares that own them, and writes its rows of the f64 frame straight to host memory; devices that
+ * cannot all map each other's memory (or more than 64 shares) gather the sums onto the first device and filter there.  The task
+ * is finished (rm_task_finished, rm_task_await) once the filtered frame is ready; the filter's kernels count in kernel_launches.
+ * Checked before any device work, in this order: a null scene or settings and the camera checks of rm_render_tiled, then
+ * sample_count < 2 and invalid settings (as rm_renderer_read_denoised) fail with RM_ERR_INVALID_ARGUMENT; one rank of a
+ * multi-process job (world_size > 1 with device_count <= 1) with RM_ERR_UNSUPPORTED. */
+rm_task* rm_render_tiled_denoised(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options,
+                                  const rm_denoise_settings* denoise);
+/* Blocks until the task is finished, then writes the W*H filtered frame (row-major) to HOST memory.
+ * RM_ERR_STATE for a task not created by rm_render_tiled_denoised. */
+int rm_task_await_denoised(rm_task* task, rm_vec3* out_host);
 int rm_renderer_stats(rm_renderer* r, rm_stats* out);
 
 /* Per-stage breakdown of the wavefront.  Slot d (1 <= d < RM_STAGE_SLOTS) is the stage that traces

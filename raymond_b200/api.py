@@ -150,7 +150,7 @@ ABI_SYMBOLS = [
     "rm_renderer_stats", "rm_renderer_stage_stats", "rm_renderer_destroy", "rm_tile_layout", "rm_renderer_read_rgb8", "rm_tonemap_rgb8",
     "rm_write_png", "rm_project_load_scene", "rm_message_to_json", "rm_release_cached_memory", "rm_measure_fp64_rate",
     "rm_render_tiled_adaptive", "rm_renderer_read_moments", "rm_renderer_tile_errors", "rm_renderer_set_active_tiles",
-    "rm_renderer_read_aovs", "rm_renderer_read_denoised",
+    "rm_renderer_read_aovs", "rm_renderer_read_denoised", "rm_render_tiled_denoised", "rm_task_await_denoised",
 ]
 
 _lib = None
@@ -198,6 +198,8 @@ def lib():
         "rm_renderer_set_active_tiles": (i32, [vp, vp, sz]),
         "rm_renderer_read_aovs": (i32, [vp, sz, vp, vp, vp]),
         "rm_renderer_read_denoised": (i32, [vp, sz, P(DenoiseSettingsC), vp]),
+        "rm_render_tiled_denoised": (vp, [vp, P(SettingsC), P(GpuOptionsC), P(DenoiseSettingsC)]),
+        "rm_task_await_denoised": (i32, [vp, vp]),
         "rm_task_poll": (i32, [vp, P(MessageC)]),
         "rm_task_await": (i32, [vp, vp]),
         "rm_task_set_callback": (i32, [vp, TILE_CALLBACK, vp]),
@@ -592,16 +594,27 @@ class TaskHandle:
         lib().rm_tile_free(C.byref(m.tile))
         return msg
 
-    def await_(self, out: Optional[np.ndarray] = None) -> np.ndarray:
-        """r#await(): block, then the averaged frame as (H, W, 3) f64 (row-major W*H Vec<Vector3>).  `out` = a C-contiguous f64
-        array of that shape to write into (a caller rendering frame after frame keeps one, as the C ABI's caller does)."""
+    def _out(self, out: Optional[np.ndarray], who: str) -> np.ndarray:
         cs = self.settings.camera_settings
         shape = (cs.backbuffer_height, cs.backbuffer_width, 3)
         if out is None:
-            out = np.zeros(shape)
-        elif out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
-            raise ValueError(f"await_: out must be a C-contiguous float64 array of shape {shape}")
+            return np.zeros(shape)
+        if out.shape != shape or out.dtype != np.float64 or not out.flags.c_contiguous:
+            raise ValueError(f"{who}: out must be a C-contiguous float64 array of shape {shape}")
+        return out
+
+    def await_(self, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """r#await(): block, then the averaged frame as (H, W, 3) f64 (row-major W*H Vec<Vector3>).  `out` = a C-contiguous f64
+        array of that shape to write into (a caller rendering frame after frame keeps one, as the C ABI's caller does)."""
+        out = self._out(out, "await_")
         _check(lib().rm_task_await(self._h, _ptr(out)))
+        return out
+
+    def await_denoised(self, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """Block, then the filtered frame of a render_tiled(..., denoise=...) task as (H, W, 3) f64; `out` as for await_().
+        RM_ERR_STATE for a task rendered without denoise."""
+        out = self._out(out, "await_denoised")
+        _check(lib().rm_task_await_denoised(self._h, _ptr(out)))
         return out
 
     def set_callback(self, callback: Optional[Callable[[Tile], None]]) -> None:
@@ -658,12 +671,21 @@ class DenoiseSettings:
 
 
 def render_tiled(scene: Scene, settings: Settings, options: Optional[GpuOptions] = None,
-                 adaptive: Optional[AdaptiveSettings] = None) -> TaskHandle:
+                 adaptive: Optional[AdaptiveSettings] = None, denoise=None) -> TaskHandle:
     """render_tiled(scene, settings) -> TaskHandle (src/trace.rs:137-230). Returns immediately.  `adaptive` adds per-tile early
-    stopping at the samples_per_iteration checkpoints (rm_render_tiled_adaptive); read such a task with poll() or await_()."""
+    stopping at the samples_per_iteration checkpoints (rm_render_tiled_adaptive); read such a task with poll() or await_().
+    `denoise` (a DenoiseSettings, or True for the library's defaults) also filters the finished frame across the task's devices
+    (rm_render_tiled_denoised): read it with await_denoised(); messages and await_() stay those of the plain render."""
+    if adaptive is not None and denoise is not None:
+        raise ValueError("render_tiled: adaptive and denoise cannot be combined (an adaptive task's tiles stop at different counts)")
+    if denoise is not None and denoise is not True and not isinstance(denoise, DenoiseSettings):
+        raise TypeError("render_tiled: denoise must be a DenoiseSettings or True")
     s = settings._c()
     o = (options or GpuOptions())._c()
-    if adaptive is None:
+    if denoise is not None:
+        d = None if denoise is True else C.byref(denoise._c())
+        h = _require(lib().rm_render_tiled_denoised(scene._h, C.byref(s), C.byref(o), d), "render_tiled_denoised")
+    elif adaptive is None:
         h = _require(lib().rm_render_tiled(scene._h, C.byref(s), C.byref(o)), "render_tiled")
     else:
         a = adaptive._c()

@@ -1185,6 +1185,99 @@ int tile_errors_to_host(rm_renderer* const* rs, int count, size_t n, double* out
     return st;
 }
 
+// The sliced filter: stage 0 reduces and packs every share's rows, stage i + 1 is pass i.  A stage reads what the previous one
+// wrote, in place on every peer, and overwrites the colour plane the previous one read, so every share's stage waits for every
+// share's previous stage (cross-device events, as the accumulator exchange orders itself).
+static int denoise_sliced(rm_renderer* const* rs, int count, size_t n, const rm_denoise_settings& s, rm_vec3* out_dev) {
+    const size_t W = rs[0]->settings.camera_settings.backbuffer_width, H = rs[0]->settings.camera_settings.backbuffer_height;
+    DenoiseSlices d{};
+    d.count = count;
+    std::vector<size_t> bytes(count);
+    cudaError_t e = cudaSuccess;
+    for (int g = 0; g < count; g++) {
+        d.sums[g] = rs[g]->accum;
+        d.moments[g] = rs[g]->moments;
+        d.aov[g] = rs[g]->aov;
+    }
+    // not from the pool: peers read the packed rows in place
+    for (int g = 0; g < count && e == cudaSuccess; g++) {
+        bytes[g] = std::max<size_t>((slice_begin(H, g + 1, count) - slice_begin(H, g, count)) * W, 1) * 4 * sizeof(float4);
+        e = cudaSetDevice(rs[g]->device);
+        if (e == cudaSuccess) e = visible_acquire(rs[g]->device, bytes[g], &d.packed[g]);
+    }
+    for (int g = 0; g < count && e == cudaSuccess; g++) {       // the sums every share reads are complete
+        e = cudaSetDevice(rs[g]->device);
+        if (e == cudaSuccess && !rs[g]->ev_rendered) e = cudaEventCreateWithFlags(&rs[g]->ev_rendered, cudaEventDisableTiming);
+        if (e == cudaSuccess) e = cudaEventRecord(rs[g]->ev_rendered, rs[g]->stream);
+    }
+    for (uint32_t stage = 0; stage <= s.iterations && e == cudaSuccess; stage++) {
+        // all waits of a stage are enqueued before any share records the stage's event
+        for (int g = 0; g < count && e == cudaSuccess; g++) {
+            e = cudaSetDevice(rs[g]->device);
+            for (int j = 0; j < count && e == cudaSuccess; j++)
+                if (j != g) e = cudaStreamWaitEvent(rs[g]->stream, rs[j]->ev_rendered, 0);
+        }
+        for (int g = 0; g < count && e == cudaSuccess; g++) {
+            rm_renderer* r = rs[g];
+            e = cudaSetDevice(r->device);
+            if (e == cudaSuccess)
+                e = (cudaError_t)(stage == 0 ? denoise_reduce_slice(d, g, W, H, (double)n, r->stream)
+                                             : denoise_pass_slice(d, g, W, H, stage - 1, s, stage == s.iterations ? out_dev : nullptr, r->stream));
+            if (e == cudaSuccess && slice_begin(H, g + 1, count) > slice_begin(H, g, count)) r->launches++;
+            if (e == cudaSuccess) e = cudaEventRecord(r->ev_rendered, r->stream);
+        }
+    }
+    for (int g = 0; g < count; g++) {           // before the packed rows go back to the cache
+        cudaSetDevice(rs[g]->device);
+        const cudaError_t done = cudaStreamSynchronize(rs[g]->stream);
+        if (e == cudaSuccess) e = done;
+    }
+    for (int g = 0; g < count; g++) visible_release(rs[g]->device, bytes[g], d.packed[g]);
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("sliced denoiser: ") + cudaGetErrorString(e));
+    return RM_OK;
+}
+
+int denoise_shares_to_host(rm_renderer* const* rs, int count, size_t n, const rm_denoise_settings& s, rm_vec3* out_pinned) {
+    if (count <= 0 || !rs || !out_pinned) return fail(RM_ERR_INVALID_ARGUMENT, "denoise_shares_to_host: bad argument");
+    for (int g = 0; g < count; g++)
+        if (!rs[g]->aov || !rs[g]->moments) return fail(RM_ERR_STATE, "the denoiser needs RM_FLAG_AOV and RM_FLAG_MOMENTS");
+    rm_renderer* r0 = rs[0];
+    const size_t W = r0->settings.camera_settings.backbuffer_width, H = r0->settings.camera_settings.backbuffer_height, np = W * H;
+    RM_CUDA(cudaSetDevice(r0->device));
+    rm_vec3* out_dev = nullptr;      // the frame as the devices see it (the same address under unified addressing)
+    RM_CUDA(cudaHostGetDevicePointer((void**)&out_dev, (void*)out_pinned, 0));
+    if (count == 1) {
+        const int st = denoise_to_host(r0->accum, r0->moments, r0->aov, W, H, (double)n, s, out_dev, r0->stream);
+        if (st == RM_OK) r0->launches += 1 + s.iterations;
+        return st;
+    }
+    if (peers_mapped(rs, count)) return denoise_sliced(rs, count, n, s, out_dev);
+    // no peer mapping (or more shares than one kernel takes): S, Q and the features staged onto the first device
+    for (int g = 0; g < count; g++) {
+        RM_CUDA(cudaSetDevice(rs[g]->device));
+        RM_CUDA(cudaStreamSynchronize(rs[g]->stream));
+    }
+    RM_CUDA(cudaSetDevice(r0->device));
+    double *S = nullptr, *Q = nullptr, *A = nullptr, *part = nullptr;
+    cudaError_t e = dev_malloc(&S, np * 3 * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&Q, np * 3 * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&A, np * 7 * sizeof(double));
+    if (e == cudaSuccess) e = dev_malloc(&part, np * 7 * sizeof(double));
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::accum, S, part, np * 3);
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::moments, Q, part, np * 3);
+    if (e == cudaSuccess) e = stage_sum(rs, count, &rm_renderer::aov, A, part, np * 7);
+    int st = RM_OK;
+    if (e == cudaSuccess) {
+        st = denoise_to_host(S, Q, A, W, H, (double)n, s, out_dev, r0->stream);
+        if (st == RM_OK) r0->launches += 1 + s.iterations;
+    }
+    const cudaError_t done = cudaStreamSynchronize(r0->stream);      // before the staging buffers go back to the pool
+    if (e == cudaSuccess) e = done;
+    dev_free(S); dev_free(Q); dev_free(A); dev_free(part);
+    if (e != cudaSuccess) return fail(RM_ERR_CUDA, std::string("staged denoiser: ") + cudaGetErrorString(e));
+    return st;
+}
+
 }  // namespace rm
 
 // ===================================================================== C ABI (device level)
@@ -1450,22 +1543,17 @@ int rm_renderer_read_denoised(rm_renderer* r, size_t sample_count, const rm_deno
     if (!r->aov || !r->moments) return fail(RM_ERR_STATE, "rm_renderer_read_denoised: needs a renderer created with RM_FLAG_AOV and RM_FLAG_MOMENTS");
     if (r->opt.world_size > 1) return fail(RM_ERR_UNSUPPORTED, "rm_renderer_read_denoised: the filter needs the whole frame's sums (world_size > 1)");
     if (sample_count < 2) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_denoised: the variance needs sample_count >= 2");
-    rm_denoise_settings s{1, 0, 1e4, 0.1, 0.3, 1.0};       // the defaults stated in include/raymond.h
-    if (settings) s = *settings;
-    // the filter uses each sigma as an f32, and the squares of sigma_normal and sigma_albedo: all of them must be normal f32 values
-    // (a square that underflows to 0 or a sigma that overflows to inf would make the centre tap's weight NaN)
-    const auto usable = [](double x, bool squared) {
-        const float f = (float)x, g = squared ? f * f : f;
-        return std::isfinite(x) && x > 0.0 && std::isfinite(g) && g >= FLT_MIN;
-    };
-    if (s.iterations < 1 || s.iterations > 10 || !usable(s.sigma_color, false) || !usable(s.sigma_normal, true) || !usable(s.sigma_albedo, true) ||
-        !usable(s.sigma_depth, false))
-        return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_read_denoised: iterations outside 1..10 or a sigma outside the f32 range the filter needs");
+    rm_denoise_settings s;
+    if (int st = resolve_denoise_settings(settings, &s, "rm_renderer_read_denoised")) return st;
     RM_CUDA(cudaSetDevice(r->device));
-    const size_t W = r->settings.camera_settings.backbuffer_width, H = r->settings.camera_settings.backbuffer_height;
-    const int st = denoise_to_host(r->accum, r->moments, r->aov, W, H, (double)sample_count, s, out, r->stream);
+    const size_t n = r->settings.camera_settings.backbuffer_width * r->settings.camera_settings.backbuffer_height;
+    // the last pass writes the f64 frame into a pinned block; a copy moves it on to the caller's memory
+    rm_vec3* pin = (rm_vec3*)pinned_acquire(std::max<size_t>(n, 1) * sizeof(rm_vec3));
+    if (!pin) return fail(RM_ERR_CUDA, std::string("denoiser: ") + cudaGetErrorString(cudaErrorMemoryAllocation));
+    const int st = denoise_shares_to_host(&r, 1, sample_count, s, pin);
     harvest_events(r);
-    if (st == RM_OK) r->launches += 1 + s.iterations;
+    if (st == RM_OK) memcpy((void*)out, (const void*)pin, n * sizeof(rm_vec3));
+    pinned_release(pin);
     return st;
 }
 

@@ -124,10 +124,42 @@ int reduce_accumulators_to_host(rm_renderer* const* renderers, int count, rm_vec
 int tile_errors_to_host(rm_renderer* const* renderers, int count, size_t n, double* out_pinned, size_t n_tiles, size_t first, size_t step);
 // display transform kernel (rm_display.cu): sums / divisor -> tonemap -> 8-bit RGB, device pointers
 int tonemap_device(const double* sums_device, size_t n_pixels, double divisor, double exposure, double gamma, unsigned char* out_device, void* stream);
-// the a-trous denoiser (rm_display.cu, rm_renderer_read_denoised): from the device sums S, Q and the RM_FLAG_AOV planes of a W x H
-// frame after n samples to W*H denoised means in HOST memory, on `stream`.  Synchronous; launches 1 + s.iterations kernels.
+
+// ---- the a-trous denoiser of rm_renderer_read_denoised and rm_render_tiled_denoised (kernels in rm_display.cu)
+// `settings` NULL = the defaults of include/raymond.h; RM_ERR_INVALID_ARGUMENT (no device work) for iterations outside 1..10 or a
+// sigma the f32 filter cannot use.  `who` names the entry point in the message.
+int resolve_denoise_settings(const rm_denoise_settings* settings, rm_denoise_settings* out, const char* who);
+// The whole filter on one device: from the device sums S, Q and the RM_FLAG_AOV planes of a W x H frame after n samples to W*H
+// denoised means, written as f64 by the last pass into `out_mapped` (the device address of a pinned, mapped host frame), on `stream`.
+// Synchronous; launches 1 + s.iterations kernels.
 int denoise_to_host(const double* sums, const double* moments, const double* aov, size_t W, size_t H, double n, const rm_denoise_settings& s,
-                    rm_vec3* out_host, void* stream);
+                    rm_vec3* out_mapped, void* stream);
+// The same filter with the frame sliced by rows over the shares of a task: share g of count owns rows [H*g/count, H*(g+1)/count).
+// Every share's sums (whole-frame planes, zeros where it rendered nothing) and packed rows are read in place by the other shares'
+// kernels (peer mappings): `packed[g]` holds 4 planes of (rows of g) * W float4 — colour + variance ping, pong, albedo + depth,
+// normal — from the peer-visible block cache.
+constexpr int kMaxShares = 64;      // pointers one kernel parameter block takes per kind of buffer
+struct DenoiseSlices {
+    const double* sums[kMaxShares];
+    const double* moments[kMaxShares];
+    const double* aov[kMaxShares];
+    void* packed[kMaxShares];
+    int count;
+};
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+inline size_t slice_begin(size_t H, size_t g, size_t count) { return H * g / count; }
+// Launchers of one share's part (0 = launched or nothing to do, else a cudaError_t value).  denoise_reduce_slice: its rows of S, Q and
+// the features summed over all shares in share order, packed as the one-device filter packs them.  denoise_pass_slice: pass `pass`
+// (step 2^pass) of its rows, taps read from whichever share owns them; `out_mapped` non-NULL: the result goes there as f64 instead.
+int denoise_reduce_slice(const DenoiseSlices& d, int share, size_t W, size_t H, double n, void* stream);
+int denoise_pass_slice(const DenoiseSlices& d, int share, size_t W, size_t H, uint32_t pass, const rm_denoise_settings& s, rm_vec3* out_mapped,
+                       void* stream);
+// The filter over the sums of several renderers (rm_device.cu; one renderer: rm_renderer_read_denoised).  Sliced as above when every
+// device maps every other's memory and count <= kMaxShares; otherwise S, Q and the features are staged onto the first device and the
+// one-device filter runs there.  The W*H result lands in `out_pinned` (a pinned_acquire block).  Synchronous.
+int denoise_shares_to_host(rm_renderer* const* renderers, int count, size_t n, const rm_denoise_settings& s, rm_vec3* out_pinned);
 // Device memory from the cached stream-ordered pool (rm_device.cu); dev_alloc returns a cudaError_t value (0 = ok).
 int dev_alloc(void** p, size_t bytes);
 void dev_release(void* p);

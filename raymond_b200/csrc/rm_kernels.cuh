@@ -1268,7 +1268,6 @@ __global__ void __launch_bounds__(kBlock) k_aov(const __grid_constant__ DevScene
 }
 
 // Sums of several renderers' accumulators (and second moments), read in place in device order like the accumulator exchange.
-constexpr int kMaxShares = 64;
 struct ShareMoments {
     const double* acc[kMaxShares];
     const double* mom[kMaxShares];

@@ -7,6 +7,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 
 #include "rm_internal.hpp"
 
@@ -52,6 +53,9 @@ struct rm_task {
     void* callback_user = nullptr;
     bool adaptive = false;          // rm_render_tiled_adaptive with settings
     rm_adaptive_settings adaptive_settings{};
+    bool denoise = false;           // rm_render_tiled_denoised: the filter runs after the final exchange
+    rm_denoise_settings denoise_settings{};
+    rm_vec3* denoised = nullptr;    // ... into this pinned W * H frame
 };
 
 namespace {
@@ -185,6 +189,12 @@ void drive(rm_task* t) {
             }
             trace.mark("driver: TileFinished messages posted");
         }
+        if (st == RM_OK && t->denoise) {
+            t->denoised = (rm_vec3*)pinned_acquire(std::max<size_t>(W * H, 1) * sizeof(rm_vec3));
+            if (!t->denoised) throw std::bad_alloc();
+            st = denoise_shares_to_host(t->renderers.data(), (int)G, total, t->denoise_settings, t->denoised);
+            trace.mark("driver: denoised frame on the host");
+        }
     } catch (const std::bad_alloc&) {
         st = fail(RM_ERR_OUT_OF_MEMORY, "out of host memory in the render driver");
     }
@@ -207,8 +217,10 @@ void drive(rm_task* t) {
     t->cv.notify_all();
 }
 
-// render_tiled; `adaptive` (optional, validated by the caller) adds per-tile early stopping, for which every share keeps Q
-rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive) {
+// render_tiled; `adaptive` (optional, validated by the caller) adds per-tile early stopping, for which every share keeps Q;
+// `denoise` (optional, validated) the filter of the whole frame, for which every share keeps Q and the feature sums
+rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_adaptive_settings* adaptive,
+                     const rm_denoise_settings* denoise = nullptr) {
     rm_task* t = new rm_task();
     t->settings = *settings;
     if (options) t->options = *options;
@@ -216,6 +228,11 @@ rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const r
         t->adaptive = true;
         t->adaptive_settings = *adaptive;
         t->options.flags |= RM_FLAG_MOMENTS;
+    }
+    if (denoise) {
+        t->denoise = true;
+        t->denoise_settings = *denoise;
+        t->options.flags |= RM_FLAG_AOV | RM_FLAG_MOMENTS;
     }
     const size_t G = t->options.device_count > 1 ? t->options.device_count : 1;
     if (G > 1 && (t->options.world_size > 1 || t->options.stream || t->options.accum_device)) {
@@ -294,11 +311,23 @@ rm_task* create_task(const rm_scene* scene, const rm_settings* settings, const r
     return t;
 }
 
-// A task has no reader of the first-hit feature sums: RM_FLAG_AOV would cost a kernel per batch and 56 B per pixel for nothing.
+// Only a denoised task reads the first-hit feature sums: elsewhere RM_FLAG_AOV would cost a kernel per batch and 56 B per pixel
+// for nothing.
 bool refuse_aov(const rm_gpu_options* options, const char* who) {
     if (!options || !(options->flags & RM_FLAG_AOV)) return false;
-    fail(RM_ERR_UNSUPPORTED, std::string(who) + ": RM_FLAG_AOV is for rm_renderer_* (a task cannot read the feature sums)");
+    fail(RM_ERR_UNSUPPORTED, std::string(who) + ": RM_FLAG_AOV is for rm_renderer_* (this task cannot read the feature sums; "
+                             "rm_render_tiled_denoised keeps them and filters the frame)");
     return true;
+}
+
+// rows(y0, y1) over the rows of a W x H frame, split between a few host threads when the frame is large
+void by_row_ranges(size_t W, size_t H, const std::function<void(size_t, size_t)>& rows) {
+    const unsigned hw = std::thread::hardware_concurrency();
+    const size_t workers = W * H < ((size_t)1 << 18) ? 1 : std::min<size_t>(hw ? hw : 4, 8);
+    std::vector<std::thread> pool;
+    for (size_t w = 1; w < workers; w++) pool.emplace_back(rows, H * w / workers, H * (w + 1) / workers);
+    rows(0, H / workers);
+    for (std::thread& th : pool) th.join();
 }
 
 }  // namespace
@@ -331,6 +360,19 @@ rm_task* rm_render_tiled_adaptive(const rm_scene* scene, const rm_settings* sett
         }
     }
     return create_task(scene, settings, options, adaptive);
+}
+
+rm_task* rm_render_tiled_denoised(const rm_scene* scene, const rm_settings* settings, const rm_gpu_options* options, const rm_denoise_settings* denoise) {
+    if (!scene || !settings) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_denoised: null argument"); return nullptr; }
+    if (validate_camera(settings->camera_settings, "rm_render_tiled_denoised") != RM_OK) return nullptr;
+    if (settings->sample_count < 2) { fail(RM_ERR_INVALID_ARGUMENT, "rm_render_tiled_denoised: the variance needs sample_count >= 2"); return nullptr; }
+    rm_denoise_settings s;
+    if (resolve_denoise_settings(denoise, &s, "rm_render_tiled_denoised") != RM_OK) return nullptr;
+    if (options && options->world_size > 1 && options->device_count <= 1) {
+        fail(RM_ERR_UNSUPPORTED, "rm_render_tiled_denoised: one rank of a multi-process job cannot see the other ranks' sums");
+        return nullptr;
+    }
+    return create_task(scene, settings, options, nullptr, &s);
 }
 
 int rm_task_poll(rm_task* t, rm_message* out) {
@@ -389,13 +431,25 @@ int rm_task_await(rm_task* t, rm_vec3* out) {
             }
         }
     };
-    const unsigned hw = std::thread::hardware_concurrency();
-    const size_t workers = W * H < ((size_t)1 << 18) ? 1 : std::min<size_t>(hw ? hw : 4, 8);
-    std::vector<std::thread> pool;
-    for (size_t w = 1; w < workers; w++) pool.emplace_back(rows, H * w / workers, H * (w + 1) / workers);
-    rows(0, H / workers);
-    for (std::thread& th : pool) th.join();
+    by_row_ranges(W, H, rows);
     trace.mark("await: averaged frame written");
+    return RM_OK;
+}
+
+int rm_task_await_denoised(rm_task* t, rm_vec3* out) {
+    if (!t || !out) return fail(RM_ERR_INVALID_ARGUMENT, "rm_task_await_denoised: null argument");
+    if (!t->denoise) return fail(RM_ERR_STATE, "rm_task_await_denoised: the task was not created by rm_render_tiled_denoised");
+    Trace trace;
+    {
+        std::unique_lock<std::mutex> lk(t->mu);
+        t->cv.wait(lk, [&] { return t->finished; });
+        if (t->status != RM_OK) return fail(t->status, t->error);
+    }
+    trace.mark("await_denoised: render and filter finished");
+    // the filter's last pass wrote the f64 frame on the devices: rows are copied
+    const size_t W = t->settings.camera_settings.backbuffer_width, H = t->settings.camera_settings.backbuffer_height;
+    by_row_ranges(W, H, [&](size_t y0, size_t y1) { memcpy((void*)(out + y0 * W), (const void*)(t->denoised + y0 * W), (y1 - y0) * W * sizeof(rm_vec3)); });
+    trace.mark("await_denoised: filtered frame written");
     return RM_OK;
 }
 
@@ -451,6 +505,7 @@ void rm_task_destroy(rm_task* t) {
     if (!t) return;
     if (t->driver.joinable()) t->driver.join();
     for (rm_renderer* r : t->renderers) rm_renderer_destroy(r);
+    pinned_release(t->denoised);
     delete t;
 }
 
