@@ -89,6 +89,8 @@ def lib():
     L.rmo_camera_rays.argtypes = [C.POINTER(CameraC), C.c_uint64, C.c_uint32, vp]
     L.rmo_rng_draw.restype = C.c_double
     L.rmo_rng_draw.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]
+    L.rmo_rng_draw_f32.restype = C.c_double
+    L.rmo_rng_draw_f32.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]
     L.rmo_tile_layout.restype = sz
     L.rmo_tile_layout.argtypes = [C.POINTER(SettingsC), vp, sz]
     L.rmo_render.restype = C.c_int
@@ -307,8 +309,15 @@ def camera_rays(cam: dict, seed: int, sample: int) -> np.ndarray:
     return out
 
 
-def rng_draw(seed, pixel, sample, depth, index) -> float:
-    return float(lib().rmo_rng_draw(seed, pixel, sample, depth, index))
+DRAWS = ("f64", "f32")
+
+
+def rng_draw(seed, pixel, sample, depth, index, draws: str = "f64") -> float:
+    """Draw `index` of (seed; pixel, sample, depth).  draws="f32": the stream of the product's f32 shading mode (23-bit
+    uniforms, all three shading draws of a depth from one Philox block); its camera draws (depth 0) are the f64 ones."""
+    assert draws in DRAWS, draws
+    f = lib().rmo_rng_draw_f32 if draws == "f32" else lib().rmo_rng_draw
+    return float(f(seed, pixel, sample, depth, index))
 
 
 def tile_layout(cam: dict, tile_size) -> np.ndarray:
@@ -320,13 +329,16 @@ def tile_layout(cam: dict, tile_size) -> np.ndarray:
 
 
 def render(scene: Scene, cam: dict, sample_count: int, *, seed: int = 0, tile_size=(32, 32), bounce_limit: int = 5,
-           worker_count: int = 0, first_sample: int = 0, sample_stride: int = 1, drop_nonfinite: bool = True):
-    """render_tiled + await.  Returns (running sums H x W x 3, counters)."""
+           worker_count: int = 0, first_sample: int = 0, sample_stride: int = 1, drop_nonfinite: bool = True, draws: str = "f64"):
+    """render_tiled + await.  Returns (running sums H x W x 3, counters).  draws="f32": the shading draws are those of the
+    product's f32 shading mode (see rng_draw), so that mode can be compared path for path; the arithmetic stays f64."""
+    assert draws in DRAWS, draws
     s = settings_c(cam, sample_count, tile_size, bounce_limit, worker_count)
     W, H = s.camera.width, s.camera.height
     out = np.zeros((H, W, 3))
     cnt = CountersC()
-    rc = lib().rmo_render(scene._h, C.byref(s), seed, first_sample, sample_stride, 1 if drop_nonfinite else 0, _ptr(out), C.byref(cnt))
+    rc = lib().rmo_render(scene._h, C.byref(s), seed, first_sample, sample_stride,
+                          (1 if drop_nonfinite else 0) | (2 if draws == "f32" else 0), _ptr(out), C.byref(cnt))
     if rc != 0:
         raise OracleError(rc, "render")
     return out, cnt.as_dict()

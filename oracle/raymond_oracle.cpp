@@ -27,6 +27,10 @@
 // same uniforms from a counter-based Philox4x32-10 stream keyed by
 // (seed; pixel, sample, depth, draw index) so that a CUDA render can be compared
 // sample-for-sample.  All citations are relative to the reference checkout.
+//
+// The f32-draw mode (bit 1 of rmo_render's flags) exists only to give the product's f32 shading mode
+// (RM_PRECISION_F32_SHADING) a same-stream reference: the shading draws of depth >= 1 are that mode's 23-bit uniforms
+// instead of the 52-bit ones, and everything else, the arithmetic included, stays this file's f64 restatement.
 
 #include <algorithm>
 #include <atomic>
@@ -612,11 +616,22 @@ inline double u52(uint32_t hi, uint32_t lo) {
     uint64_t bits = ((uint64_t)hi << 32) | lo;
     return ((double)(bits >> 12) + 0.5) * (1.0 / 4503599627370496.0);
 }
+// 23 random bits -> (k + 0.5) * 2^-23, the f32 shading mode's uniform; exact as a double
+inline double u23(uint32_t x) {
+    return ((double)(x >> 9) + 0.5) * (1.0 / 8388608.0);
+}
 // Stands in for rand::random::<f64>(): draw number `index` of (pixel, sample, depth).
+// f32_draws: the shading draws (depth >= 1) are those of the product's f32 shading mode, all three from one Philox block:
+// the lobe choice from word 0, the next draw (diffuse theta / specular phi) from word 2, the last (diffuse phi / GGX theta)
+// from word 1.  Camera draws (depth 0) are the 52-bit ones in both modes.
 struct Sampler {
-    uint64_t seed; uint32_t pixel; uint32_t sample;
+    uint64_t seed; uint32_t pixel; uint32_t sample; bool f32_draws = false;
     double draw(uint32_t depth, uint32_t index) const {
         uint32_t w[4];
+        if (f32_draws && depth >= 1) {
+            Philox::block(seed, pixel, sample, depth, 0, w);
+            return u23(w[index == 0 ? 0 : (index == 1 ? 2 : 1)]);
+        }
         Philox::block(seed, pixel, sample, depth, index >> 1, w);
         return (index & 1) ? u52(w[2], w[3]) : u52(w[0], w[1]);
     }
@@ -972,6 +987,10 @@ void rmo_camera_rays(const rmo_camera* cam, uint64_t seed, uint32_t sample, rmo_
 double rmo_rng_draw(uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t depth, uint32_t index) {
     return Sampler{seed, pixel, sample}.draw(depth, index);
 }
+// the same draw of the f32-draw stream (the product's f32 shading mode); index 0..2
+double rmo_rng_draw_f32(uint64_t seed, uint32_t pixel, uint32_t sample, uint32_t depth, uint32_t index) {
+    return Sampler{seed, pixel, sample, true}.draw(depth, index);
+}
 
 size_t rmo_tile_layout(const rmo_settings* s, size_t* rects, size_t capacity) {
     Settings st = tosettings(*s);
@@ -988,6 +1007,7 @@ size_t rmo_tile_layout(const rmo_settings* s, size_t* rects, size_t capacity) {
 // and retire for good the first time they find the queue empty (:189-195).
 //   first_sample/sample_stride: global sample index of pass k is first + k*stride
 //   flags bit 0: drop (and count) non-finite samples instead of accumulating them
+//   flags bit 1: the f32-draw stream (see Sampler)
 //   out_sum: W*H*3 running sums (row-major) — divide by sample_count for await()'s output
 int rmo_render(const rmo_scene* scene, const rmo_settings* s, uint64_t seed, uint32_t first_sample, uint32_t sample_stride,
                uint32_t flags, double* out_sum, rmo_counters* counters) {
@@ -1017,7 +1037,7 @@ int rmo_render(const rmo_scene* scene, const rmo_settings* s, uint64_t seed, uin
                 uint32_t sample = first_sample + (uint32_t)tile.sample_count * sample_stride;
                 for (size_t y = tile.top; y < tile.top + tile.height; y++) {
                     for (size_t x = tile.left; x < tile.left + tile.width; x++) {
-                        Sampler rng{seed, (uint32_t)(x + y * W), sample};
+                        Sampler rng{seed, (uint32_t)(x + y * W), sample, (flags & 2u) != 0};
                         Ray primary = camera_ray(x, y, settings.camera_settings, rng);
                         V3 smp = trace(primary, ctx, 1, rng);
                         tl_counters.samples++;

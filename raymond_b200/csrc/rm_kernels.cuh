@@ -543,9 +543,11 @@ __device__ __forceinline__ void lobe_f64(const RenderParams& rp, D3 normal, D3 t
 }
 
 // The same bounce with the statistical scope in f32 (RM_PRECISION_F32_SHADING): same formulas, same lobe probabilities, 23-bit
-// uniforms from one Philox call, FMAs, rsqrt normalisations.  The result agrees with lobe_f64 to ~1e-6 relative, i.e. far
-// inside the Monte-Carlo noise the image tolerance of SURVEY 8d is defined by; the direction is re-normalised in f64 so the
-// intersection code downstream still sees |d| = 1 to f64 accuracy.
+// uniforms from one Philox call, FMAs, rsqrt normalisations.  Against the oracle's f64 integrator on the same 23-bit draws
+// (tests/test_gpu_f32_paths.py, measured on a B200 over 1.7 M whole paths of up to 8 bounces), the 99th percentile of the
+// per-path relative difference is 2e-7 to 1.4e-6 and at most 2e-4 of the paths differ by more than 1e-3 (continuation rays
+// that cross a silhouette), i.e. far inside the Monte-Carlo noise the image tolerance of SURVEY 8d is defined by; the
+// direction is re-normalised in f64 so the intersection code downstream still sees |d| = 1 to f64 accuracy.
 __device__ __forceinline__ void lobe_f32(const RenderParams& rp, D3 normal64, D3 to_camera, D3 color64, double rough64, double metal64, unsigned pixel,
                                          unsigned sample, unsigned depth, D3& dir_out, D3& wgt_out, double& eps) {
     const F3 normal = f3(normal64), view = normalizef(f3(to_camera)), color = f3(color64);

@@ -3,7 +3,8 @@
 The two modes draw their uniforms from the same Philox blocks but not from the same words (the f32 mode makes one Philox call
 per bounce instead of two), so they are different sample streams of the same estimator: what must hold is that the f32 image
 is as close to an f64 image as two f64 images with different seeds are to each other (the noise floor of SURVEY 8d), that the
-mean agrees (no bias), that the path-length statistics agree — and that the bit-exact scope is untouched."""
+mean agrees (no bias), that the path-length statistics agree — and that the bit-exact scope is untouched.  The same-stream,
+path-for-path comparison of the f32 mode is test_gpu_f32_paths.py, against the oracle given the f32 mode's own draws."""
 import numpy as np
 import pytest
 

@@ -5,7 +5,8 @@ of field and two grids.
 lobe_f64 does not repeat the reference's trace operation for operation (a re-associated throughput product, sqrt closed forms
 for cos / sin(acos(x)), pow5, div0, a shared lobe frame, the D5 stop); every fixture here holds those choices to the same
 bars as the benchmark scenes: in drop mode no path may differ beyond 1e-9 relative, in keep mode the NaN / +Inf / -Inf
-classes are equal per path and channel.  The f32 shading mode is held to test_gpu_precision's estimator checks."""
+classes are equal per path and channel.  The f32 shading mode is held to test_gpu_precision's estimator checks here, and
+path for path on every fixture by test_gpu_f32_paths.py, against the oracle given the f32 mode's own draws."""
 import numpy as np
 import pytest
 
