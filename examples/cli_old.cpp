@@ -11,6 +11,8 @@
 // (rm_render_tiled_adaptive) and prints the samples actually rendered.
 // --denoise [ITERATIONS] renders through rm_render_tiled_denoised and writes the filtered frame (the library's default sigmas;
 // ITERATIONS a-trous passes, 1 when omitted).
+// --env FILE.hdr [--env-scale S] [--env-rotation R] lights the scene with a Radiance .hdr environment map (rm_load_hdr,
+// rm_scene_set_environment); --open drops the walls and the ceiling of the box (floor, sphere and mesh stay), so the map is seen.
 // Compile:  g++ -O2 -std=c++17 -Iinclude examples/cli_old.cpp -Lraymond_b200 -lraymond_cuda -Wl,-rpath,$PWD/raymond_b200 -o cli_old
 #include <arpa/inet.h>
 #include <netinet/in.h>
@@ -44,6 +46,9 @@ int main(int argc, char** argv) {
     size_t min_spp = 0;
     bool denoise = false;
     rm_denoise_settings denoise_settings{1, 0, 1e4, 0.1, 0.3, 1.0};      // the defaults of include/raymond.h
+    const char* env_path = nullptr;
+    double env_scale = 1.0, env_rotation = 0.0;
+    bool open = false;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--mesh") && i + 1 < argc) mesh_path = argv[++i];
         else if (!strcmp(argv[i], "--out") && i + 1 < argc) out_path = argv[++i];
@@ -57,12 +62,16 @@ int main(int argc, char** argv) {
         else if (!strcmp(argv[i], "--spi") && i + 1 < argc) spi = strtoull(argv[++i], nullptr, 10);
         else if (!strcmp(argv[i], "--adaptive") && i + 1 < argc) adaptive = strtod(argv[++i], nullptr);
         else if (!strcmp(argv[i], "--min-spp") && i + 1 < argc) min_spp = strtoull(argv[++i], nullptr, 10);
+        else if (!strcmp(argv[i], "--env") && i + 1 < argc) env_path = argv[++i];
+        else if (!strcmp(argv[i], "--env-scale") && i + 1 < argc) env_scale = strtod(argv[++i], nullptr);
+        else if (!strcmp(argv[i], "--env-rotation") && i + 1 < argc) env_rotation = strtod(argv[++i], nullptr);
+        else if (!strcmp(argv[i], "--open")) open = true;
         else if (!strcmp(argv[i], "--denoise")) {
             denoise = true;
             if (i + 1 < argc && argv[i + 1][0] >= '0' && argv[i + 1][0] <= '9') denoise_settings.iterations = (uint32_t)strtoul(argv[++i], nullptr, 10);
         } else {
             fprintf(stderr, "usage: cli_old [--mesh dragon.ply] [--out output.png] [--width W --height H --spp N --seed S --gpus G --repeat R --serve PORT --spi N"
-                            " --adaptive T --min-spp N --denoise [ITERATIONS]]\n");
+                            " --adaptive T --min-spp N --denoise [ITERATIONS] --env FILE.hdr --env-scale S --env-rotation R --open]\n");
             return 2;
         }
     }
@@ -92,11 +101,22 @@ int main(int argc, char** argv) {
         CHECK(rm_scene_add_sphere(scene, {0.74, -0.25, 3.5}, 0.75, &m));                      // :56-58
     }
     m = diffuse(0.75, 0.75, 0.75, 0.5); CHECK(rm_scene_add_plane(scene, {0, -1, 0}, {0, 1, 0}, &m));      // floor      :77-84
-    m = emission(1.5);                  CHECK(rm_scene_add_plane(scene, {0, 2, 0}, {0, -1, 0}, &m));      // ceiling    :85-92
-    m = diffuse(1, 1, 1, 0.4);          CHECK(rm_scene_add_plane(scene, {0, 0, -2}, {0, 0, 1}, &m));      // front wall :93-100
-    m = diffuse(0, 0, 0, 0.9);          CHECK(rm_scene_add_plane(scene, {0, 0, 5}, {0, 0, -1}, &m));      // back wall  :101-108
-    m = diffuse(0, 0, 0, 0.3);          CHECK(rm_scene_add_plane(scene, {-2, 0, 0}, {1, 0, 0}, &m));      // left wall  :109-117
-    m = diffuse(0, 0, 0, 0.3);          CHECK(rm_scene_add_plane(scene, {2, 0, 0}, {-1, 0, 0}, &m));      // right wall :118-126
+    if (!open) {
+        m = emission(1.5);              CHECK(rm_scene_add_plane(scene, {0, 2, 0}, {0, -1, 0}, &m));      // ceiling    :85-92
+        m = diffuse(1, 1, 1, 0.4);      CHECK(rm_scene_add_plane(scene, {0, 0, -2}, {0, 0, 1}, &m));      // front wall :93-100
+        m = diffuse(0, 0, 0, 0.9);      CHECK(rm_scene_add_plane(scene, {0, 0, 5}, {0, 0, -1}, &m));      // back wall  :101-108
+        m = diffuse(0, 0, 0, 0.3);      CHECK(rm_scene_add_plane(scene, {-2, 0, 0}, {1, 0, 0}, &m));      // left wall  :109-117
+        m = diffuse(0, 0, 0, 0.3);      CHECK(rm_scene_add_plane(scene, {2, 0, 0}, {-1, 0, 0}, &m));      // right wall :118-126
+    }
+    if (env_path) {
+        size_t ew = 0, eh = 0;
+        CHECK(rm_load_hdr(env_path, &ew, &eh, nullptr));
+        std::vector<float> texels(ew * eh * 3);
+        CHECK(rm_load_hdr(env_path, &ew, &eh, texels.data()));
+        const rm_environment env{texels.data(), ew, eh, env_scale, env_rotation};
+        CHECK(rm_scene_set_environment(scene, &env));
+        lap("environment map loaded");
+    }
 
     rm_settings settings{};                                                                   // :134-150
     settings.camera_settings.backbuffer_width = width;

@@ -100,6 +100,21 @@ extern "C" {
     pub fn rm_task_await_denoised(t: *mut rm_task, out: *mut rm_vec3) -> c_int;
 }
 
+// ---- environment maps (include/raymond.h states the lookup and what a ray that leaves the scene delivers)
+#[repr(C)] #[derive(Clone, Copy)] pub struct rm_environment {
+    pub texels: *const f32,            // width*height RGB triples, row-major, row 0 = +y; copied
+    pub width: usize, pub height: usize, // 1..32768 each
+    pub scale: f64,                    // finite, >= 0
+    pub rotation: f64,                 // radians about +y, finite
+}
+extern "C" {
+    // null env clears the map; RM_ERR_INVALID_ARGUMENT (scene unchanged) for a NaN / Inf / negative texel or a bad size, scale or rotation
+    pub fn rm_scene_set_environment(s: *mut rm_scene, env: *const rm_environment) -> c_int;
+    // Radiance RGBE (.hdr); texels null = only the size; RM_ERR_IO / RM_ERR_IMAGE
+    pub fn rm_load_hdr(path: *const c_char, width: *mut usize, height: *mut usize, texels: *mut f32) -> c_int;
+}
+pub const RM_ERR_IMAGE: c_int = -12;            // a malformed or unsupported image file (rm_load_hdr)
+
 // ---- values of the enum / flag fields (include/raymond.h, RM_ABI_VERSION 2)
 pub const RM_PARTITION_SAMPLES: u32 = 0;        // rank g renders global samples g, g+G, ...
 pub const RM_PARTITION_TILES: u32 = 1;          // tiles dealt round-robin in the reference's queue order (src/trace.rs:146-172)

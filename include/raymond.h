@@ -49,7 +49,8 @@ typedef enum rm_status {
     RM_ERR_UNSUPPORTED = -8,
     RM_ERR_OUT_OF_MEMORY = -9,
     RM_ERR_STATE = -10,
-    RM_ERR_PROJECT = -11          /* serde_json::from_reader(file)? fails     project.rs:35   */
+    RM_ERR_PROJECT = -11,         /* serde_json::from_reader(file)? fails     project.rs:35   */
+    RM_ERR_IMAGE = -12            /* a malformed or unsupported image file (rm_load_hdr)               */
 } rm_status;
 
 const char* rm_last_error(void);
@@ -163,6 +164,44 @@ int rm_scene_add_grid(rm_scene* scene, rm_grid* grid, const rm_material* materia
 rm_scene* rm_project_load_scene(const char* path, int* status);
 size_t rm_scene_object_count(const rm_scene* scene);
 void rm_scene_destroy(rm_scene* scene);
+
+/* Environment map (no counterpart in the reference, whose Scene has none: a scene without one renders exactly as the
+ * reference's).  An equirectangular map of width x height RGB texels, row 0 at the top (+y), lights every ray that leaves the
+ * scene.  For the direction d of such a ray, as it is (not renormalised), in f64 with no FMA contraction, in this order:
+ *   u = 0.5 + (atan2(d.x, d.z) + rotation) / (2 pi);   u -= floor(u)          (+z, the default camera's forward, is the centre column)
+ *   v = acos(clamp(d.y, -1, 1)) / pi
+ *   x = u W - 0.5,  y = v H - 0.5,  x0 = floor(x),  y0 = floor(y),  fx = x - x0,  fy = y - y0
+ *   columns x0, x0 + 1 wrap modulo W; rows y0, y0 + 1 clamp to [0, H - 1]; t(row, column) = the texel widened exactly to f64
+ *   top = t(y0, x0) + fx (t(y0, x1) - t(y0, x0)),   bot = t(y1, x0) + fx (t(y1, x1) - t(y1, x0))
+ *   L(d) = scale (top + fy (bot - top))
+ * A NaN component of d gives L = NaN.  The lerp form makes a 1 x 1 map return exactly scale * texel, and keeps L continuous across
+ * texel edges, the u seam and the poles.
+ * Integrator: at every depth 1 <= depth <= bounce_limit a ray that misses every object delivers T (*) L(d) (T = the path's
+ * throughput) where it delivered 0 — camera rays (the background, depth of field included) and rays at the bounce limit
+ * alike, as an emitter hit does; with RM_FLAG_KEEP_NONFINITE, T (*) L(d) where it delivered T (*) 0.  bounce_limit 0 still renders
+ * zeros.  The random draws, the hits, rm_stats.rays / samples and the feature buffers (RM_FLAG_AOV: a miss adds zeros) are those
+ * of the same scene without a map.  The map is reached only by the BRDF-sampled bounce (no importance sampling of the map, no
+ * next-event estimation), so a small, very bright region such as a sun disc is a noisy light.
+ * The texels cross the bus once per device the scene is placed on and count in rm_stats.upload_bytes (16 bytes per texel). */
+typedef struct rm_environment {
+    const float* texels;   /* width*height RGB triples, row-major, row 0 = +y; copied */
+    size_t width, height;  /* 1..32768 each */
+    double scale;          /* finite, >= 0 */
+    double rotation;       /* radians about +y, finite */
+} rm_environment;
+/* Sets (copies) the scene's environment map; NULL clears it.  RM_ERR_INVALID_ARGUMENT, with the scene left as it was, for a null
+ * scene, null texels, a dimension outside 1..32768, a texel that is NaN, infinite or negative, a scale that is not finite or
+ * < 0, or a rotation that is not finite.  Device scenes, renderers and tasks made from the scene before the call keep the
+ * map they were made with. */
+int rm_scene_set_environment(rm_scene* scene, const rm_environment* env);
+/* Reads a Radiance RGBE (.hdr) file: a "#?RADIANCE" or "#?RGBE" first line, header lines up to an empty line (FORMAT, when given,
+ * must be 32-bit_rle_rgbe), the resolution line "-Y H +X W" (the only orientation accepted: rows top to bottom, columns left to
+ * right), then H scanlines, each flat (4 bytes R G B E per pixel) or new-style run-length encoded (2 2 W>>8 W&255, then the four
+ * channels one after the other, runs of count-128 copies for count > 128 and literal spans for 1..128).  Texel channel =
+ * (m + 0.5) * 2^(e - 136), and 0 for e == 0 (exact in f32).  Writes width*height RGB triples, row-major, row 0 first, to `texels`;
+ * call with texels NULL to get only the size.  RM_ERR_IO for a file that cannot be read, RM_ERR_IMAGE for a malformed,
+ * truncated or unsupported one. */
+int rm_load_hdr(const char* path, size_t* width, size_t* height, float* texels);
 
 /* Scene::intersect(&self, Ray) -> Option<(&Object, Hit)>          scene.rs:54-74
  * batched over `count` rays held in HOST memory; results to HOST memory:

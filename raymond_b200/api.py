@@ -45,6 +45,7 @@ RM_ERR_CUDA = -7
 RM_ERR_UNSUPPORTED = -8
 RM_ERR_STATE = -10
 RM_ERR_PROJECT = -11
+RM_ERR_IMAGE = -12
 
 PARTITION_SAMPLES = 0
 PARTITION_TILES = 1
@@ -103,6 +104,10 @@ class DenoiseSettingsC(C.Structure):
                 ("sigma_albedo", C.c_double), ("sigma_depth", C.c_double)]
 
 
+class EnvironmentC(C.Structure):
+    _fields_ = [("texels", C.c_void_p), ("width", C.c_size_t), ("height", C.c_size_t), ("scale", C.c_double), ("rotation", C.c_double)]
+
+
 class TileC(C.Structure):
     _fields_ = [("sample_count", C.c_size_t), ("width", C.c_size_t), ("height", C.c_size_t), ("left", C.c_size_t), ("top", C.c_size_t),
                 ("data", C.POINTER(Vec3C))]
@@ -151,6 +156,7 @@ ABI_SYMBOLS = [
     "rm_write_png", "rm_project_load_scene", "rm_message_to_json", "rm_release_cached_memory", "rm_measure_fp64_rate",
     "rm_render_tiled_adaptive", "rm_renderer_read_moments", "rm_renderer_tile_errors", "rm_renderer_set_active_tiles",
     "rm_renderer_read_aovs", "rm_renderer_read_denoised", "rm_render_tiled_denoised", "rm_task_await_denoised",
+    "rm_scene_set_environment", "rm_load_hdr",
 ]
 
 _lib = None
@@ -189,6 +195,8 @@ def lib():
         "rm_scene_add_grid": (i32, [vp, vp, P(MaterialC)]),
         "rm_scene_object_count": (sz, [vp]),
         "rm_scene_destroy": (None, [vp]),
+        "rm_scene_set_environment": (i32, [vp, P(EnvironmentC)]),
+        "rm_load_hdr": (i32, [C.c_char_p, P(sz), P(sz), vp]),
         "rm_scene_intersect": (i32, [vp, i32, vp, sz, vp, vp, vp]),
         "rm_tile_free": (None, [P(TileC)]),
         "rm_render_tiled": (vp, [vp, P(SettingsC), P(GpuOptionsC)]),
@@ -433,6 +441,25 @@ class Scene:
         s._h = h
         s._grids = []
         return s
+
+    def set_environment(self, image: np.ndarray, scale: float = 1.0, rotation: float = 0.0) -> None:
+        """Light the rays that leave the scene with an equirectangular map: `image` is (H, W, 3) float32 radiance, row 0 at
+        the top (+y); `rotation` in radians about +y.  The lookup and its semantics are rm_environment's (include/raymond.h).
+        The texels are copied; RM_ERR_INVALID_ARGUMENT (scene unchanged) for a NaN, infinite or negative texel, a dimension
+        outside 1..32768, a scale that is not finite or < 0, or a rotation that is not finite."""
+        img = np.asarray(image)
+        if img.ndim != 3 or img.shape[2] != 3:
+            raise RaymondError(RM_ERR_INVALID_ARGUMENT, f"set_environment: image must be (H, W, 3), got {img.shape}")
+        t = np.ascontiguousarray(img, dtype=np.float32)
+        env = EnvironmentC(t.ctypes.data, t.shape[1], t.shape[0], float(scale), float(rotation))
+        _check(lib().rm_scene_set_environment(self._h, C.byref(env)))
+
+    def set_background(self, rgb, scale: float = 1.0) -> None:
+        """A constant environment: every ray that leaves the scene delivers scale * rgb (a 1 x 1 map)."""
+        self.set_environment(np.asarray(rgb, dtype=np.float32).reshape(1, 1, 3), scale)
+
+    def clear_environment(self) -> None:
+        _check(lib().rm_scene_set_environment(self._h, None))
 
     def __len__(self) -> int:
         return int(lib().rm_scene_object_count(self._h))
@@ -691,6 +718,16 @@ def render_tiled(scene: Scene, settings: Settings, options: Optional[GpuOptions]
         a = adaptive._c()
         h = _require(lib().rm_render_tiled_adaptive(scene._h, C.byref(s), C.byref(o), C.byref(a)), "render_tiled_adaptive")
     return TaskHandle(h, settings)
+
+
+def load_hdr(path: str) -> np.ndarray:
+    """A Radiance RGBE (.hdr) file as (H, W, 3) float32, row 0 first (rm_load_hdr).  RM_ERR_IO for a file that cannot be
+    read, RM_ERR_IMAGE for a malformed, truncated or unsupported one."""
+    W, H = C.c_size_t(0), C.c_size_t(0)
+    _check(lib().rm_load_hdr(os.fsencode(path), C.byref(W), C.byref(H), None))
+    out = np.zeros((H.value, W.value, 3), dtype=np.float32)
+    _check(lib().rm_load_hdr(os.fsencode(path), C.byref(W), C.byref(H), _ptr(out)))
+    return out
 
 
 def tonemap(frame: np.ndarray, exposure: float = 1.0, gamma: float = 2.2, device: int = 0) -> np.ndarray:

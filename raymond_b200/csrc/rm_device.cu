@@ -265,7 +265,9 @@ struct rm_device_scene {
     DevScene scene{};
     std::vector<int> grid_objects;          // object indices with Geometry::Grid, ascending
     bool emissive_grid = false;             // a grid object has an Emission material: its traversal can decide a last-depth path
-    std::vector<void*> allocations;         // one device block per distinct grid, in DevScene::grid order
+    bool has_env = false;                   // the scene has an environment map: `env` points at this device's copy of its texels
+    DevEnv env{};
+    std::vector<void*> allocations;         // one device block per distinct grid, in DevScene::grid order, then the environment map
     std::vector<size_t> allocation_bytes;
     std::vector<std::shared_ptr<Grid>> keep;
     double upload_ms = 0.0;
@@ -442,6 +444,7 @@ struct rm_scene_group {
     DevScene table{};                               // every share's object table; the grid arrays are pointed per share
     std::vector<int> grid_objects;                  // object indices with Geometry::Grid, ascending
     bool emissive_grid = false;
+    std::shared_ptr<const Environment> env;         // the scene's environment map (or none); every share uploads its own copy
     std::vector<std::shared_ptr<Grid>> grids;       // distinct grids, in DevScene::grid order
     std::vector<GridImage> images;                  // ... and their host images
     double flatten_ms = 0.0;                        // host time of the table and the images
@@ -472,6 +475,7 @@ static int build_scene_table(rm_scene_group* grp, const rm_scene* scene) {
     if (scene->objects.size() > (size_t)kMaxObjects)
         return fail(RM_ERR_UNSUPPORTED, "scene has more than " + std::to_string(kMaxObjects) + " objects");
     std::map<const Grid*, int> grid_index;
+    grp->env = scene->env;
     DevScene& s = grp->table;
     s.n_objects = (int)scene->objects.size();
     s.n_grids = 0;
@@ -555,6 +559,20 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* grp, int share) {
         slice(im, share, &b, &en);
         if (en > b) e = cudaMemcpyAsync((char*)dev + b, im.host + b, en - b, cudaMemcpyHostToDevice, 0);
         ds->bytes += en - b;                                      // bytes that crossed the bus for this share
+    }
+    if (e == cudaSuccess && grp->env) {                          // the environment map: a copy per share, host -> device
+        const Environment& env = *grp->env;
+        const size_t bytes = env.rgba.size() * sizeof(float);
+        void* dev = nullptr;
+        e = visible_acquire(device, bytes, &dev);
+        if (e == cudaSuccess) {
+            ds->allocations.push_back(dev);
+            ds->allocation_bytes.push_back(bytes);
+            e = cudaMemcpyAsync(dev, env.rgba.data(), bytes, cudaMemcpyHostToDevice, 0);
+            ds->bytes += bytes;
+            ds->has_env = true;
+            ds->env = DevEnv{(const float4*)dev, (int)env.width, (int)env.height, env.scale, env.rotation};
+        }
     }
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&grp->uploaded[(size_t)share], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventRecord(grp->uploaded[(size_t)share], 0);
@@ -906,6 +924,14 @@ struct StageHook : LaunchHook {
     }
 };
 
+// k_shade with or without the scene's environment map (env = NULL: none)
+template <bool FIRST, int PREC, bool KEEP, bool LAST>
+static void launch_shade(rm_renderer* r, unsigned grid, const RenderParams& rp, const Queue& qin, const Queue& qout, unsigned depth, unsigned n_first,
+                         const DevEnv* env) {
+    if (env) k_shade<FIRST, PREC, KEEP, LAST, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_first, *env);
+    else k_shade<FIRST, PREC, KEEP, LAST, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_first, DevEnv{});
+}
+
 template <int PREC>
 static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_samples, unsigned stride) {
     RenderParams rp = r->rp;
@@ -919,9 +945,11 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
     // Drop mode at depth == bounce_limit: only whether the closest object is an emitter decides the path (k_shade<..., LAST>).
     // k_setup then skips the grids for rays whose closest analytic hit is not an emitter, unless a grid emits, or the work
     // counters must stay comparable with the reference's at every depth.  RM_FULL_LAST_BOUNCE=1 in the environment renders
-    // the last depth like every other (tests compare the two; the frame is the same to the last bit).
+    // the last depth like every other (tests compare the two; the frame is the same to the last bit).  With an environment map
+    // a ray with no hit so far delivers radiance, so no traversal is skipped (k_shade<..., LAST, true> still shades the misses).
     const bool last_shade = !keep && r->last_depth_shortcut;
-    const bool last_skip = last_shade && !count && !r->ds->emissive_grid;
+    const bool last_skip = last_shade && !count && !r->ds->emissive_grid && !r->ds->has_env;
+    const DevEnv* env = r->ds->has_env ? &r->ds->env : nullptr;
     const unsigned persistent_grid = (unsigned)r->sms * 8u;
     RM_CUDA(cudaMemsetAsync(r->counters, 0, r->counter_slots * 3 * sizeof(unsigned), r->stream));
     if (limit == 0) RM_CUDA(cudaMemsetAsync(rp.contrib, 0, (size_t)rp.cap * 3 * sizeof(double), r->stream));   // trace() returns 0 at depth 1 > 0
@@ -953,13 +981,13 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         const bool last = last_shade && depth == limit;
         if (depth == 1) {
             const unsigned grid = std::min<unsigned>((n_paths + kBlock - 1) / kBlock, persistent_grid * 4u);
-            if (keep) k_shade<true, PREC, true, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
-            else if (last) k_shade<true, PREC, false, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
-            else k_shade<true, PREC, false, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_paths);
+            if (keep) launch_shade<true, PREC, true, false>(r, grid, rp, qin, qout, depth, n_paths, env);
+            else if (last) launch_shade<true, PREC, false, true>(r, grid, rp, qin, qout, depth, n_paths, env);
+            else launch_shade<true, PREC, false, false>(r, grid, rp, qin, qout, depth, n_paths, env);
         } else {
-            if (keep) k_shade<false, PREC, true, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
-            else if (last) k_shade<false, PREC, false, true><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
-            else k_shade<false, PREC, false, false><<<persistent_grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, 0u);
+            if (keep) launch_shade<false, PREC, true, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
+            else if (last) launch_shade<false, PREC, false, true>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
+            else launch_shade<false, PREC, false, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
         }
         hook.end(2);
     }

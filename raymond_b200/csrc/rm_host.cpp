@@ -529,6 +529,116 @@ int rm_scene_add_grid(rm_scene* scene, rm_grid* grid, const rm_material* materia
 size_t rm_scene_object_count(const rm_scene* scene) { return scene ? scene->objects.size() : 0; }
 void rm_scene_destroy(rm_scene* scene) { delete scene; }
 
+int rm_scene_set_environment(rm_scene* scene, const rm_environment* env) {
+    if (!scene) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: null scene");
+    if (!env) { scene->env.reset(); return RM_OK; }
+    if (!env->texels) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: null texels");
+    if (env->width < 1 || env->width > 32768 || env->height < 1 || env->height > 32768)
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: width and height must be 1..32768");
+    if (!std::isfinite(env->scale) || env->scale < 0.0) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: scale must be finite and >= 0");
+    if (!std::isfinite(env->rotation)) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: rotation must be finite");
+    const size_t n = env->width * env->height;
+    for (size_t i = 0; i < 3 * n; i++)
+        if (!std::isfinite(env->texels[i]) || env->texels[i] < 0.0f)
+            return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_environment: texel value " + std::to_string(i) + " is negative, NaN or infinite");
+    auto e = std::make_shared<Environment>();
+    try {
+        e->rgba.resize(4 * n);
+    } catch (const std::bad_alloc&) {
+        return fail(RM_ERR_OUT_OF_MEMORY, "rm_scene_set_environment: cannot hold the texels");
+    }
+    for (size_t i = 0; i < n; i++) {
+        e->rgba[4 * i] = env->texels[3 * i];
+        e->rgba[4 * i + 1] = env->texels[3 * i + 1];
+        e->rgba[4 * i + 2] = env->texels[3 * i + 2];
+        e->rgba[4 * i + 3] = 0.0f;
+    }
+    e->width = env->width;
+    e->height = env->height;
+    e->scale = env->scale;
+    e->rotation = env->rotation;
+    scene->env = std::move(e);       // placements made before keep the map they share
+    return RM_OK;
+}
+
+// Radiance RGBE (.hdr) body: see rm_load_hdr in include/raymond.h.  `texels` NULL = size only.
+static int decode_hdr(const std::string& buf, const char* path, size_t* width, size_t* height, float* texels) {
+    auto bad = [&](const std::string& why) { return fail(RM_ERR_IMAGE, std::string(path) + ": " + why); };
+    size_t p = 0;
+    auto line = [&](std::string* out) {
+        const size_t e = buf.find('\n', p);
+        if (e == std::string::npos) return false;
+        *out = buf.substr(p, e - p);
+        p = e + 1;
+        return true;
+    };
+    std::string l;
+    if (!line(&l) || (l != "#?RADIANCE" && l != "#?RGBE")) return bad("not a Radiance RGBE file (no #?RADIANCE / #?RGBE line)");
+    for (;;) {
+        if (!line(&l)) return bad("header does not end");
+        if (l.empty()) break;
+        if (l.compare(0, 7, "FORMAT=") == 0 && l != "FORMAT=32-bit_rle_rgbe") return bad("unsupported " + l);
+    }
+    if (!line(&l)) return bad("no resolution line");
+    char ys[3] = {0}, xs[3] = {0};
+    unsigned long long H = 0, W = 0;
+    int used = 0;
+    if (sscanf(l.c_str(), "%2s %llu %2s %llu%n", ys, &H, xs, &W, &used) != 4 || (size_t)used != l.size())
+        return bad("malformed resolution line");
+    if (strcmp(ys, "-Y") != 0 || strcmp(xs, "+X") != 0) return bad("unsupported orientation \"" + l + "\" (only -Y H +X W)");
+    if (W < 1 || H < 1 || W > ((size_t)1 << 31) / H) return bad("unsupported size " + std::to_string(W) + " x " + std::to_string(H));
+    *width = (size_t)W;
+    *height = (size_t)H;
+    if (!texels) return RM_OK;
+    const unsigned char* b = (const unsigned char*)buf.data();
+    const size_t n = buf.size();
+    std::vector<unsigned char> row((size_t)W * 4);
+    for (size_t y = 0; y < H; y++) {
+        const bool rle = W >= 8 && W <= 32767 && p + 4 <= n && b[p] == 2 && b[p + 1] == 2 && !(b[p + 2] & 0x80);
+        if (rle) {
+            if ((((size_t)b[p + 2] << 8) | b[p + 3]) != W) return bad("scanline " + std::to_string(y) + ": run-length width differs");
+            p += 4;
+            for (int c = 0; c < 4; c++)
+                for (size_t x = 0; x < W;) {
+                    if (p >= n) return bad("truncated");
+                    size_t count = b[p++];
+                    if (count > 128) {
+                        count -= 128;
+                        if (p >= n) return bad("truncated");
+                        if (x + count > W) return bad("scanline " + std::to_string(y) + ": run overruns the row");
+                        for (size_t k = 0; k < count; k++) row[4 * (x + k) + c] = b[p];
+                        p++;
+                    } else {
+                        if (count == 0 || x + count > W) return bad("scanline " + std::to_string(y) + ": bad literal span");
+                        if (p + count > n) return bad("truncated");
+                        for (size_t k = 0; k < count; k++) row[4 * (x + k) + c] = b[p + k];
+                        p += count;
+                    }
+                    x += count;
+                }
+        } else {
+            if (p + 4 * (size_t)W > n) return bad("truncated");
+            memcpy(row.data(), b + p, 4 * (size_t)W);
+            p += 4 * (size_t)W;
+        }
+        float* out = texels + y * W * 3;
+        for (size_t x = 0; x < W; x++) {
+            const int e = row[4 * x + 3];
+            for (int c = 0; c < 3; c++) out[3 * x + c] = e == 0 ? 0.0f : (float)std::ldexp((double)row[4 * x + c] + 0.5, e - 136);
+        }
+    }
+    return RM_OK;
+}
+
+int rm_load_hdr(const char* path, size_t* width, size_t* height, float* texels) {
+    if (!path || !width || !height) return fail(RM_ERR_INVALID_ARGUMENT, "rm_load_hdr: null argument");
+    std::ifstream f(path, std::ios::binary);
+    if (!f) return fail(RM_ERR_IO, std::string("cannot read ") + path);
+    std::string buf((std::istreambuf_iterator<char>(f)), std::istreambuf_iterator<char>());
+    if (f.bad()) return fail(RM_ERR_IO, std::string("cannot read ") + path);
+    return decode_hdr(buf, path, width, height, texels);
+}
+
 size_t rm_tile_layout(const rm_settings* s, size_t* rects, size_t capacity) {
     if (!s) return 0;
     std::vector<TileRect> t = tile_layout(s->camera_settings.backbuffer_width, s->camera_settings.backbuffer_height, s->tile_size[0], s->tile_size[1]);

@@ -79,6 +79,14 @@ struct Object {                                             // scene.rs:33-37
     rm_material material;
 };
 
+// The environment map of a scene (rm_scene_set_environment), immutable once set: width x height texels, row 0 = +y, stored as
+// RGBA f32 (A = 0) in the layout the device reads.  Scenes and the placements made from them share it.
+struct Environment {
+    std::vector<float> rgba;
+    size_t width = 0, height = 0;
+    double scale = 1.0, rotation = 0.0;
+};
+
 struct TileRect { size_t left, top, width, height; };
 // tile split of render_tiled                               src/trace.rs:142-173
 std::vector<TileRect> tile_layout(size_t W, size_t H, size_t tw, size_t th);
@@ -191,4 +199,4 @@ rm_device_scene* rm_renderer_device_scene(rm_renderer* r);
 
 struct rm_mesh { rm::Mesh mesh; };
 struct rm_grid { std::shared_ptr<rm::Grid> grid; std::atomic<int> refs{1}; };
-struct rm_scene { std::vector<rm::Object> objects; };
+struct rm_scene { std::vector<rm::Object> objects; std::shared_ptr<const rm::Environment> env; };

@@ -134,6 +134,14 @@ struct RenderParams {
     DevTotals* totals;
 };
 
+// The environment map of a scene (rm_scene_set_environment): W x H texels, row 0 = +y, RGB in .xyz.  k_shade takes it as its
+// last parameter, not inside DevScene, so that the parameter layout of every kernel that takes a DevScene stays as it was.
+struct DevEnv {
+    const float4* texels;
+    int W, H;
+    double scale, rotation;
+};
+
 __host__ __device__ inline unsigned stage_slot(unsigned depth) { return depth < RM_STAGE_SLOTS - 1 ? depth : RM_STAGE_SLOTS - 1; }
 
 // ===================================================================== device math (cgmath semantics)
@@ -632,10 +640,40 @@ __device__ __forceinline__ D3 surface_normal(const DevScene& sc, const DevObject
     return normal;
 }
 
-template <int PREC, bool KEEP>
-__device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, double hit_t, int hit_obj, unsigned hit_sub, unsigned pixel,
-                                        unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
-    if (hit_obj < 0) return BOUNCE_NONE;                                    // :242
+// Radiance of the environment map for the direction d of a ray that leaves the scene (include/raymond.h, rm_environment):
+// equirectangular, bilinear in the lerp form, f64 with every operation in the order the header gives (tests/env_oracle.cpp
+// and tests/env_ref.py restate it).  A NaN component of d gives NaN.
+__device__ __forceinline__ D3 env_radiance(const DevEnv& e, D3 d) {
+    const double kPi = 3.141592653589793;
+    double u = 0.5 + (atan2(d.x, d.z) + e.rotation) / (2.0 * kPi);
+    u -= floor(u);
+    const double cy = d.y < -1.0 ? -1.0 : d.y > 1.0 ? 1.0 : d.y;
+    const double v = acos(cy) / kPi;
+    if (!(u == u) || !(v == v)) { const double nan = __longlong_as_double(0x7ff8000000000000ll); return d3(nan, nan, nan); }
+    const double x = u * (double)e.W - 0.5, y = v * (double)e.H - 0.5;
+    const double x0 = floor(x), y0 = floor(y);
+    const double fx = x - x0, fy = y - y0;
+    int ix0 = (int)x0, iy0 = (int)y0;                  // ix0 in [-1, W - 1], iy0 in [-1, H - 1]
+    int ix1 = ix0 + 1, iy1 = iy0 + 1;
+    if (ix0 < 0) ix0 += e.W;
+    if (ix1 >= e.W) ix1 -= e.W;
+    if (iy0 < 0) iy0 = 0;
+    if (iy1 > e.H - 1) iy1 = e.H - 1;
+    const float4 a = __ldg(&e.texels[(size_t)iy0 * e.W + ix0]), b = __ldg(&e.texels[(size_t)iy0 * e.W + ix1]);
+    const float4 c = __ldg(&e.texels[(size_t)iy1 * e.W + ix0]), f = __ldg(&e.texels[(size_t)iy1 * e.W + ix1]);
+    const D3 t00 = d3(a.x, a.y, a.z), t01 = d3(b.x, b.y, b.z), t10 = d3(c.x, c.y, c.z), t11 = d3(f.x, f.y, f.z);
+    const D3 top = t00 + fx * (t01 - t00), bot = t10 + fx * (t11 - t10);
+    return e.scale * (top + fy * (bot - top));
+}
+
+// ENV: the scene has an environment map; a ray that misses delivers T (*) env_radiance(d) (BOUNCE_EMIT) instead of ending with 0.
+template <int PREC, bool KEEP, bool ENV>
+__device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, const DevEnv& env, double hit_t, int hit_obj, unsigned hit_sub,
+                                        unsigned pixel, unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
+    if (hit_obj < 0) {                                                      // :242
+        if (ENV) { v = env_radiance(env, d); return BOUNCE_EMIT; }
+        return BOUNCE_NONE;
+    }
     const DevObject& ob = sc.obj[hit_obj];
     const D3 frag = o + d * hit_t;                                          // :246
     if (ob.mat == RM_MATERIAL_EMISSION) { v = ld3(ob.color); return BOUNCE_EMIT; }   // :250
@@ -1126,14 +1164,18 @@ __global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const
 // Stage part 3: shade, then deliver radiance or append the next ray (warp-aggregated compaction) to the next depth's queue.
 // KEEP = RM_FLAG_KEEP_NONFINITE: the path's value is formed as the reference forms it, so that a NaN / Inf weight anywhere on
 // the path poisons the sample: no path is stopped for a zero throughput (D5), and a path that ends without emission delivers
-// T (*) 0 on a miss and T (*) w (*) 0 at the bounce limit instead of an exact (0, 0, 0).  The default instantiation is the
+// T (*) 0 on a miss (T (*) L(d) with an environment map, ENV) and T (*) w (*) 0 at the bounce limit instead of an exact (0, 0, 0).  The default instantiation is the
 // one the benchmark runs.
 // LAST (drop mode, depth == bounce_limit): shade() ends every path there, delivering T (*) emission for an emitter hit and an
 // exact (0, 0, 0) otherwise, so this instantiation reads only the hit object, the slot and the throughput of emitter hits,
 // and forms T (*) emission with the same multiplication as the general body.  No path continues and no triangle is shaded.
-template <bool FIRST, int PREC, bool KEEP, bool LAST>
+// ENV: the scene has an environment map `env` (the last parameter, unused otherwise, so that the instantiations without one keep
+// the parameter layout and the code they had before it existed).  A miss delivers T (*) env_radiance(d); the LAST body reads d
+// from the queue for misses only.
+template <bool FIRST, int PREC, bool KEEP, bool LAST, bool ENV>
 __global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
-                                                   const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first) {
+                                                   const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first,
+                                                   const DevEnv env) {
     static_assert(!(LAST && KEEP), "keep mode computes the last weight: it has no last-depth shortcut");
     const unsigned n = FIRST ? n_first : rp.cnt.rays[depth - 1];
     const unsigned lane = threadIdx.x & 31u;
@@ -1146,6 +1188,8 @@ __global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __gri
             D3 result = d3(0.0, 0.0, 0.0);
             if (ob >= 0 && sc.obj[ob].mat == RM_MATERIAL_EMISSION)
                 result = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), ld3(sc.obj[ob].color));
+            else if (ENV && ob < 0)
+                result = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), env_radiance(env, d3(qin.f[3][i], qin.f[4][i], qin.f[5][i])));
             rp.contrib[slot] = result.x;
             rp.contrib[(size_t)rp.cap + slot] = result.y;
             rp.contrib[2 * (size_t)rp.cap + slot] = result.z;
@@ -1164,7 +1208,7 @@ __global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __gri
             d = d3(qin.f[3][i], qin.f[4][i], qin.f[5][i]);
             const unsigned q = slot % rp.n_pixels, s_local = slot / rp.n_pixels;
             D3 v = d3(0.0, 0.0, 0.0);
-            const Bounce b = shade<PREC, KEEP>(sc, rp, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
+            const Bounce b = shade<PREC, KEEP, ENV>(sc, rp, env, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
             // the path's value is (prod of weights) (*) emission (src/trace.rs:281-282,315-319): the throughput so far comes in only now
             T = d3(0.0, 0.0, 0.0);
             if (KEEP || b != BOUNCE_NONE) T = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), v);

@@ -58,6 +58,108 @@ def gold_dragon(triangles: np.ndarray) -> list:
     return [RED_SPHERE, ("grid", translate(triangles, DRAGON_TRANSLATE), DRAGON_MATERIAL)] + BOX_PLANES
 
 
+FLOOR = BOX_PLANES[0]
+
+
+def open_dragon(triangles: np.ndarray) -> list:
+    """The GoldDragon scene without its walls and ceiling: floor, red sphere and the dragon under the open sky (the scene
+    `cli_old --open` builds).  Rays that leave it see the environment map, if the scene has one."""
+    return [RED_SPHERE, ("grid", translate(triangles, DRAGON_TRANSLATE), DRAGON_MATERIAL), FLOOR]
+
+
+def open_spheres() -> list:
+    """Spheres on a floor under the open sky: diffuse and metal, rough and smooth."""
+    return [RED_SPHERE, BLUE_SPHERE,
+            ("sphere", (0.0, -0.6, 4.6), 0.4, ("Metal", (0.9, 0.9, 0.9), 0.6)),
+            ("sphere", (1.3, -0.7, 2.8), 0.3, ("Diffuse", (0.2, 0.8, 0.3), 0.9)), FLOOR]
+
+
+def sky(width: int = 256, height: int = 128, *, sun_dir=(0.4, 0.6, 0.7), sun_radius_deg: float = 2.5, sun_radiance: float = 400.0) -> np.ndarray:
+    """Procedural equirectangular sky, (height, width, 3) float32 in the layout of include/raymond.h's rm_environment: a
+    horizon-to-zenith gradient above, a dim ground below, and a small bright sun disc in direction `sun_dir`."""
+    v = (np.arange(height) + 0.5) / height
+    u = (np.arange(width) + 0.5) / width
+    V, U = np.meshgrid(v, u, indexing="ij")
+    theta = V * np.pi                              # 0 = +y
+    phi = (U - 0.5) * 2.0 * np.pi                  # atan2(d.x, d.z)
+    d = np.stack([np.sin(theta) * np.sin(phi), np.cos(theta), np.sin(theta) * np.cos(phi)], axis=-1)
+    up = np.clip(d[..., 1], 0.0, 1.0)[..., None]
+    horizon = np.array([0.9, 0.95, 1.0])
+    zenith = np.array([0.25, 0.45, 0.95])
+    ground = np.array([0.18, 0.16, 0.14])
+    img = np.where(d[..., 1:2] >= 0.0, horizon + (zenith - horizon) * np.sqrt(up), ground)
+    sd = np.asarray(sun_dir, dtype=np.float64)
+    sd = sd / np.linalg.norm(sd)
+    sun = (d @ sd) >= np.cos(np.radians(sun_radius_deg))
+    img[sun] = sun_radiance * np.array([1.0, 0.95, 0.85])
+    return np.ascontiguousarray(img, dtype=np.float32)
+
+
+def write_hdr(path: str, image: np.ndarray, rle: bool = True) -> None:
+    """Write (H, W, 3) radiance as a Radiance RGBE (.hdr) file ("-Y H +X W"); scanlines run-length encoded when `rle` and
+    8 <= W <= 32767 (the only widths the format encodes), else flat."""
+    img = np.asarray(image, dtype=np.float64)
+    H, W = img.shape[:2]
+    rgbe = rgbe_encode(img)
+    with open(path, "wb") as f:
+        f.write(b"#?RADIANCE\nFORMAT=32-bit_rle_rgbe\n\n" + f"-Y {H} +X {W}\n".encode())
+        for y in range(H):
+            row = rgbe[y]
+            if rle and 8 <= W <= 32767:
+                f.write(bytes([2, 2, W >> 8, W & 255]))
+                for c in range(4):
+                    f.write(_rle_channel(row[:, c]))
+            else:
+                f.write(row.tobytes())
+
+
+def rgbe_encode(img: np.ndarray) -> np.ndarray:
+    """(…, 3) radiance -> (…, 4) uint8 RGBE (m = floor(v * 256 / 2^e'), exponent of the largest channel)."""
+    img = np.asarray(img, dtype=np.float64)
+    mx = img.max(axis=-1)
+    m, e = np.frexp(mx)                            # mx = m * 2^e, m in [0.5, 1)
+    scale = np.where(mx > 1e-32, np.ldexp(256.0, -e), 0.0)
+    out = np.zeros(img.shape[:-1] + (4,), dtype=np.uint8)
+    out[..., :3] = np.clip(np.floor(img * scale[..., None]), 0, 255).astype(np.uint8)
+    out[..., 3] = np.where(mx > 1e-32, np.clip(e + 128, 0, 255), 0).astype(np.uint8)
+    return out
+
+
+def rgbe_decode(rgbe: np.ndarray) -> np.ndarray:
+    """uint8 RGBE -> float32 radiance: (m + 0.5) * 2^(e - 136), 0 for e == 0 (include/raymond.h, rm_load_hdr)."""
+    q = np.asarray(rgbe, dtype=np.uint8)
+    e = q[..., 3:4].astype(np.int64)
+    v = np.ldexp(q[..., :3].astype(np.float64) + 0.5, e - 136)
+    return np.where(e == 0, 0.0, v).astype(np.float32)
+
+
+def _rle_channel(vals: np.ndarray) -> bytes:
+    """New-style RLE of one channel of a scanline: runs of >= 3 equal bytes as (128 + n, value), n <= 127; the rest as
+    literal spans (n, bytes...), n <= 128."""
+    out = bytearray()
+    v = np.asarray(vals, dtype=np.uint8)
+    n = len(v)
+    i = 0
+    lit = []
+    while i < n:
+        j = i
+        while j < n and j - i < 127 and v[j] == v[i]:
+            j += 1
+        if j - i >= 3:
+            while lit:
+                out += bytes([min(len(lit), 128)]) + bytes(lit[:128])
+                lit = lit[128:]
+            out += bytes([128 + (j - i), int(v[i])])
+            i = j
+        else:
+            lit.append(int(v[i]))
+            i += 1
+    while lit:
+        out += bytes([min(len(lit), 128)]) + bytes(lit[:128])
+        lit = lit[128:]
+    return bytes(out)
+
+
 def soup_scene(triangles: np.ndarray) -> list:
     """C4: one Grid object, Metal((1,1,0.1), 0.15) (SURVEY §8d)."""
     return [("grid", triangles, DRAGON_MATERIAL)]

@@ -1,0 +1,135 @@
+"""ctypes binding of tests/env_oracle.cpp: the CPU oracle with an environment map (test infrastructure only).
+
+The library is compiled on first use into a directory under the system's temporary directory (keyed by the hash of the
+sources), so the test tree is never written to.  It contains its own copy of the oracle, so its scenes are built through it.
+"""
+from __future__ import annotations
+
+import ctypes as C
+import hashlib
+import os
+import subprocess
+import tempfile
+
+import numpy as np
+
+from oracle import oracle as O
+
+_HERE = os.path.dirname(os.path.abspath(__file__))
+_SRC = os.path.join(_HERE, "env_oracle.cpp")
+_ORACLE_SRC = os.path.join(os.path.dirname(_HERE), "oracle", "raymond_oracle.cpp")
+_lib = None
+
+
+def lib():
+    global _lib
+    if _lib is not None:
+        return _lib
+    h = hashlib.sha256()
+    for p in (_SRC, _ORACLE_SRC):
+        with open(p, "rb") as f:
+            h.update(f.read())
+    out_dir = os.path.join(tempfile.gettempdir(), f"raymond_env_oracle_{os.getuid()}")
+    os.makedirs(out_dir, exist_ok=True)
+    so = os.path.join(out_dir, f"libenv_oracle_{h.hexdigest()[:16]}.so")
+    if not os.path.exists(so):
+        tmp = f"{so}.{os.getpid()}.tmp"
+        subprocess.run(["g++", "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-pthread", "-shared", "-o", tmp,
+                        _SRC, "-lm"], check=True)
+        os.replace(tmp, so)
+    L = C.CDLL(so, mode=os.RTLD_LOCAL)
+    vp, sz = C.c_void_p, C.c_size_t
+    L.rmo_mesh_from_triangles.restype = vp
+    L.rmo_mesh_from_triangles.argtypes = [vp, sz]
+    L.rmo_mesh_destroy.argtypes = [vp]
+    L.rmo_grid_build.restype = vp
+    L.rmo_grid_build.argtypes = [vp, C.POINTER(C.c_int)]
+    L.rmo_grid_destroy.argtypes = [vp]
+    L.rmo_scene_create.restype = vp
+    L.rmo_scene_destroy.argtypes = [vp]
+    L.rmo_scene_add_sphere.argtypes = [vp, O.Vec3, C.c_double, C.POINTER(O.MaterialC)]
+    L.rmo_scene_add_plane.argtypes = [vp, O.Vec3, O.Vec3, C.POINTER(O.MaterialC)]
+    L.rmo_scene_add_grid.argtypes = [vp, vp, C.POINTER(O.MaterialC)]
+    L.rmoe_env_create.restype = vp
+    L.rmoe_env_create.argtypes = [vp, sz, sz, C.c_double, C.c_double]
+    L.rmoe_env_destroy.argtypes = [vp]
+    L.rmoe_env_lookup.argtypes = [vp, vp, sz, vp]
+    L.rmoe_render_sample.restype = C.c_int
+    L.rmoe_render_sample.argtypes = [vp, vp, C.POINTER(O.SettingsC), C.c_uint64, C.c_uint32, C.c_uint32, C.c_int, vp,
+                                     C.POINTER(O.CountersC)]
+    _lib = L
+    return L
+
+
+def _ptr(a: np.ndarray):
+    return a.ctypes.data_as(C.c_void_p)
+
+
+class Environment:
+    """The map of rm_environment (include/raymond.h): (H, W, 3) texels, taken as f32."""
+
+    def __init__(self, image, scale: float = 1.0, rotation: float = 0.0):
+        t = np.ascontiguousarray(image, dtype=np.float32)
+        assert t.ndim == 3 and t.shape[2] == 3
+        self._h = lib().rmoe_env_create(_ptr(t), t.shape[1], t.shape[0], float(scale), float(rotation))
+
+    def lookup(self, dirs) -> np.ndarray:
+        """L(d) for (n, 3) directions."""
+        d = np.ascontiguousarray(dirs, dtype=np.float64).reshape(-1, 3)
+        out = np.zeros_like(d)
+        lib().rmoe_env_lookup(self._h, _ptr(d), d.shape[0], _ptr(out))
+        return out
+
+    def __del__(self):
+        if getattr(self, "_h", None) and _lib is not None:
+            _lib.rmoe_env_destroy(self._h)
+            self._h = None
+
+
+class Scene:
+    """A fixture scene (raymond_b200.fixtures object tuples) with an environment map."""
+
+    def __init__(self, objects, env: Environment):
+        L = lib()
+        self.env = env
+        self._h = L.rmo_scene_create()
+        self._grids = []
+        for o in objects:
+            if o[0] == "sphere":
+                m = O._mat(o[3])
+                L.rmo_scene_add_sphere(self._h, O.Vec3(*o[1]), float(o[2]), C.byref(m))
+            elif o[0] == "plane":
+                m = O._mat(o[3])
+                L.rmo_scene_add_plane(self._h, O.Vec3(*o[1]), O.Vec3(*o[2]), C.byref(m))
+            else:
+                t = np.ascontiguousarray(o[1], dtype=np.float64).reshape(-1, O.TRI_DOUBLES)
+                mesh = L.rmo_mesh_from_triangles(_ptr(t), t.shape[0])
+                st = C.c_int(0)
+                g = L.rmo_grid_build(mesh, C.byref(st))
+                L.rmo_mesh_destroy(mesh)
+                assert g, f"grid build: oracle status {st.value}"
+                self._grids.append(g)
+                m = O._mat(o[2])
+                L.rmo_scene_add_grid(self._h, g, C.byref(m))
+
+    def render_sample(self, cam: dict, sample: int, *, seed: int, bounce_limit: int = 5, drop_nonfinite: bool = True,
+                      draws: str = "f64", threads: int = 0):
+        """One sample per pixel (global sample index `sample`): (H x W x 3 radiance, counters), as O.render(.., 1,
+        first_sample=sample) renders it without a map."""
+        assert draws in O.DRAWS, draws
+        s = O.settings_c(cam, 1, (32, 32), bounce_limit, 1)
+        out = np.zeros((s.camera.height, s.camera.width, 3))
+        cnt = O.CountersC()
+        flags = (1 if drop_nonfinite else 0) | (2 if draws == "f32" else 0)
+        lib().rmoe_render_sample(self._h, self.env._h, C.byref(s), seed, sample, flags, threads or (os.cpu_count() or 1), _ptr(out),
+                                 C.byref(cnt))
+        return out, cnt.as_dict()
+
+    def __del__(self):
+        if _lib is not None:
+            if getattr(self, "_h", None):
+                _lib.rmo_scene_destroy(self._h)
+                self._h = None
+            for g in getattr(self, "_grids", []):
+                _lib.rmo_grid_destroy(g)
+            self._grids = []
