@@ -866,6 +866,19 @@ class Renderer:
         _check(lib().rm_renderer_read_rgb8(self._h, sample_count, exposure, gamma, _ptr(out)))
         return out
 
+    def coverage(self) -> Optional[np.ndarray]:
+        """The coverage mask of the camera rays (DESIGN §3.7), (H, W) bool: False = no triangle of the first grid object can be
+        hit from that pixel, so its camera rays skip the grid.  None when the renderer has no mask."""
+        fn = lib().rm_renderer_coverage      # internal entry point, not part of include/raymond.h
+        fn.restype, fn.argtypes = C.c_int, [C.c_void_p, C.c_void_p]
+        cs = self.settings.camera_settings
+        out = np.zeros((cs.backbuffer_height, cs.backbuffer_width), dtype=np.int32)
+        st = fn(self._h, _ptr(out))
+        if st == RM_ERR_STATE:
+            return None
+        _check(st)
+        return out != 0
+
     def stats(self) -> dict:
         s = StatsC()
         _check(lib().rm_renderer_stats(self._h, C.byref(s)))

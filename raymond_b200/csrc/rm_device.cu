@@ -264,6 +264,8 @@ struct rm_device_scene {
     int traverse_blocks_per_sm = 2;
     DevScene scene{};
     std::vector<int> grid_objects;          // object indices with Geometry::Grid, ascending
+    const float4* tri_spheres[kMaxGrids] = {};  // per distinct grid: one bounding sphere per triangle (§3.1), in the grid's block ...
+    size_t n_triangles[kMaxGrids] = {};     // ... and its triangle count
     bool emissive_grid = false;             // a grid object has an Emission material: its traversal can decide a last-depth path
     bool has_env = false;                   // the scene has an environment map: `env` points at this device's copy of its texels
     DevEnv env{};
@@ -301,7 +303,7 @@ __global__ void __launch_bounds__(256) k_spread_spheres(const float4* __restrict
 // images above kImageCacheLimit are staged through a pooled pinned block per upload.
 struct GridImage {
     DevGrid header{};          // geometry of the grid; the array pointers are set by point_grid()
-    size_t off_tri = 0, off_shd = 0, off_cells = 0, off_occ = 0, off_refs = 0, off_spht = 0, host_total = 0, off_sph = 0, total = 0, nr = 0;
+    size_t off_tri = 0, off_shd = 0, off_cells = 0, off_occ = 0, off_refs = 0, off_spht = 0, host_total = 0, off_sph = 0, total = 0, nr = 0, nt = 0;
     char* host = nullptr;
     bool cached = false;       // the host image belongs to the grid (not released after the upload)
 };
@@ -321,6 +323,7 @@ static int prepare_grid_image(const Grid& g, GridImage* out) {
     const size_t n_occ = (nc + 31) / 32;
     auto pad = [](size_t b) { return (b + 255) & ~(size_t)255; };
     im.nr = nr;
+    im.nt = nt;
     im.off_tri = 0;
     im.off_shd = im.off_tri + pad(nt * 12 * sizeof(double));
     im.off_cells = im.off_shd + pad(nt * 18 * sizeof(double));
@@ -599,7 +602,11 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* grp, int share) {
     ok = grp->barrier(1, ok && e == cudaSuccess);
     if (ok) {
         ds->scene = grp->table;
-        for (size_t i = 0; i < grp->images.size(); i++) point_grid(grp->images[i], mine[i], &ds->scene.grid[i]);
+        for (size_t i = 0; i < grp->images.size(); i++) {
+            point_grid(grp->images[i], mine[i], &ds->scene.grid[i]);
+            ds->tri_spheres[i] = (const float4*)((char*)mine[i] + grp->images[i].off_spht);
+            ds->n_triangles[i] = grp->images[i].nt;
+        }
         ds->grid_objects = grp->grid_objects;
         ds->emissive_grid = grp->emissive_grid;
         ds->keep = grp->grids;
@@ -637,11 +644,11 @@ struct NoHook : LaunchHook {
 
 // Scene::intersect for a batch of rays: k_setup (+ k_traverse per grid object).  On return (stream
 // order) `buf.hit` holds the closest hit of every ray.  `trav_count` / `cursor` are zero on entry and
-// re-zeroed between grid passes.
+// re-zeroed between grid passes.  `cover` (camera rays only): the coverage mask of the first grid object, or null (§3.7).
 template <int SRC>
 static int launch_intersect(rm_device_scene* ds, const RenderParams& rp, SetupArgs sa, const HitArrays& hit, double* trav, unsigned* trav_count,
                             unsigned* cursor, unsigned n_upper, unsigned depth, bool count_work, DevTotals* totals, cudaStream_t stream,
-                            LaunchHook& hook) {
+                            LaunchHook& hook, const int* cover = nullptr) {
     const unsigned setup_grid = std::max<unsigned>(1u, std::min<unsigned>((n_upper + kBlock - 1) / kBlock, (unsigned)ds->sms * 16u));
     const unsigned trav_grid = (unsigned)(ds->sms * ds->traverse_blocks_per_sm);
     sa.hit = hit;
@@ -652,6 +659,7 @@ static int launch_intersect(rm_device_scene* ds, const RenderParams& rp, SetupAr
         const int gobj = n_grid_objects ? ds->grid_objects[pass] : -1;
         sa.grid_object = gobj;
         sa.analytic = pass == 0 ? 1 : 0;
+        sa.cover = pass == 0 ? cover : nullptr;
         if (pass > 0) {
             RM_CUDA(cudaMemsetAsync(trav_count, 0, sizeof(unsigned), stream));
             RM_CUDA(cudaMemsetAsync(cursor, 0, sizeof(unsigned), stream));
@@ -711,6 +719,8 @@ struct rm_renderer {
     DevTotals* totals = nullptr;
     size_t batch_spp = 1;
     bool last_depth_shortcut = true;                // RM_FULL_LAST_BOUNCE unset: see renderer_batch_t
+    bool cover_allowed = true;                      // RM_NO_COVER_MASK unset: see build_cover
+    int* cover = nullptr;                           // coverage mask of the camera rays for the first grid object, null = none (§3.7)
     uint64_t launches = 0;
     double device_ms = 0.0;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
@@ -735,6 +745,7 @@ struct rm_renderer {
         if (moments) visible_release(device, accum_bytes, moments);
         if (aov) visible_release(device, aov_bytes, aov);
         dev_free(active_map); dev_free(active_runs);
+        dev_free(cover);
         if (owns_stream && stream) cudaStreamDestroy(stream);
         if (owns_scene) delete ds;
     }
@@ -823,6 +834,7 @@ static int renderer_init(rm_renderer* r) {
     RM_CUDA(cudaSetDevice(r->device));
     r->sms = sm_count(r->device);
     r->last_depth_shortcut = getenv("RM_FULL_LAST_BOUNCE") == nullptr;
+    r->cover_allowed = getenv("RM_NO_COVER_MASK") == nullptr;
     if (r->opt.stream) r->stream = (cudaStream_t)r->opt.stream;
     else { RM_CUDA(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking)); r->owns_stream = true; }
 
@@ -896,6 +908,62 @@ static int renderer_init(rm_renderer* r) {
     return RM_OK;
 }
 
+// The coverage mask of the camera rays (§3.7) for the first grid object (the grid pass k_setup<SRC_CAMERA> sets up), built
+// on the renderer's stream once its scene is bound: it depends only on the camera, the frame and the grid, so every batch
+// and frame of the renderer reuses it.  No mask with DoF (the rays do not share an apex), under RM_FLAG_COUNT_WORK (the
+// per-stage cells and tests stay comparable with the oracle's, §3.4), with RM_NO_COVER_MASK in the environment, or when the
+// grid's box is not strictly in front of the camera, the error bound below is not far below a pixel, or a triangle of the
+// grid cannot be projected.
+static int build_cover(rm_renderer* r) {
+    if (r->cover) { RM_CUDA(cudaStreamSynchronize(r->stream)); dev_free(r->cover); r->cover = nullptr; }
+    const DevCamera& cam = r->rp.cam;
+    if (!r->cover_allowed || cam.use_dof || (r->opt.flags & RM_FLAG_COUNT_WORK) || r->ds->grid_objects.empty()) return RM_OK;
+    Trace trace;
+    const int gi = r->ds->scene.obj[r->ds->grid_objects[0]].grid;
+    const DevGrid& g = r->ds->scene.grid[gi];
+    const size_t W = (size_t)cam.W, H = (size_t)cam.H, npx = W * H;
+    // A hit Triangle::intersects accepts lies within 4e-7 * |o - v0| * diag2 of the exact triangle (the form of the bound
+    // k_setup uses for t), and |o - v0| <= the distance to the farthest corner of the box: the spheres are inflated by that.
+    // In pixels, a point at depth z >= zmin with |x/z|, |y/z| <= rmax moves by at most bound * (1 + rmax) / zmin.
+    const double zmin = g.bmin[2] - cam.pos[2];
+    double far2 = 0.0, rmax = 0.0;
+    for (int k = 0; k < 8; k++) {
+        const double x = (k & 1 ? g.bmax[0] : g.bmin[0]) - cam.pos[0];
+        const double y = (k & 2 ? g.bmax[1] : g.bmin[1]) - cam.pos[1];
+        const double z = (k & 4 ? g.bmax[2] : g.bmin[2]) - cam.pos[2];
+        far2 = std::max(far2, x * x + y * y + z * z);
+        rmax = std::max(rmax, std::max(std::fabs(x / z), std::fabs(y / z)));
+    }
+    const double inflate = 4e-7 * (std::sqrt(far2) + g.diag) * g.diag2;
+    const double px_per_unit = std::max(cam.width / (2.0 * cam.tan_half * cam.aspect), cam.height / (2.0 * cam.tan_half));
+    const double bound_px = inflate * (1.0 + rmax) / zmin * px_per_unit;
+    if (!(zmin > 0.0) || !(bound_px < 0.25)) return RM_OK;        // NaN fails too
+    int* c = nullptr;
+    RM_CUDA(dev_malloc(&c, (npx + 1) * sizeof(int)));
+    r->cover = c;
+    RM_CUDA(cudaMemsetAsync(c, 0, (npx + 1) * sizeof(int), r->stream));
+    const size_t n = r->ds->n_triangles[gi];
+    if (n) {
+        k_cover_rects<<<(unsigned)std::min<size_t>((n + kBlock - 1) / kBlock, (size_t)r->sms * 8), kBlock, 0, r->stream>>>(r->ds->tri_spheres[gi], n, cam,
+                                                                                                                     inflate, c);
+        r->launches++;
+    }
+    k_cover_cols<<<(unsigned)((W + kBlock - 1) / kBlock), kBlock, 0, r->stream>>>(c, (int)W, (int)H);
+    k_cover_rows<<<(unsigned)((H * 32 + kBlock - 1) / kBlock), kBlock, 0, r->stream>>>(c, (int)W, (int)H);
+    r->launches += 2;
+    RM_CUDA(cudaGetLastError());
+    int unprojectable = 0;
+    RM_CUDA(cudaMemcpyAsync(&unprojectable, c + npx, sizeof(int), cudaMemcpyDeviceToHost, r->stream));
+    RM_CUDA(cudaStreamSynchronize(r->stream));
+    if (unprojectable) { dev_free(r->cover); r->cover = nullptr; }
+    if (trace.on) {
+        char line[160];
+        snprintf(line, sizeof line, "renderer: coverage mask of the camera rays %s (error bound %.3g px)", r->cover ? "built" : "dropped", bound_px);
+        trace.mark(line);
+    }
+    return RM_OK;
+}
+
 static cudaEvent_t take_event(rm_renderer* r) {
     if (!r->event_pool.empty()) { cudaEvent_t e = r->event_pool.back(); r->event_pool.pop_back(); return e; }
     cudaEvent_t e = nullptr;
@@ -965,7 +1033,7 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         if (depth == 1) {
             sa.n_ptr = nullptr; sa.n_direct = n_paths;
             st = launch_intersect<SRC_CAMERA>(r->ds, rp, sa, r->isect.hit, r->isect.trav, &rp.cnt.trav[depth], &rp.cnt.cursor[depth], n_paths, depth, count,
-                                              r->totals, r->stream, hook);
+                                              r->totals, r->stream, hook, r->cover);
         } else {
             sa.n_ptr = &rp.cnt.rays[depth - 1]; sa.n_direct = 0;
             st = launch_intersect<SRC_QUEUE>(r->ds, rp, sa, r->isect.hit, r->isect.trav, &rp.cnt.trav[depth], &rp.cnt.cursor[depth], persistent_grid * kBlock,
@@ -1417,6 +1485,18 @@ int rm_renderer_bind_scene(rm_renderer* r, rm_device_scene* ds, int owning) {
     if (ds->device != r->device) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_bind_scene: the scene lives on another device");
     r->ds = ds;
     r->owns_scene = owning != 0;
+    RM_CUDA(cudaSetDevice(r->device));
+    return build_cover(r);
+}
+
+// The coverage mask of the camera rays (§3.7), as W*H ints 0 / 1 (row-major); RM_ERR_STATE when the renderer has none.
+int rm_renderer_coverage(rm_renderer* r, int32_t* out_host) {
+    if (!r || !out_host) return fail(RM_ERR_INVALID_ARGUMENT, "rm_renderer_coverage: null argument");
+    const int* c = r->cover;
+    if (!c) return fail(RM_ERR_STATE, "rm_renderer_coverage: the renderer's camera rays have no coverage mask");
+    RM_CUDA(cudaSetDevice(r->device));
+    RM_CUDA(cudaMemcpyAsync(out_host, c, (size_t)r->rp.cam.W * r->rp.cam.H * sizeof(int), cudaMemcpyDeviceToHost, r->stream));
+    RM_CUDA(cudaStreamSynchronize(r->stream));
     return RM_OK;
 }
 

@@ -195,6 +195,8 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* group, int share);
 void rm_scene_group_destroy(rm_scene_group* group);
 int rm_renderer_bind_scene(rm_renderer* r, rm_device_scene* ds, int owning);
 rm_device_scene* rm_renderer_device_scene(rm_renderer* r);
+// the coverage mask of the camera rays (DESIGN §3.7), W*H ints 0 / 1; RM_ERR_STATE when the renderer has none
+int rm_renderer_coverage(rm_renderer* r, int32_t* out_host);
 }
 
 struct rm_mesh { rm::Mesh mesh; };

@@ -706,6 +706,8 @@ struct SetupArgs {
     int grid_object;           // object index of the grid this pass sets up, -1 = none
     int analytic;              // 1: evaluate the Sphere/Plane objects and initialise the hit record
     int emitters_only;         // 1: the grid can only matter when the closest hit so far is an emitter (see k_setup)
+    const int* cover;          // SRC_CAMERA: W*H coverage mask of this pass's grid (k_cover_*), 0 = no triangle can be hit
+                               // from that frame pixel, so its ray is not traversed; null = traverse every ray
 };
 
 // Stage part 1.  See the header comment.
@@ -758,7 +760,10 @@ __global__ void __launch_bounds__(kBlock, kSetupBlocksPerSm) k_setup(const __gri
             // emitters_only (drop mode at the bounce limit, no grid object emits): the path delivers its throughput times the
             // emission of the closest object if that is an emitter, else an exact 0 (shade()).  A non-emissive grid can only
             // hide an emitter, so when the closest hit so far is not one, every answer of the traversal delivers the same 0.
-            const bool decided = a.emitters_only && (best_obj < 0 || sc.obj[best_obj].mat != RM_MATERIAL_EMISSION);
+            bool decided = a.emitters_only && (best_obj < 0 || sc.obj[best_obj].mat != RM_MATERIAL_EMISSION);
+            // a camera ray from a pixel outside the projection of every triangle's bounding sphere cannot hit the grid
+            // (DESIGN §3.7): AccGrid::intersects answers None and the hit record keeps the analytic answer
+            if (SRC == SRC_CAMERA && a.cover && a.cover[rp.pixel_map[i % rp.n_pixels]] == 0) decided = true;
             if (a.grid_object >= 0 && !decided) {
                 const DevGrid& g = sc.grid[sc.obj[a.grid_object].grid];
                 double tmin, tmax;
@@ -1381,6 +1386,89 @@ __global__ void __launch_bounds__(kBlock) k_primary_rays(const __grid_constant__
         double* r = reinterpret_cast<double*>(rays + i);
         r[0] = cam.pos[0]; r[1] = cam.pos[1]; r[2] = cam.pos[2];
         r[3] = d.x; r[4] = d.y; r[5] = d.z;
+    }
+}
+
+// ===================================================================== coverage mask of the camera rays (DESIGN §3.7)
+//
+// cover[W*H + 1] is zeroed by the caller; k_cover_rects marks one rectangle per triangle into cover[0, W*H) as a 2-D
+// difference array (and sets cover[W*H] when a triangle cannot be projected: the caller then drops the mask), k_cover_cols
+// and k_cover_rows turn it into per-pixel counts and then into 0 / 1.  Without DoF every camera ray starts at cam.pos and points along (px, py, 1), so it can only meet points whose
+// ratios (x/z, y/z) relative to the camera equal (px, py).
+
+constexpr int kCoverPad = 1;   // pixels added on every side of a projected box
+
+__global__ void __launch_bounds__(kBlock) k_cover_rects(const float4* __restrict__ spheres, const size_t n, const __grid_constant__ DevCamera cam,
+                                                         const double inflate, int* __restrict__ cover) {
+    const int W = cam.W, H = cam.H;
+    const double sx = cam.tan_half * cam.aspect, sy = cam.tan_half;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const float4 s = spheres[i];
+        const double r = (double)s.w + inflate;
+        // the sphere's axis-aligned box c +- r, relative to the camera
+        const double lx = (double)s.x - r - cam.pos[0], hx = (double)s.x + r - cam.pos[0];
+        const double ly = (double)s.y - r - cam.pos[1], hy = (double)s.y + r - cam.pos[1];
+        const double lz = (double)s.z - r - cam.pos[2], hz = (double)s.z + r - cam.pos[2];
+        // every corner strictly in front (NaN and an infinite radius fail here); otherwise no pixel can be ruled out
+        if (!(lz > 0.0) || !isfinite(hx) || !isfinite(lx) || !isfinite(hy) || !isfinite(ly) || !isfinite(hz)) {
+            cover[(size_t)W * H] = 1;
+            continue;
+        }
+        // x/z over the box is linear-fractional: its extremes are at corners, and for one x they are at z = lz or hz
+        const double xa = lx / lz, xb = lx / hz, xc = hx / lz, xd = hx / hz;
+        const double ya = ly / lz, yb = ly / hz, yc = hy / lz, yd = hy / hz;
+        const double xmin = fmin(fmin(xa, xb), fmin(xc, xd)), xmax = fmax(fmax(xa, xb), fmax(xc, xd));
+        const double ymin = fmin(fmin(ya, yb), fmin(yc, yd)), ymax = fmax(fmax(ya, yb), fmax(yc, yd));
+        // inverse of primary_direction: pixel x takes X = x + 0.5 + jitter in [x, x + 1), likewise Y
+        const double X0 = fmin(fmax((xmin / sx + 1.0) * 0.5 * cam.width, -4.0), (double)W + 4.0);
+        const double X1 = fmin(fmax((xmax / sx + 1.0) * 0.5 * cam.width, -4.0), (double)W + 4.0);
+        const double Y0 = fmin(fmax((1.0 - ymax / sy) * 0.5 * cam.height, -4.0), (double)H + 4.0);
+        const double Y1 = fmin(fmax((1.0 - ymin / sy) * 0.5 * cam.height, -4.0), (double)H + 4.0);
+        const int x0 = max((int)floor(X0) - kCoverPad, 0), x1 = min((int)floor(X1) + kCoverPad, W - 1);
+        const int y0 = max((int)floor(Y0) - kCoverPad, 0), y1 = min((int)floor(Y1) + kCoverPad, H - 1);
+        if (x0 > x1 || y0 > y1) continue;    // off the frame
+        atomicAdd(&cover[(size_t)y0 * W + x0], 1);
+        if (x1 + 1 < W) atomicAdd(&cover[(size_t)y0 * W + x1 + 1], -1);
+        if (y1 + 1 < H) {
+            atomicAdd(&cover[(size_t)(y1 + 1) * W + x0], -1);
+            if (x1 + 1 < W) atomicAdd(&cover[(size_t)(y1 + 1) * W + x1 + 1], 1);
+        }
+    }
+}
+
+// running sum down every column (one thread per column: adjacent threads read adjacent words)
+__global__ void __launch_bounds__(kBlock) k_cover_cols(int* __restrict__ cover, const int W, const int H) {
+    for (int x = blockIdx.x * blockDim.x + threadIdx.x; x < W; x += gridDim.x * blockDim.x) {
+        int sum = 0, y = 0;
+        for (; y + 8 <= H; y += 8) {
+            int v[8];
+#pragma unroll
+            for (int k = 0; k < 8; k++) v[k] = cover[(size_t)(y + k) * W + x];
+#pragma unroll
+            for (int k = 0; k < 8; k++) { sum += v[k]; cover[(size_t)(y + k) * W + x] = sum; }
+        }
+        for (; y < H; y++) { sum += cover[(size_t)y * W + x]; cover[(size_t)y * W + x] = sum; }
+    }
+}
+
+// running sum along every row (one warp per row, shuffle scan), stored as 0 / 1
+__global__ void __launch_bounds__(kBlock) k_cover_rows(int* __restrict__ cover, const int W, const int H) {
+    const unsigned lane = threadIdx.x & 31u;
+    const unsigned warps = (gridDim.x * blockDim.x) >> 5;
+    for (unsigned y = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; y < (unsigned)H; y += warps) {
+        int carry = 0;
+        for (int x0 = 0; x0 < W; x0 += 32) {
+            const int x = x0 + (int)lane;
+            int v = x < W ? cover[(size_t)y * W + x] : 0;
+#pragma unroll
+            for (int k = 1; k < 32; k <<= 1) {
+                const int u = __shfl_up_sync(0xffffffffu, v, k);
+                if ((int)lane >= k) v += u;
+            }
+            v += carry;
+            if (x < W) cover[(size_t)y * W + x] = v > 0 ? 1 : 0;
+            carry = __shfl_sync(0xffffffffu, v, 31);
+        }
     }
 }
 

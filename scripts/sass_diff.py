@@ -3,8 +3,9 @@
     python scripts/sass_diff.py OLD.so NEW.so
 
 Splits `cuobjdump -sass` of each library into one listing per kernel and compares the instruction text of every kernel of
-OLD with the kernel of NEW that stands for the same instantiation.  k_shade gained a trailing template flag ENV and a
-trailing DevEnv parameter with the environment map: k_shade<F, P, K, L> of OLD is k_shade<F, P, K, L, false> of NEW.
+OLD with the kernel of NEW that stands for the same instantiation: the kernel of the same name, or, for an OLD built before
+k_shade gained its trailing template flag ENV and DevEnv parameter (the environment map), k_shade<F, P, K, L> of OLD is
+k_shade<F, P, K, L, false> of NEW.
 Prints one line per kernel of OLD and the kernels only NEW has; exits 1 when any kernel of OLD differs or is missing.
 """
 from __future__ import annotations
@@ -49,10 +50,10 @@ def old_name(new: str):
 
 def main(old_lib: str, new_lib: str) -> int:
     old, new = kernels(old_lib), kernels(new_lib)
-    by_old = {}
+    by_old = {n: n for n in new if n in old}
     for n in new:
         o = old_name(n)
-        if o is not None:
+        if o is not None and o in old and o not in by_old:
             by_old[o] = n
     bad = 0
     for o in sorted(old):
