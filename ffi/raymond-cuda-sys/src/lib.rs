@@ -115,6 +115,18 @@ extern "C" {
 }
 pub const RM_ERR_IMAGE: c_int = -12;            // a malformed or unsupported image file (rm_load_hdr)
 
+// ---- colour textures (include/raymond.h states the uv of each geometry kind, the lookup and what a textured colour replaces)
+#[repr(C)] #[derive(Clone, Copy)] pub struct rm_texture {
+    pub texels: *const f32,            // width*height RGB triples, row-major, row 0 = top; copied
+    pub width: usize, pub height: usize, // 1..32768 each
+    pub scale_u: f64, pub scale_v: f64, // finite
+}
+extern "C" {
+    // null texture unbinds; RM_ERR_INVALID_ARGUMENT (scene unchanged) for a bad index, a NaN / Inf / negative texel, a bad size
+    // or scale; RM_ERR_UNSUPPORTED for an Emission object
+    pub fn rm_scene_set_texture(s: *mut rm_scene, object_index: usize, texture: *const rm_texture) -> c_int;
+}
+
 // ---- values of the enum / flag fields (include/raymond.h, RM_ABI_VERSION 2)
 pub const RM_PARTITION_SAMPLES: u32 = 0;        // rank g renders global samples g, g+G, ...
 pub const RM_PARTITION_TILES: u32 = 1;          // tiles dealt round-robin in the reference's queue order (src/trace.rs:146-172)

@@ -203,6 +203,39 @@ int rm_scene_set_environment(rm_scene* scene, const rm_environment* env);
  * truncated or unsupported one. */
 int rm_load_hdr(const char* path, size_t* width, size_t* height, float* texels);
 
+/* Colour texture of one object (no counterpart in the reference, whose materials have one colour: an object without a texture
+ * renders exactly as the reference's).  A texture is width x height RGB texels, row-major, row 0 at the top (t = 1), with a uv
+ * scale (su, sv); only a Diffuse or Metal object takes one.  At a hit on a textured object the colour a of its material is
+ * replaced, everywhere the integrator uses it (the diffuse albedo, f0 through the metal lerp, the RM_FLAG_AOV albedo), by
+ *   c = a (*) T(s, t)          componentwise: (a.x T.x, a.y T.y, a.z T.z)
+ * Every operation is f64 with no FMA contraction, in this order; frag = o + d t_hit is the hit point and n the surface normal:
+ *   grid    (ba, bb, bc) = the Heron weights of the surface normal (triangle.rs:47-68), uvK = rm_vertex.uv of vertex K of the hit
+ *           triangle:  (s, t) = ((uv2 ba) + (uv1 bb)) + (uv0 bc), per component (the normal's own expression)
+ *   sphere  s = 0.5 + atan2(n.x, n.z) / (2 pi),   t = 1 - acos(clamp(n.y, -1, 1)) / pi
+ *   plane   (tg, bt) = create_coordinate_system_of_n(normal as stored) (trace.rs:408-416),  p = frag - origin,
+ *           s = dot(p, tg),  t = dot(p, bt)           dot(a, b) = (a.x b.x + a.y b.y) + a.z b.z
+ * The lookup T(s, t):
+ *   s' = s su,  t' = t sv;  either NaN or infinite: T = (NaN, NaN, NaN)
+ *   s' -= floor(s'),  t' -= floor(t')
+ *   x = s' W - 0.5,  y = (1 - t') H - 0.5,  x0 = floor(x),  y0 = floor(y),  fx = x - x0,  fy = y - y0
+ *   columns x0, x0 + 1 wrap modulo W; rows y0, y0 + 1 wrap modulo H (repeat on both axes); t(row, column) = the texel widened
+ *   exactly to f64
+ *   top = t(y0, x0) + fx (t(y0, x1) - t(y0, x0)),   bot = t(y1, x0) + fx (t(y1, x1) - t(y1, x0)),   T = top + fy (bot - top)
+ * So a 1 x 1 texture returns exactly its texel, and a texture of all 1.0 gives c = a to the last bit.  The random draws, the
+ * hits, rm_stats.rays / samples and the emitters are those of the same scene without textures.  The texels of each textured
+ * object (16 bytes per texel) and, for each grid a textured object references, the uvs of its triangles (48 bytes per
+ * triangle) cross the bus once per device the scene is placed on and count in rm_stats.upload_bytes. */
+typedef struct rm_texture {
+    const float* texels;     /* width*height RGB triples, row-major, row 0 = top; copied */
+    size_t width, height;    /* 1..32768 each */
+    double scale_u, scale_v; /* finite */
+} rm_texture;
+/* Binds (copies) a texture to object `object_index` of the scene; NULL unbinds.  RM_ERR_INVALID_ARGUMENT for a null scene,
+ * an index >= the object count, null texels, a dimension outside 1..32768, a texel that is NaN, infinite or negative, or a
+ * scale that is not finite; RM_ERR_UNSUPPORTED for an Emission object.  On failure the scene is left as it was.  Device
+ * scenes, renderers and tasks made from the scene before the call keep the textures they were made with. */
+int rm_scene_set_texture(rm_scene* scene, size_t object_index, const rm_texture* texture);
+
 /* Scene::intersect(&self, Ray) -> Option<(&Object, Hit)>          scene.rs:54-74
  * batched over `count` rays held in HOST memory; results to HOST memory:
  *   object_index[i]    index into scene.objects, -1 for a miss

@@ -108,6 +108,10 @@ class EnvironmentC(C.Structure):
     _fields_ = [("texels", C.c_void_p), ("width", C.c_size_t), ("height", C.c_size_t), ("scale", C.c_double), ("rotation", C.c_double)]
 
 
+class TextureC(C.Structure):
+    _fields_ = [("texels", C.c_void_p), ("width", C.c_size_t), ("height", C.c_size_t), ("scale_u", C.c_double), ("scale_v", C.c_double)]
+
+
 class TileC(C.Structure):
     _fields_ = [("sample_count", C.c_size_t), ("width", C.c_size_t), ("height", C.c_size_t), ("left", C.c_size_t), ("top", C.c_size_t),
                 ("data", C.POINTER(Vec3C))]
@@ -156,7 +160,7 @@ ABI_SYMBOLS = [
     "rm_write_png", "rm_project_load_scene", "rm_message_to_json", "rm_release_cached_memory", "rm_measure_fp64_rate",
     "rm_render_tiled_adaptive", "rm_renderer_read_moments", "rm_renderer_tile_errors", "rm_renderer_set_active_tiles",
     "rm_renderer_read_aovs", "rm_renderer_read_denoised", "rm_render_tiled_denoised", "rm_task_await_denoised",
-    "rm_scene_set_environment", "rm_load_hdr",
+    "rm_scene_set_environment", "rm_load_hdr", "rm_scene_set_texture",
 ]
 
 _lib = None
@@ -197,6 +201,7 @@ def lib():
         "rm_scene_destroy": (None, [vp]),
         "rm_scene_set_environment": (i32, [vp, P(EnvironmentC)]),
         "rm_load_hdr": (i32, [C.c_char_p, P(sz), P(sz), vp]),
+        "rm_scene_set_texture": (i32, [vp, sz, P(TextureC)]),
         "rm_scene_intersect": (i32, [vp, i32, vp, sz, vp, vp, vp]),
         "rm_tile_free": (None, [P(TileC)]),
         "rm_render_tiled": (vp, [vp, P(SettingsC), P(GpuOptionsC)]),
@@ -460,6 +465,25 @@ class Scene:
 
     def clear_environment(self) -> None:
         _check(lib().rm_scene_set_environment(self._h, None))
+
+    def set_texture(self, index: int, image: np.ndarray, scale=(1.0, 1.0)) -> None:
+        """Texture the colour of object `index` (Diffuse or Metal): `image` is (H, W, 3) float32, row 0 at the top (t = 1),
+        repeated on both axes; `scale` = (su, sv) multiplies the uv of the hit.  The uv of a grid hit comes from its vertices'
+        uv, a sphere and a plane have their own mapping; the lookup and its semantics are rm_texture's (include/raymond.h).  A
+        .hdr image can be read with load_hdr.  The texels are copied; RM_ERR_INVALID_ARGUMENT (scene unchanged) for an index out
+        of range, a NaN, infinite or negative texel, a dimension outside 1..32768 or a scale that is not finite, and
+        RM_ERR_UNSUPPORTED for an Emission object."""
+        img = np.asarray(image)
+        if img.ndim != 3 or img.shape[2] != 3:
+            raise RaymondError(RM_ERR_INVALID_ARGUMENT, f"set_texture: image must be (H, W, 3), got {img.shape}")
+        su, sv = scale
+        t = np.ascontiguousarray(img, dtype=np.float32)
+        tex = TextureC(t.ctypes.data, t.shape[1], t.shape[0], float(su), float(sv))
+        _check(lib().rm_scene_set_texture(self._h, int(index), C.byref(tex)))
+
+    def clear_texture(self, index: int) -> None:
+        """Give object `index` its material's one colour again."""
+        _check(lib().rm_scene_set_texture(self._h, int(index), None))
 
     def __len__(self) -> int:
         return int(lib().rm_scene_object_count(self._h))

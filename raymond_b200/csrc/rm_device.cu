@@ -269,7 +269,10 @@ struct rm_device_scene {
     bool emissive_grid = false;             // a grid object has an Emission material: its traversal can decide a last-depth path
     bool has_env = false;                   // the scene has an environment map: `env` points at this device's copy of its texels
     DevEnv env{};
-    std::vector<void*> allocations;         // one device block per distinct grid, in DevScene::grid order, then the environment map
+    bool has_tex = false;                   // an object has a colour texture: `tex` points at this device's copies
+    DevTex tex{};
+    std::vector<void*> allocations;         // one device block per distinct grid, in DevScene::grid order, then the environment map,
+                                            // the textures in object order and the uvs of the textured grids
     std::vector<size_t> allocation_bytes;
     std::vector<std::shared_ptr<Grid>> keep;
     double upload_ms = 0.0;
@@ -448,6 +451,8 @@ struct rm_scene_group {
     std::vector<int> grid_objects;                  // object indices with Geometry::Grid, ascending
     bool emissive_grid = false;
     std::shared_ptr<const Environment> env;         // the scene's environment map (or none); every share uploads its own copy
+    std::vector<std::shared_ptr<const Texture>> textures;   // per object: its colour texture (or none); every share uploads its own copies
+    std::vector<std::vector<double>> grid_uv;       // per distinct grid: 6 f64 per triangle (uv0 uv1 uv2) when a textured object references it
     std::vector<std::shared_ptr<Grid>> grids;       // distinct grids, in DevScene::grid order
     std::vector<GridImage> images;                  // ... and their host images
     double flatten_ms = 0.0;                        // host time of the table and the images
@@ -506,6 +511,25 @@ static int build_scene_table(rm_scene_group* grp, const rm_scene* scene) {
             d.grid = it->second;
             grp->grid_objects.push_back((int)i);
             if (d.mat == RM_MATERIAL_EMISSION) grp->emissive_grid = true;
+        }
+        grp->textures.push_back(o.texture);
+    }
+    // the uvs of a grid go up only when a textured object references it, so that an untextured scene uploads what it always did
+    grp->grid_uv.assign((size_t)s.n_grids, {});
+    for (size_t i = 0; i < scene->objects.size(); i++) {
+        if (!scene->objects[i].texture || scene->objects[i].geometry != GEOM_GRID) continue;
+        std::vector<double>& uv = grp->grid_uv[(size_t)s.obj[i].grid];
+        const std::vector<rm_triangle>& tris = scene->objects[i].grid->triangles;
+        if (!uv.empty() || tris.empty()) continue;
+        try {
+            uv.resize(tris.size() * 6);
+        } catch (const std::bad_alloc&) {
+            return fail(RM_ERR_OUT_OF_MEMORY, "cannot hold the uvs of a textured grid");
+        }
+        for (size_t k = 0; k < tris.size(); k++) {
+            const rm_triangle& t = tris[k];
+            double* u = uv.data() + 6 * k;
+            u[0] = t.v0.uv.x; u[1] = t.v0.uv.y; u[2] = t.v1.uv.x; u[3] = t.v1.uv.y; u[4] = t.v2.uv.x; u[5] = t.v2.uv.y;
         }
     }
     return RM_OK;
@@ -576,6 +600,29 @@ rm_device_scene* rm_scene_group_join(rm_scene_group* grp, int share) {
             ds->has_env = true;
             ds->env = DevEnv{(const float4*)dev, (int)env.width, (int)env.height, env.scale, env.rotation};
         }
+    }
+    // the colour textures and the uvs of the textured grids: a copy per share, host -> device
+    auto upload = [&](const void* src, size_t bytes, void** dev) {
+        cudaError_t ue = visible_acquire(device, bytes, dev);
+        if (ue != cudaSuccess) return ue;
+        ds->allocations.push_back(*dev);
+        ds->allocation_bytes.push_back(bytes);
+        ds->bytes += bytes;
+        return cudaMemcpyAsync(*dev, src, bytes, cudaMemcpyHostToDevice, 0);
+    };
+    for (size_t i = 0; i < grp->textures.size() && e == cudaSuccess; i++) {
+        if (!grp->textures[i]) continue;
+        const Texture& t = *grp->textures[i];
+        void* dev = nullptr;
+        e = upload(t.rgba.data(), t.rgba.size() * sizeof(float), &dev);
+        ds->tex.obj[i] = DevTexObject{(const float4*)dev, (int)t.width, (int)t.height, t.scale_u, t.scale_v};
+        ds->has_tex = true;
+    }
+    for (size_t g = 0; g < grp->grid_uv.size() && e == cudaSuccess; g++) {
+        if (grp->grid_uv[g].empty()) continue;
+        void* dev = nullptr;
+        e = upload(grp->grid_uv[g].data(), grp->grid_uv[g].size() * sizeof(double), &dev);
+        ds->tex.uv[g] = (const double*)dev;
     }
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&grp->uploaded[(size_t)share], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventRecord(grp->uploaded[(size_t)share], 0);
@@ -992,12 +1039,22 @@ struct StageHook : LaunchHook {
     }
 };
 
-// k_shade with or without the scene's environment map (env = NULL: none)
+static const DevTex no_tex{};      // the last parameter of k_shade / k_aov for a scene without textures
+
+// k_shade with or without the scene's environment map (env = NULL: none) and its colour textures (tex = NULL: none).  The
+// LAST body shades no surface: it runs without the textures.
+template <bool FIRST, int PREC, bool KEEP, bool LAST, bool ENV, bool TEX>
+static void launch_shade_t(rm_renderer* r, unsigned grid, const RenderParams& rp, const Queue& qin, const Queue& qout, unsigned depth, unsigned n_first,
+                           const DevEnv& env, const DevTex& tex) {
+    k_shade<FIRST, PREC, KEEP, LAST, ENV, TEX><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_first, env, tex);
+}
 template <bool FIRST, int PREC, bool KEEP, bool LAST>
 static void launch_shade(rm_renderer* r, unsigned grid, const RenderParams& rp, const Queue& qin, const Queue& qout, unsigned depth, unsigned n_first,
-                         const DevEnv* env) {
-    if (env) k_shade<FIRST, PREC, KEEP, LAST, true><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_first, *env);
-    else k_shade<FIRST, PREC, KEEP, LAST, false><<<grid, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, qout, r->isect.hit, depth, n_first, DevEnv{});
+                         const DevEnv* env, const DevTex* tex) {
+    if (env && tex && !LAST) launch_shade_t<FIRST, PREC, KEEP, LAST, true, !LAST>(r, grid, rp, qin, qout, depth, n_first, *env, *tex);
+    else if (env) launch_shade_t<FIRST, PREC, KEEP, LAST, true, false>(r, grid, rp, qin, qout, depth, n_first, *env, no_tex);
+    else if (tex && !LAST) launch_shade_t<FIRST, PREC, KEEP, LAST, false, !LAST>(r, grid, rp, qin, qout, depth, n_first, DevEnv{}, *tex);
+    else launch_shade_t<FIRST, PREC, KEEP, LAST, false, false>(r, grid, rp, qin, qout, depth, n_first, DevEnv{}, no_tex);
 }
 
 template <int PREC>
@@ -1018,6 +1075,7 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
     const bool last_shade = !keep && r->last_depth_shortcut;
     const bool last_skip = last_shade && !count && !r->ds->emissive_grid && !r->ds->has_env;
     const DevEnv* env = r->ds->has_env ? &r->ds->env : nullptr;
+    const DevTex* tex = r->ds->has_tex ? &r->ds->tex : nullptr;
     const unsigned persistent_grid = (unsigned)r->sms * 8u;
     RM_CUDA(cudaMemsetAsync(r->counters, 0, r->counter_slots * 3 * sizeof(unsigned), r->stream));
     if (limit == 0) RM_CUDA(cudaMemsetAsync(rp.contrib, 0, (size_t)rp.cap * 3 * sizeof(double), r->stream));   // trace() returns 0 at depth 1 > 0
@@ -1042,20 +1100,22 @@ static int renderer_batch_t(rm_renderer* r, unsigned first_sample, unsigned n_sa
         if (st != RM_OK) return st;
         if (depth == 1 && r->aov) {     // before k_shade: the next depth's k_setup overwrites the hit records
             const size_t W = r->settings.camera_settings.backbuffer_width, H = r->settings.camera_settings.backbuffer_height;
-            k_aov<<<(rp.n_pixels + kBlock - 1) / kBlock, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, r->isect.hit, n_samples, W * H, r->aov);
+            const unsigned blocks = (rp.n_pixels + kBlock - 1) / kBlock;
+            if (tex) k_aov<true><<<blocks, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, r->isect.hit, n_samples, W * H, r->aov, *tex);
+            else k_aov<false><<<blocks, kBlock, 0, r->stream>>>(r->ds->scene, rp, qin, r->isect.hit, n_samples, W * H, r->aov, no_tex);
             r->launches++;
         }
         hook.begin(2);
         const bool last = last_shade && depth == limit;
         if (depth == 1) {
             const unsigned grid = std::min<unsigned>((n_paths + kBlock - 1) / kBlock, persistent_grid * 4u);
-            if (keep) launch_shade<true, PREC, true, false>(r, grid, rp, qin, qout, depth, n_paths, env);
-            else if (last) launch_shade<true, PREC, false, true>(r, grid, rp, qin, qout, depth, n_paths, env);
-            else launch_shade<true, PREC, false, false>(r, grid, rp, qin, qout, depth, n_paths, env);
+            if (keep) launch_shade<true, PREC, true, false>(r, grid, rp, qin, qout, depth, n_paths, env, tex);
+            else if (last) launch_shade<true, PREC, false, true>(r, grid, rp, qin, qout, depth, n_paths, env, tex);
+            else launch_shade<true, PREC, false, false>(r, grid, rp, qin, qout, depth, n_paths, env, tex);
         } else {
-            if (keep) launch_shade<false, PREC, true, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
-            else if (last) launch_shade<false, PREC, false, true>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
-            else launch_shade<false, PREC, false, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env);
+            if (keep) launch_shade<false, PREC, true, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env, tex);
+            else if (last) launch_shade<false, PREC, false, true>(r, persistent_grid, rp, qin, qout, depth, 0u, env, tex);
+            else launch_shade<false, PREC, false, false>(r, persistent_grid, rp, qin, qout, depth, 0u, env, tex);
         }
         hook.end(2);
     }

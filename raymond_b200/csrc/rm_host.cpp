@@ -561,6 +561,42 @@ int rm_scene_set_environment(rm_scene* scene, const rm_environment* env) {
     return RM_OK;
 }
 
+int rm_scene_set_texture(rm_scene* scene, size_t object_index, const rm_texture* texture) {
+    if (!scene) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: null scene");
+    if (object_index >= scene->objects.size())
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: object index " + std::to_string(object_index) + " out of range");
+    Object& o = scene->objects[object_index];
+    if (!texture) { o.texture.reset(); return RM_OK; }
+    if (o.material.kind == RM_MATERIAL_EMISSION) return fail(RM_ERR_UNSUPPORTED, "rm_scene_set_texture: an Emission object cannot be textured");
+    if (!texture->texels) return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: null texels");
+    if (texture->width < 1 || texture->width > 32768 || texture->height < 1 || texture->height > 32768)
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: width and height must be 1..32768");
+    if (!std::isfinite(texture->scale_u) || !std::isfinite(texture->scale_v))
+        return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: scale_u and scale_v must be finite");
+    const size_t n = texture->width * texture->height;
+    for (size_t i = 0; i < 3 * n; i++)
+        if (!std::isfinite(texture->texels[i]) || texture->texels[i] < 0.0f)
+            return fail(RM_ERR_INVALID_ARGUMENT, "rm_scene_set_texture: texel value " + std::to_string(i) + " is negative, NaN or infinite");
+    auto t = std::make_shared<Texture>();
+    try {
+        t->rgba.resize(4 * n);
+    } catch (const std::bad_alloc&) {
+        return fail(RM_ERR_OUT_OF_MEMORY, "rm_scene_set_texture: cannot hold the texels");
+    }
+    for (size_t i = 0; i < n; i++) {
+        t->rgba[4 * i] = texture->texels[3 * i];
+        t->rgba[4 * i + 1] = texture->texels[3 * i + 1];
+        t->rgba[4 * i + 2] = texture->texels[3 * i + 2];
+        t->rgba[4 * i + 3] = 0.0f;
+    }
+    t->width = texture->width;
+    t->height = texture->height;
+    t->scale_u = texture->scale_u;
+    t->scale_v = texture->scale_v;
+    o.texture = std::move(t);        // placements made before keep the texture they share
+    return RM_OK;
+}
+
 // Radiance RGBE (.hdr) body: see rm_load_hdr in include/raymond.h.  `texels` NULL = size only.
 static int decode_hdr(const std::string& buf, const char* path, size_t* width, size_t* height, float* texels) {
     auto bad = [&](const std::string& why) { return fail(RM_ERR_IMAGE, std::string(path) + ": " + why); };

@@ -70,6 +70,14 @@ int build_grid_device(std::vector<rm_triangle>&& tris, const rm_aabb& bounds, in
 
 enum GeometryKind : int { GEOM_PLANE = 0, GEOM_SPHERE = 1, GEOM_GRID = 2 };   // scene.rs:9-13
 
+// The colour texture of one object (rm_scene_set_texture), immutable once set: width x height texels, row 0 = top, stored as
+// RGBA f32 (A = 0) in the layout the device reads.  Scenes and the placements made from them share it.
+struct Texture {
+    std::vector<float> rgba;
+    size_t width = 0, height = 0;
+    double scale_u = 1.0, scale_v = 1.0;
+};
+
 struct Object {                                             // scene.rs:33-37
     int geometry;
     rm_vec3 origin;
@@ -77,6 +85,7 @@ struct Object {                                             // scene.rs:33-37
     double radius;
     std::shared_ptr<Grid> grid;
     rm_material material;
+    std::shared_ptr<const Texture> texture;                 // none in the reference: null = the material's one colour
 };
 
 // The environment map of a scene (rm_scene_set_environment), immutable once set: width x height texels, row 0 = +y, stored as

@@ -142,6 +142,19 @@ struct DevEnv {
     double scale, rotation;
 };
 
+// The colour textures of a scene (rm_scene_set_texture), per object: W x H texels, row 0 = top, RGB in .xyz (texels null = the
+// object has none); per grid: 6 f64 per triangle (uv0 uv1 uv2) in grid triangle order, set only for the grids a textured object
+// references.  k_shade and k_aov take it as their last parameter (about 2 KB), for the reason DevEnv is one.
+struct DevTexObject {
+    const float4* texels;
+    int W, H;
+    double su, sv;
+};
+struct DevTex {
+    DevTexObject obj[kMaxObjects];
+    const double* uv[kMaxGrids];
+};
+
 __host__ __device__ inline unsigned stage_slot(unsigned depth) { return depth < RM_STAGE_SLOTS - 1 ? depth : RM_STAGE_SLOTS - 1; }
 
 // ===================================================================== device math (cgmath semantics)
@@ -446,16 +459,21 @@ __device__ __forceinline__ double heron(D3 a, D3 b, D3 c) {
     const double s = (ab + ac + bc) / 2.0;
     return sqrt(s * (s - ab) * (s - ac) * (s - bc));
 }
-__device__ __forceinline__ D3 triangle_normal(const DevGrid& g, unsigned ti, D3 p) {
+// ... that also returns the weights ba, bb, bc of v2, v1, v0 (the texture's uv of the hit, see surface_normal_color)
+__device__ __forceinline__ D3 triangle_normal_weights(const DevGrid& g, unsigned ti, D3 p, double& ba, double& bb, double& bc) {
     const double* tp = g.shd + (size_t)ti * 18;
     const D3 v0 = ld3(tp), v1 = ld3(tp + 3), v2 = ld3(tp + 6);
     const D3 n0 = ld3(tp + 9), n1 = ld3(tp + 12), n2 = ld3(tp + 15);
     const double abc = heron(v0, v1, v2);
     const double abp = heron(v0, v1, p);
     const double bcp = heron(v0, v2, p);
-    const double ba = abp / abc, bb = bcp / abc;
-    const double bc = 1.0 - (ba + bb);
+    ba = abp / abc; bb = bcp / abc;
+    bc = 1.0 - (ba + bb);
     return normalize((n2 * ba) + (n1 * bb) + (n0 * bc));
+}
+__device__ __forceinline__ D3 triangle_normal(const DevGrid& g, unsigned ti, D3 p) {
+    double ba, bb, bc;
+    return triangle_normal_weights(g, ti, p, ba, bb, bc);
 }
 
 // ---- f32 helpers of the statistical scope (RM_PRECISION_F32_SHADING).  The TU is compiled with -fmad=false (the bit-exact
@@ -666,10 +684,69 @@ __device__ __forceinline__ D3 env_radiance(const DevEnv& e, D3 d) {
     return e.scale * (top + fy * (bot - top));
 }
 
+// T(s, t) of a colour texture (include/raymond.h, rm_texture): repeat on both axes, bilinear in the lerp form, f64 with every
+// operation in the order the header gives (tests/tex_oracle.cpp and tests/tex_ref.py restate it).
+__device__ __forceinline__ D3 tex_lookup(const DevTexObject& x, double s, double t) {
+    double sp = s * x.su, tp = t * x.sv;
+    if (!isfinite(sp) || !isfinite(tp)) { const double nan = __longlong_as_double(0x7ff8000000000000ll); return d3(nan, nan, nan); }
+    sp -= floor(sp);
+    tp -= floor(tp);                                   // both in [0, 1]: 1 when a tiny negative value rounds up
+    const double fxx = sp * (double)x.W - 0.5, fyy = (1.0 - tp) * (double)x.H - 0.5;
+    const double x0 = floor(fxx), y0 = floor(fyy);
+    const double fx = fxx - x0, fy = fyy - y0;
+    int ix0 = (int)x0, iy0 = (int)y0;                  // ix0 in [-1, W - 1], iy0 in [-1, H - 1]
+    int ix1 = ix0 + 1, iy1 = iy0 + 1;
+    if (ix0 < 0) ix0 += x.W;
+    if (ix1 >= x.W) ix1 -= x.W;
+    if (iy0 < 0) iy0 += x.H;
+    if (iy1 >= x.H) iy1 -= x.H;
+    const float4 a = __ldg(&x.texels[(size_t)iy0 * x.W + ix0]), b = __ldg(&x.texels[(size_t)iy0 * x.W + ix1]);
+    const float4 c = __ldg(&x.texels[(size_t)iy1 * x.W + ix0]), f = __ldg(&x.texels[(size_t)iy1 * x.W + ix1]);
+    const D3 t00 = d3(a.x, a.y, a.z), t01 = d3(b.x, b.y, b.z), t10 = d3(c.x, c.y, c.z), t11 = d3(f.x, f.y, f.z);
+    const D3 top = t00 + fx * (t01 - t00), bot = t10 + fx * (t11 - t10);
+    return top + fy * (bot - top);
+}
+
+// surface_normal in a scene with textures, and in `color` the colour the material's a stands for at the hit: a, or a (*) T(s, t)
+// for a textured object, with (s, t) the uv of the hit (include/raymond.h, rm_texture).  Scenes without textures keep the
+// plain surface_normal and ld3(ob.color), so that their kernels are the code they were.
+__device__ __forceinline__ D3 surface_normal_color(const DevScene& sc, const DevTex& tex, int hit_obj, unsigned hit_sub, D3 frag, unsigned& shaded_tri,
+                                                   D3& color) {
+    const DevObject& ob = sc.obj[hit_obj];
+    color = ld3(ob.color);
+    if (!tex.obj[hit_obj].texels) return surface_normal(sc, ob, hit_sub, frag, shaded_tri);
+    const double kPi = 3.141592653589793;
+    D3 normal;
+    double s, t;
+    if (ob.geom == GEOM_PLANE) {
+        normal = ld3(ob.g + 3);
+        D3 tg, bt;
+        onb(normal, tg, bt);
+        const D3 p = frag - ld3(ob.g);
+        s = dot(p, tg);
+        t = dot(p, bt);
+    } else if (ob.geom == GEOM_SPHERE) {
+        normal = normalize(frag - ld3(ob.g));
+        s = 0.5 + atan2(normal.x, normal.z) / (2.0 * kPi);
+        const double cy = normal.y < -1.0 ? -1.0 : normal.y > 1.0 ? 1.0 : normal.y;
+        t = 1.0 - acos(cy) / kPi;
+    } else {
+        double ba, bb, bc;
+        normal = triangle_normal_weights(sc.grid[ob.grid], hit_sub, frag, ba, bb, bc);
+        shaded_tri++;
+        const double* uv = tex.uv[ob.grid] + (size_t)hit_sub * 6;
+        s = ((uv[4] * ba) + (uv[2] * bb)) + (uv[0] * bc);
+        t = ((uv[5] * ba) + (uv[3] * bb)) + (uv[1] * bc);
+    }
+    color = mul(color, tex_lookup(tex.obj[hit_obj], s, t));
+    return normal;
+}
+
 // ENV: the scene has an environment map; a ray that misses delivers T (*) env_radiance(d) (BOUNCE_EMIT) instead of ending with 0.
-template <int PREC, bool KEEP, bool ENV>
-__device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, const DevEnv& env, double hit_t, int hit_obj, unsigned hit_sub,
-                                        unsigned pixel, unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
+// TEX: the scene has colour textures; the lobe takes the textured colour (surface_normal_color).
+template <int PREC, bool KEEP, bool ENV, bool TEX>
+__device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& rp, const DevEnv& env, const DevTex& tex, double hit_t, int hit_obj,
+                                        unsigned hit_sub, unsigned pixel, unsigned sample, unsigned depth, D3& o, D3& d, D3& v, unsigned& shaded_tri) {
     if (hit_obj < 0) {                                                      // :242
         if (ENV) { v = env_radiance(env, d); return BOUNCE_EMIT; }
         return BOUNCE_NONE;
@@ -678,13 +755,14 @@ __device__ __forceinline__ Bounce shade(const DevScene& sc, const RenderParams& 
     const D3 frag = o + d * hit_t;                                          // :246
     if (ob.mat == RM_MATERIAL_EMISSION) { v = ld3(ob.color); return BOUNCE_EMIT; }   // :250
     if (!KEEP && depth >= rp.bounce_limit) return BOUNCE_NONE;              // the child call returns 0 (:235-237)
-    const D3 normal = surface_normal(sc, ob, hit_sub, frag, shaded_tri);    // :244
+    D3 color;                                                               // TEX: the textured colour
+    const D3 normal = TEX ? surface_normal_color(sc, tex, hit_obj, hit_sub, frag, shaded_tri, color) : surface_normal(sc, ob, hit_sub, frag, shaded_tri);   // :244
     const D3 to_camera = ld3(rp.cam.pos) - frag;
     const double metal = ob.mat == RM_MATERIAL_METAL ? 1.0 : 0.0;
     D3 dir;
     double eps;
-    if (PREC == RM_PRECISION_F32_SHADING) lobe_f32(rp, normal, to_camera, ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
-    else lobe_f64(rp, normal, to_camera, ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
+    if (PREC == RM_PRECISION_F32_SHADING) lobe_f32(rp, normal, to_camera, TEX ? color : ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
+    else lobe_f64(rp, normal, to_camera, TEX ? color : ld3(ob.color), ob.rough, metal, pixel, sample, depth, dir, v, eps);
     if (KEEP && depth >= rp.bounce_limit) return BOUNCE_NONE;
     o = frag + normal * eps;
     d = dir;
@@ -1177,11 +1255,14 @@ __global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const
 // ENV: the scene has an environment map `env` (the last parameter, unused otherwise, so that the instantiations without one keep
 // the parameter layout and the code they had before it existed).  A miss delivers T (*) env_radiance(d); the LAST body reads d
 // from the queue for misses only.
-template <bool FIRST, int PREC, bool KEEP, bool LAST, bool ENV>
+// TEX: the scene has colour textures `tex` (the last parameter, unused otherwise, for the same reason).  Only the general and
+// keep bodies shade a surface, so LAST never takes them.
+template <bool FIRST, int PREC, bool KEEP, bool LAST, bool ENV, bool TEX>
 __global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue qin,
                                                    const Queue qout, const HitArrays hit, const unsigned depth, const unsigned n_first,
-                                                   const DevEnv env) {
+                                                   const DevEnv env, const __grid_constant__ DevTex tex) {
     static_assert(!(LAST && KEEP), "keep mode computes the last weight: it has no last-depth shortcut");
+    static_assert(!(LAST && TEX), "the last-depth body shades no surface");
     const unsigned n = FIRST ? n_first : rp.cnt.rays[depth - 1];
     const unsigned lane = threadIdx.x & 31u;
     const unsigned warps_total = (gridDim.x * blockDim.x) >> 5;
@@ -1213,7 +1294,7 @@ __global__ void __launch_bounds__(kBlock, kShadeBlocksPerSm) k_shade(const __gri
             d = d3(qin.f[3][i], qin.f[4][i], qin.f[5][i]);
             const unsigned q = slot % rp.n_pixels, s_local = slot / rp.n_pixels;
             D3 v = d3(0.0, 0.0, 0.0);
-            const Bounce b = shade<PREC, KEEP, ENV>(sc, rp, env, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
+            const Bounce b = shade<PREC, KEEP, ENV, TEX>(sc, rp, env, tex, hit.t[i], hit.obj[i], hit.sub[i], rp.pixel_map[q], rp.first_sample + s_local * rp.sample_stride, depth, o, d, v, shaded_tri);
             // the path's value is (prod of weights) (*) emission (src/trace.rs:281-282,315-319): the throughput so far comes in only now
             T = d3(0.0, 0.0, 0.0);
             if (KEEP || b != BOUNCE_NONE) T = mul(FIRST ? d3(1.0, 1.0, 1.0) : d3(qin.f[6][i], qin.f[7][i], qin.f[8][i]), v);
@@ -1286,10 +1367,12 @@ __global__ void __launch_bounds__(kBlock) k_accumulate(const __grid_constant__ R
 // RM_FLAG_AOV: the first-hit feature sums (include/raymond.h), launched between the depth-1 intersection and k_shade<FIRST>, while
 // the depth-1 queue holds the camera rays and `hit` their closest hits.  One thread per owned pixel adds the batch's samples
 // i = s * n_pixels + q in global sample order, as k_accumulate does; a miss adds zeros.  `aov` holds three planes of the frame:
-// albedo (3 doubles per pixel), normal (3), depth (1).
+// albedo (3 doubles per pixel), normal (3), depth (1).  TEX: the scene has colour textures `tex` (the last parameter, unused
+// otherwise); the albedo is the textured colour.
+template <bool TEX>
 __global__ void __launch_bounds__(kBlock) k_aov(const __grid_constant__ DevScene sc, const __grid_constant__ RenderParams rp, const Queue q1,
                                                  const HitArrays hit, const unsigned n_batch_samples, const size_t frame_pixels,
-                                                 double* __restrict__ aov) {
+                                                 double* __restrict__ aov, const __grid_constant__ DevTex tex) {
     const unsigned q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= rp.n_pixels) return;
     const size_t p = rp.pixel_map[q];
@@ -1308,8 +1391,11 @@ __global__ void __launch_bounds__(kBlock) k_aov(const __grid_constant__ DevScene
             const DevObject& o = sc.obj[ob];
             t = hit.t[i];
             const D3 frag = d3(q1.f[0][i], q1.f[1][i], q1.f[2][i]) + d3(q1.f[3][i], q1.f[4][i], q1.f[5][i]) * t;
-            a = ld3(o.color);
-            n = surface_normal(sc, o, hit.sub[i], frag, unused);
+            if (TEX) n = surface_normal_color(sc, tex, ob, hit.sub[i], frag, unused, a);
+            else {
+                a = ld3(o.color);
+                n = surface_normal(sc, o, hit.sub[i], frag, unused);
+            }
         }
         sa = sa + a; sn = sn + n; sz += t;
     }

@@ -239,19 +239,23 @@ def cube(half: float = 0.521075) -> np.ndarray:
     return make_triangles(p[:, 0], p[:, 1], p[:, 2])
 
 
-def bumpy_sphere(n_lat: int = 24, n_lon: int = 48, radius: float = 1.0, bump: float = 0.12, squash=(1.0, 0.8, 0.6)) -> np.ndarray:
+def bumpy_sphere(n_lat: int = 24, n_lon: int = 48, radius: float = 1.0, bump: float = 0.12, squash=(1.0, 0.8, 0.6), *,
+                 uv: bool = False) -> np.ndarray:
     """Closed bumpy ellipsoid with smooth vertex normals — a small anisotropic test mesh
-    (res.y > res.z after the grid resolution estimate => exercises the aliasing quirk A1)."""
+    (res.y > res.z after the grid resolution estimate => exercises the aliasing quirk A1).  `uv`: see _grid_surface."""
     th = np.linspace(0.0, np.pi, n_lat + 1)
     ph = np.linspace(0.0, 2.0 * np.pi, n_lon, endpoint=False)
     T, P = np.meshgrid(th, ph, indexing="ij")
     r = radius * (1.0 + bump * np.sin(5.0 * T) * np.cos(4.0 * P) + 0.5 * bump * np.cos(3.0 * T + 1.0))
     pts = np.stack([r * np.sin(T) * np.cos(P), r * np.cos(T), r * np.sin(T) * np.sin(P)], axis=-1) * np.asarray(squash)
-    return _grid_surface(pts, wrap_u=False, wrap_v=True)
+    return _grid_surface(pts, wrap_u=False, wrap_v=True, uv=uv)
 
 
-def _grid_surface(pts: np.ndarray, wrap_u: bool, wrap_v: bool) -> np.ndarray:
-    """Triangulate a (nu, nv, 3) point grid; smooth vertex normals from central differences."""
+def _grid_surface(pts: np.ndarray, wrap_u: bool, wrap_v: bool, uv: bool = False) -> np.ndarray:
+    """Triangulate a (nu, nv, 3) point grid; smooth vertex normals from central differences.  `uv`: every vertex carries its
+    surface parameter as its uv, (i, j) / (the number of cells along u, along v), so the texture of rm_texture spans the
+    surface once; the last cell of a wrapped axis ends at 1, not 0.  Without `uv` the uvs stay zero (the arrays the fixtures
+    always had)."""
     nu, nv, _ = pts.shape
     du = np.roll(pts, -1, axis=0) - np.roll(pts, 1, axis=0)
     dv = np.roll(pts, -1, axis=1) - np.roll(pts, 1, axis=1)
@@ -275,6 +279,12 @@ def _grid_surface(pts: np.ndarray, wrap_u: bool, wrap_v: bool) -> np.ndarray:
     n = lambda ij: nrm[ij[0], ij[1]].reshape(-1, 3)
     t1 = make_triangles(p(a), p(b), p(c), n(a), n(b), n(c))
     t2 = make_triangles(p(a), p(c), p(d), n(a), n(c), n(d))
+    if uv:
+        cu, cv = float(len(iu)), float(len(iv))
+        st = lambda i, j: np.stack([i.reshape(-1) / cu, j.reshape(-1) / cv], axis=-1)
+        for t, corners in ((t1, (st(I, J), st(I + 1, J), st(I + 1, J + 1))), (t2, (st(I, J), st(I + 1, J + 1), st(I, J + 1)))):
+            for k, c2 in enumerate(corners):
+                t[:, 11 * k + _UV:11 * k + _UV + 2] = c2
     out = np.empty((t1.shape[0] * 2, TRI_DOUBLES))
     out[0::2] = t1
     out[1::2] = t2
@@ -284,14 +294,14 @@ def _grid_surface(pts: np.ndarray, wrap_u: bool, wrap_v: bool) -> np.ndarray:
     return np.ascontiguousarray(out[area2 > 1e-14])
 
 
-def dragon_standin(nu: int = 1320, nv: int = 330) -> np.ndarray:
+def dragon_standin(nu: int = 1320, nv: int = 330, *, uv: bool = False) -> np.ndarray:
     """STAND-IN for the missing dragon_vrip.ply: a closed, bumpy tube around a closed space curve.
 
     Default 1320 x 330 x 2 = 871 200 triangles (the Stanford dragon has 871 414), smooth vertex
     normals, mesh-local bounding box ~ x[-1.14, 1.14] y[-0.63, 0.85] z[-0.50, 0.50] — the regime
     SURVEY.md Appendix D estimates from examples/GoldDragon.png (res.y > res.z, so the grid's
     index aliasing A1 is exercised; rests near the floor after the (0, -0.3, 2.9) translate).
-    Deterministic (no RNG).
+    Deterministic (no RNG).  `uv`: the tube's (curve, around) parameter as the vertices' uv (see _grid_surface).
     """
     s = np.linspace(0.0, 2.0 * np.pi, nu, endpoint=False)
     ph = np.linspace(0.0, 2.0 * np.pi, nv, endpoint=False)
@@ -305,7 +315,7 @@ def dragon_standin(nu: int = 1320, nv: int = 330) -> np.ndarray:
     S, P = np.meshgrid(s, ph, indexing="ij")
     r = 0.17 + 0.045 * np.sin(5.0 * S) + 0.012 * np.sin(40.0 * S) * np.sin(24.0 * P) + 0.004 * np.sin(130.0 * S + 7.0 * P)
     pts = c[:, None, :] + r[..., None] * (np.cos(P)[..., None] * n1[:, None, :] + np.sin(P)[..., None] * n2[:, None, :])
-    return _grid_surface(pts, wrap_u=True, wrap_v=True)
+    return _grid_surface(pts, wrap_u=True, wrap_v=True, uv=uv)
 
 
 # ---------------------------------------------------------------------------- triangle soup (C4)

@@ -5,7 +5,8 @@
 Splits `cuobjdump -sass` of each library into one listing per kernel and compares the instruction text of every kernel of
 OLD with the kernel of NEW that stands for the same instantiation: the kernel of the same name, or, for an OLD built before
 k_shade gained its trailing template flag ENV and DevEnv parameter (the environment map), k_shade<F, P, K, L> of OLD is
-k_shade<F, P, K, L, false> of NEW.
+k_shade<F, P, K, L, false> of NEW.  Likewise for an OLD built before the colour textures gave k_shade the flag TEX and a DevTex
+parameter: k_shade<F, P, K, L, E> of OLD is k_shade<F, P, K, L, E, false> of NEW, and k_aov of OLD is k_aov<false>.
 Prints one line per kernel of OLD and the kernels only NEW has; exits 1 when any kernel of OLD differs or is missing.
 """
 from __future__ import annotations
@@ -42,6 +43,12 @@ def kernels(lib: str) -> dict:
 
 def old_name(new: str):
     """The OLD kernel a NEW one stands for (None: new instantiation)."""
+    m = re.match(r"(_ZN2rm7k_shadeILb[01]ELi[01]ELb[01]ELb[01]ELb[01])ELb([01])(EEEv.*jjNS_6DevEnvE)NS_6DevTexE$", new)
+    if m:
+        return m.group(1) + m.group(3) if m.group(2) == "0" else None
+    m = re.match(r"_ZN2rm5k_aovILb([01])EEEv(.*Pd)NS_6DevTexE$", new)
+    if m:
+        return "_ZN2rm5k_aovE" + m.group(2) if m.group(1) == "0" else None
     m = re.match(r"(_ZN2rm7k_shadeILb[01]ELi[01]ELb[01]ELb[01])ELb([01])(EEEv.*jj)NS_6DevEnvE$", new)
     if m:
         return m.group(1) + m.group(3) if m.group(2) == "0" else None
