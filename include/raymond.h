@@ -533,6 +533,8 @@ typedef struct rm_stage_stats {
     uint64_t occupied_cells[RM_STAGE_SLOTS];   /* of cells, the ones with a non-empty list (RM_FLAG_COUNT_WORK) */
     uint64_t evaluated_test_flops[RM_STAGE_SLOTS]; /* f64 add/sub/mul/div executed by the evaluated Triangle::intersects calls: 20, 30, 46 or 52
                                                 * per call depending on the exit taken, triangle.rs:11-44 (RM_FLAG_COUNT_WORK) */
+    uint64_t cell_sphere_tests[RM_STAGE_SLOTS];  /* of occupied_cells, the ones whose cell-wide bounding sphere was tested; zero with
+                                                  * RM_NO_CELL_SPHERES set when the scene was placed (RM_FLAG_COUNT_WORK) */
 } rm_stage_stats;
 int rm_renderer_stage_stats(rm_renderer* r, rm_stage_stats* out);
 void rm_renderer_destroy(rm_renderer* r);

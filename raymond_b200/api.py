@@ -134,12 +134,12 @@ KERNEL_KINDS = ("setup", "traverse", "shade", "accumulate", "bin")      # kind 4
 
 class StageStatsC(C.Structure):
     _fields_ = [("ms", (C.c_double * STAGE_SLOTS) * len(KERNEL_KINDS)), ("launches", (C.c_uint64 * STAGE_SLOTS) * len(KERNEL_KINDS))] + \
-               [(n, C.c_uint64 * STAGE_SLOTS) for n in ("rays", "grid_rays", "cells", "triangle_tests", "shaded_triangles", "evaluated_tests", "occupied_cells", "evaluated_test_flops")]
+               [(n, C.c_uint64 * STAGE_SLOTS) for n in ("rays", "grid_rays", "cells", "triangle_tests", "shaded_triangles", "evaluated_tests", "occupied_cells", "evaluated_test_flops", "cell_sphere_tests")]
 
     def as_dict(self) -> dict:
         d = {"ms": {k: list(self.ms[i]) for i, k in enumerate(KERNEL_KINDS)},
              "launches": {k: list(self.launches[i]) for i, k in enumerate(KERNEL_KINDS)}}
-        for n in ("rays", "grid_rays", "cells", "triangle_tests", "shaded_triangles", "evaluated_tests", "occupied_cells", "evaluated_test_flops"):
+        for n in ("rays", "grid_rays", "cells", "triangle_tests", "shaded_triangles", "evaluated_tests", "occupied_cells", "evaluated_test_flops", "cell_sphere_tests"):
             d[n] = list(getattr(self, n))
         return d
 

@@ -300,6 +300,37 @@ __global__ void __launch_bounds__(256) k_spread_spheres(const float4* __restrict
         per_reference[p] = __ldg(&per_triangle[__ldg(&refs[p])]);
 }
 
+// One sphere per occupied cell (DevGrid::csph) from the per-reference spheres of its list: f32 centre at the middle of the box
+// around the members' spheres, radius R_c >= (max |c_c - c_i| + R_i) (1 + 2e-6), evaluated in f64 and rounded up to f32, so that
+// every member sphere lies inside it with the margin DESIGN §3.1 needs; a member with a non-finite radius (a non-finite triangle)
+// makes the cell's infinite (never culled).  Empty cells are never read and get an infinite one.
+__global__ void __launch_bounds__(256) k_cell_spheres(const uint2* __restrict__ cells, size_t n_cells, const float4* __restrict__ sphr,
+                                                       float4* __restrict__ csph) {
+    for (size_t c = (size_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_cells; c += (size_t)gridDim.x * blockDim.x) {
+        const uint2 cell = __ldg(&cells[c]);
+        double lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+        bool finite = cell.y > 0;
+        for (unsigned p = cell.x; p < cell.x + cell.y; p++) {
+            const float4 m = __ldg(&sphr[p]);
+            const double r = (double)m.w;
+            finite = finite && isfinite(r);
+            lo[0] = fmin(lo[0], (double)m.x - r); hi[0] = fmax(hi[0], (double)m.x + r);
+            lo[1] = fmin(lo[1], (double)m.y - r); hi[1] = fmax(hi[1], (double)m.y + r);
+            lo[2] = fmin(lo[2], (double)m.z - r); hi[2] = fmax(hi[2], (double)m.z + r);
+        }
+        const float cx = (float)((lo[0] + hi[0]) * 0.5), cy = (float)((lo[1] + hi[1]) * 0.5), cz = (float)((lo[2] + hi[2]) * 0.5);
+        double reach = 0.0;
+        for (unsigned p = cell.x; finite && p < cell.x + cell.y; p++) {
+            const float4 m = __ldg(&sphr[p]);
+            const double dx = (double)cx - (double)m.x, dy = (double)cy - (double)m.y, dz = (double)cz - (double)m.z;
+            reach = fmax(reach, sqrt((dx * dx + dy * dy) + dz * dz) + (double)m.w);
+        }
+        const float rc = __double2float_ru(reach * (1.0 + 2e-6));
+        csph[c] = finite && isfinite(rc) && isfinite(cx) && isfinite(cy) && isfinite(cz) ? make_float4(cx, cy, cz, rc)
+                                                                                          : make_float4(0.f, 0.f, 0.f, INFINITY);
+    }
+}
+
 // The flattened image of one grid: the arrays of DevGrid laid out in ONE block — [tri][shd][cells][occ][refs][one sphere per
 // triangle] come from the host, [one sphere per reference] behind them is spread on the device (k_spread_spheres), so it never
 // crosses the bus.  The host image of an immutable grid is built once by a few host threads and kept (pinned) with the grid;
@@ -307,6 +338,7 @@ __global__ void __launch_bounds__(256) k_spread_spheres(const float4* __restrict
 struct GridImage {
     DevGrid header{};          // geometry of the grid; the array pointers are set by point_grid()
     size_t off_tri = 0, off_shd = 0, off_cells = 0, off_occ = 0, off_refs = 0, off_spht = 0, host_total = 0, off_sph = 0, total = 0, nr = 0, nt = 0;
+    size_t off_csph = 0, nc = 0;    // one sphere per cell behind them (none with RM_NO_CELL_SPHERES when the image was laid out)
     char* host = nullptr;
     bool cached = false;       // the host image belongs to the grid (not released after the upload)
 };
@@ -336,6 +368,11 @@ static int prepare_grid_image(const Grid& g, GridImage* out) {
     im.host_total = im.off_spht + pad(nt * sizeof(float4)) + 256;
     im.off_sph = im.host_total;
     im.total = im.off_sph + pad(nr * sizeof(float4)) + 256;
+    im.nc = nc;
+    if (getenv("RM_NO_CELL_SPHERES") == nullptr) {
+        im.off_csph = im.total;
+        im.total = im.off_csph + pad(nc * sizeof(float4)) + 256;
+    }
     const size_t host_total = im.host_total;
     std::unique_lock<std::mutex> image_lock(g.image_mu);
     const bool have_image = g.image && g.image_bytes == host_total;
@@ -426,6 +463,7 @@ static void point_grid(const GridImage& im, void* dev, DevGrid* out) {
     d.cells = (const uint2*)((char*)dev + im.off_cells);
     d.occ = (const unsigned*)((char*)dev + im.off_occ);
     d.refs = (const unsigned*)((char*)dev + im.off_refs);
+    d.csph = im.off_csph ? (const float4*)((char*)dev + im.off_csph) : nullptr;
     *out = d;
 }
 
@@ -434,6 +472,9 @@ static cudaError_t spread_spheres(const GridImage& im, void* dev, int sms, cudaS
     if (!im.nr) return cudaSuccess;
     k_spread_spheres<<<(unsigned)std::min<size_t>((im.nr + 255) / 256, (size_t)sms * 32), 256, 0, stream>>>(
         (const float4*)((char*)dev + im.off_spht), (const unsigned*)((char*)dev + im.off_refs), im.nr, (float4*)((char*)dev + im.off_sph));
+    if (!im.off_csph || !im.nc) return cudaGetLastError();
+    k_cell_spheres<<<(unsigned)std::min<size_t>((im.nc + 255) / 256, (size_t)sms * 32), 256, 0, stream>>>(
+        (const uint2*)((char*)dev + im.off_cells), im.nc, (const float4*)((char*)dev + im.off_sph), (float4*)((char*)dev + im.off_csph));
     return cudaGetLastError();
 }
 
@@ -1817,6 +1858,7 @@ int rm_renderer_stage_stats(rm_renderer* r, rm_stage_stats* out) {
         out->evaluated_tests[i] = t.survivors[i];
         out->occupied_cells[i] = t.occupied[i];
         out->evaluated_test_flops[i] = t.test_flops[i];
+        out->cell_sphere_tests[i] = t.cell_tests[i];
     }
     return RM_OK;
 }

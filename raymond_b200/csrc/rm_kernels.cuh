@@ -64,6 +64,8 @@ struct DevGrid {
     const double* tri;
     const float4* sphr;       // 16 B per REFERENCE (same order as refs): bounding sphere of the referenced triangle (see cull_sphere)
     const double* shd;
+    const float4* csph;       // 16 B per CELL: a sphere around the reference spheres of the cell's list (k_cell_spheres); null with
+                              // RM_NO_CELL_SPHERES set when the scene was placed
 };
 
 struct DevObject {
@@ -111,7 +113,7 @@ constexpr int kTravDoubles = 16;
 
 struct DevTotals {
     unsigned long long samples, rays, nonfinite;
-    unsigned long long stage_rays[RM_STAGE_SLOTS], grid_rays[RM_STAGE_SLOTS], cells[RM_STAGE_SLOTS], tests[RM_STAGE_SLOTS], shaded[RM_STAGE_SLOTS], survivors[RM_STAGE_SLOTS], occupied[RM_STAGE_SLOTS], test_flops[RM_STAGE_SLOTS];
+    unsigned long long stage_rays[RM_STAGE_SLOTS], grid_rays[RM_STAGE_SLOTS], cells[RM_STAGE_SLOTS], tests[RM_STAGE_SLOTS], shaded[RM_STAGE_SLOTS], survivors[RM_STAGE_SLOTS], occupied[RM_STAGE_SLOTS], test_flops[RM_STAGE_SLOTS], cell_tests[RM_STAGE_SLOTS];
 };
 
 // Per-batch device counters, all indexed by depth (zeroed once per batch).
@@ -954,7 +956,7 @@ __global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const
     // DDA state of MY ray (acc_grid.rs:100-125): parked in sh.dda_t / dda_c / dda_s, in registers only during phase A
     const unsigned rx = (unsigned)g.res[0], ry = (unsigned)g.res[1], rz = (unsigned)g.res[2];
     unsigned k = 0, cnt = 0;
-    unsigned n_cells = 0, n_tests = 0, n_surv = 0, n_occ = 0, n_flops = 0;
+    unsigned n_cells = 0, n_tests = 0, n_surv = 0, n_occ = 0, n_flops = 0, n_ctests = 0;
 #if defined(RM_TRAV_PROFILE)
     unsigned long long prof[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     long long prof_t = clock64();
@@ -1069,11 +1071,22 @@ __global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const
             sh.dda_t[0][lane] = tmx; sh.dda_t[1][lane] = tmy; sh.dda_t[2][lane] = tmz;
             sh.dda_c[0][lane] = cx; sh.dda_c[1][lane] = cy; sh.dda_c[2][lane] = cz;
         }
-        // the cell records of every ray that found an occupied cell, in one round trip (not one per walk iteration)
+        // the cell records of every ray that found an occupied cell, in one round trip (not one per walk iteration), with the
+        // cell's sphere: a ray whose line provably misses it cannot hit any triangle of the list (DESIGN §3.1), so the cell
+        // puts nothing into the pool and the ray walks on as from a cell without a hit
         if (state == TS_READY) {
             const uint2 cell = __ldg(&g.cells[k]);
+            bool culled = false;
+            if (g.csph) {                                        // warp-uniform
+                const float4 cs = __ldg(&g.csph[k]);
+                const double2 r0 = sh.ray[lane][0], r1 = sh.ray[lane][1], r2 = sh.ray[lane][2];
+                const double2 dl = sh.dd_lim[lane];
+                culled = cull_sphere(cs, d3(r0.x, r0.y, r1.x), d3(r1.y, r2.x, r2.y), dl.x, dl.y);
+                if (COUNT) n_ctests++;
+            }
             k = cell.x; cnt = cell.y;
             if (COUNT) { n_tests += cnt; n_occ++; }
+            if (culled) state = TS_STEP;
         }
         RM_PROF_MARK(1);
         // ---- B: pooled triangle tests of every ready cell
@@ -1234,12 +1247,14 @@ __global__ void __launch_bounds__(kTravBlock, kTravBlocksPerSm) k_traverse(const
     if (COUNT) {
         const unsigned c = __reduce_add_sync(FULL, n_cells), t = __reduce_add_sync(FULL, n_tests);
         const unsigned sv = __reduce_add_sync(FULL, n_surv), oc = __reduce_add_sync(FULL, n_occ), fl = __reduce_add_sync(FULL, n_flops);
+        const unsigned ct = __reduce_add_sync(FULL, n_ctests);
         if (lane == 0) {
             atomicAdd(&a.totals->cells[stage_slot(a.depth)], (unsigned long long)c);
             atomicAdd(&a.totals->tests[stage_slot(a.depth)], (unsigned long long)t);
             atomicAdd(&a.totals->survivors[stage_slot(a.depth)], (unsigned long long)sv);
             atomicAdd(&a.totals->occupied[stage_slot(a.depth)], (unsigned long long)oc);
             atomicAdd(&a.totals->test_flops[stage_slot(a.depth)], (unsigned long long)fl);
+            atomicAdd(&a.totals->cell_tests[stage_slot(a.depth)], (unsigned long long)ct);
         }
     }
 }
